@@ -208,6 +208,27 @@ def run_reference_arm(args):
     print(json.dumps(line), flush=True)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, res, table: np.ndarray) -> None:
+    """What one timed step hands its caller, as float64 .npy files, so that two builds can be compared output for output:
+    this rank's BatchResult (segment offsets per unit, segment lengths and means, RNG draws consumed per unit) and the
+    gathered segment table of all ranks (rows: global unit id, length, mean).  Past 64 MB in all, every array keeps the
+    same share of its rows, chosen by a fixed seed."""
+    arrays = {"seg_offsets": res.seg_offsets, "lengths": res.lengths, "means": res.means, "draws": res.draws,
+              "segment_table": table}
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(out_dir, exist_ok=True)
+    room = DUMP_LIMIT_BYTES - 4096  # .npy headers
+    for name, a in arrays.items():
+        if total > room:
+            keep = int(len(a) * room // total)
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------
 def run_gpu_arm(args):
     import torch
@@ -306,6 +327,8 @@ def run_gpu_arm(args):
 
     warm = max(args.warmup, 3) if not args.cohort_run else args.warmup
     total_ms, res, clocks = timed(step_device, args.steps, warm, sample_clocks=True)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, gather_tables.last)
     steps_device = timed.last_steps
     local_device = timed.last_local
     e2e_ms, res_h, _ = timed(step_host, args.steps, 0 if args.cohort_run else max(args.warmup, 3))
@@ -494,7 +517,11 @@ def main():
     ap.add_argument("--hybrid", action="store_true",
                     help="hybrid p-values (DNAcopy's default method, `cna segment --hybrid true`) instead of the CLI default; "
                          "not the headline configuration")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last device-resident timed step's results to DIR/<name>.npy (float64, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

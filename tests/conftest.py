@@ -22,10 +22,19 @@ def oracle():
 
 @pytest.fixture(scope="session")
 def ref():
+    """The compiled reference where oracle/_ref was built; elsewhere its stored results (tests/refgolden.py)."""
     from oracle.pyoracle import Ref
+    import refgolden
     if not Ref.available():
-        pytest.skip("oracle/_ref/libcbs_ref.so not built (reference sources absent)")
-    return Ref()
+        yield refgolden.Replay.load()
+        return
+    path = os.environ.get("CBS_REF_GOLDEN_RECORD")
+    if not path:
+        yield Ref()
+        return
+    rec = refgolden.Recorder(Ref(), path)
+    yield rec
+    rec.save()
 
 
 @pytest.fixture(scope="session")
