@@ -145,6 +145,29 @@ CBS_HD int block_end(int n, int nb, int b) {  // 1-based b; block_end(.,.,0) == 
 }
 
 // ------------------------------------------------------------------------------------
+// Binary data (ibin = true): the reject decision of a permutation (CBS.cpp:218-224, 862-864) is thresh <= M / (tss'/n)
+// with tss' = tss, or 1 when tss <= 1e-4.  A division by a positive constant is monotone in M, so the decision is
+// M >= Lstar for the smallest double Lstar that passes the reference's own expression: found by stepping from the estimate.
+// ------------------------------------------------------------------------------------
+CBS_HD double bin_reject_level(double ostat, double tss, int n) {
+    const double c = (tss <= 0.0001 ? 1.0 : tss) / (double)n;
+    const double thresh = ostat * 0.99999;
+    const double inf = HUGE_VAL;
+    double m = thresh * c;
+    if (!(m > 0.0)) m = 0.0;
+    for (int k = 0; k < 64 && m / c < thresh; ++k) m = nextafter(m, inf);
+    for (int k = 0; k < 64 && m > 0.0 && nextafter(m, 0.0) / c >= thresh; ++k) m = nextafter(m, 0.0);
+    return m;
+}
+// fac * (s - 0.5)^2 <= fac_max / 4 for every |S_j - S_i| = s < 0.5 of an arc inside the bands (al0 <= L <= n - al0), so above
+// that level only arcs with s >= 0.5 can reject, where the statistic is monotone in s.  Below it (a "weak" threshold) the
+// reference's order-dependent pair skipping decides, and the permutations take the ordered walk (binary.cuh, DESIGN 4c).
+CBS_HD bool bin_weak(double lstar, int n, int al0) {
+    const double rn = (double)n, ra = (double)al0;
+    return !(lstar > 0.25 * (rn / (ra * (rn - ra))));
+}
+
+// ------------------------------------------------------------------------------------
 // Worklist records
 // ------------------------------------------------------------------------------------
 enum TaskState {
@@ -197,6 +220,7 @@ struct Task {
     int w_tie;           // the maximum was attained in two pairs with EQUAL corner statistics: k_wobs_fin walks the pairs in the reference's
                          // own (std::sort) order to get the location (weighted.cuh wtmaxo_ordered)
     double w_delta;      // weighted hybrid: min weight of a (kmax+1)-marker arc / total weight (getmncwt, CBS.cpp:602-607)
+    long long off_bin;   // binary data: scratch of the ordered walk (binary.cuh) for the observed row / every row of a weak batch, or -1
 };
 
 struct Chain {        // MT replay: one serial stream
@@ -397,6 +421,7 @@ struct Sched {
         t.cnt_exit = -1; t.cnt_nrej = 0;
         t.e_side = 0; t.e_done = 0; t.e_batch_P = 0;
         for (int s = 0; s < 2; ++s) { t.e_status[s] = 0; t.e_nrej[s] = 0; t.e_m1[s] = 0; t.e_n1[s] = 0; t.e_n2[s] = 0; t.e_off[s] = 0; }
+        t.off_bin = -1;
         t.key = task_key(D.prm.seed, D.unit_ids ? D.unit_ids[unit] : (uint64_t)unit, (uint32_t)lo, (uint32_t)hi);
         return idx;
     }
@@ -446,6 +471,9 @@ struct Sched {
     CBS_HD static long long bs_stride(int nb) { return (3LL * nb + 4 + 3) & ~3LL; }
     // scratch of wtmaxo_ordered (weighted.cuh), in doubles: per block 2 doubles + 2 ints, per block pair 3 doubles + 3 ints
     CBS_HD static long long wexact_stride(int nb) { const long long nb2 = (long long)nb * (nb + 1) / 2; return (3 * (nb + 1) + 5 * (nb2 + 1) + 8 + 3) & ~3LL; }
+    // scratch of the binary ordered walk (binary.cuh), in doubles: per block pair a (corner statistic, index) record of 2
+    // doubles, the pair bound and 2 ints (pair, corner length)
+    CBS_HD static long long bin_stride(int nb) { const long long e = (long long)nb * (nb + 1) / 2 + 1; return (4 * e + 3) & ~3LL; }
     // 32-bit index array of the global-memory shuffle, in doubles; all strides are multiples of 4 doubles so
     // that every row of prefix sums starts on a 32-byte boundary (k_prefix moves rows with 128-bit accesses)
     CBS_HD static long long idx_stride(int n) { return (((long long)n + 1) / 2 + 1 + 3) & ~3LL; }
@@ -524,10 +552,12 @@ struct Sched {
         Task& t = D.tasks[idx];
         t.nb = block_count(t.n);
         const long long wx = D.w ? wexact_stride(t.nb) : 0;  // weighted: scratch of the ordered walk (only used when maxima tie)
-        const long long need = sx_stride(t.n) + bs_stride(t.nb) + wx;
+        const long long bx = D.prm.ibin ? bin_stride(t.nb) : 0;  // binary data: scratch of the ordered walk
+        const long long need = sx_stride(t.n) + bs_stride(t.nb) + wx + bx;
         if (need > D.arena_cap) { D.error = ERR_ARENA; return false; }
         if (arena_used + need > D.arena_cap || rej_used + 1 > D.rej_cap) { t.deferred = 1; return false; }
         t.off_sx = arena_used; t.off_bs = arena_used + sx_stride(t.n); t.off_A = wx ? t.off_bs + bs_stride(t.nb) : -1;
+        t.off_bin = bx ? t.off_bs + bs_stride(t.nb) : -1;
         arena_used += need;
         t.off_rej = rej_used; rej_used += 1;
         D.prep_task[D.n_prep++] = idx;
@@ -558,7 +588,9 @@ struct Sched {
         const int cls = shuffle_class(t.n, D.shuf_cl2 != 0);
         // fallback shuffle of segments > 65535 markers (k_perm): a 32-bit index array per permutation in the arena
         const long long idxd = (cls == SHUF_GLOBAL && D.shuf_arena) ? idx_stride(t.n) : 0;  // doubles per permutation
-        const long long per = idxd + sx_stride(t.n) + bs_stride(t.nb);
+        // binary data with a weak reject level: every permutation takes the ordered walk and needs its scratch
+        const long long bx = (p.ibin && bin_weak(bin_reject_level(t.ostat, t.tss, t.n), t.n, p.min_width)) ? bin_stride(t.nb) : 0;
+        const long long per = idxd + sx_stride(t.n) + bs_stride(t.nb) + bx;
         const bool mtwin = p.rng_mode == RNG_MT && !D.shared_stream;
         // never let one task take more than half of the arena
         long long fit = (D.arena_cap / 2) / per;
@@ -575,7 +607,7 @@ struct Sched {
             if (want > by_span) want = (int)by_span;
         }
         const int gpart = (cls == SHUF_GLOBAL) ? want : 0;
-        const long long need = idxd * gpart + (sx_stride(t.n) + bs_stride(t.nb)) * want;
+        const long long need = idxd * gpart + (sx_stride(t.n) + bs_stride(t.nb) + bx) * want;
         const long long dneed = (p.rng_mode == RNG_MT) ? (long long)want * t.n : 0;
         if (arena_used + need > D.arena_cap || rej_used + want > D.rej_cap || (mtwin && draws_used + dneed + 312 > D.draws_cap)) {
             t.deferred = 1;
@@ -598,6 +630,7 @@ struct Sched {
         t.off_A = gpart ? arena_used : -1;
         t.off_sx = arena_used + idxd * gpart;
         t.off_bs = t.off_sx + sx_stride(t.n) * want;
+        t.off_bin = bx ? t.off_bs + bs_stride(t.nb) * want : -1;
         arena_used += need;
         t.off_rej = rej_used; rej_used += want;
         t.batch_P = want;

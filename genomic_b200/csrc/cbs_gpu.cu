@@ -165,7 +165,7 @@ void collect_timers(cbs_gpu_ctx* c) {
 
 int validate_params(cbs_gpu_ctx* c, const cbs_gpu_params* p) {
     if (!p) return fail(c, CBS_GPU_ERR_INVALID, "params is NULL");
-    if (p->ibin) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "ibin=true is only implemented for cbs::tmaxo / cbs::tmaxp (cbs_gpu_tmaxo, cbs_gpu_tmaxp), not for the segmentation worklist: `cna segment` never sets it");
+    if (p->ibin && p->hybrid) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "ibin=true with hybrid=true is not implemented: htmaxp has no binary variant");
     if (p->hybrid && (p->kmax < 1 || p->kmax > 128)) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "hybrid: kmax must be in 1..128");
     if (p->min_width < 1) return fail(c, CBS_GPU_ERR_INVALID, "min_width must be >= 1");
     if (p->nperm < 0) return fail(c, CBS_GPU_ERR_INVALID, "nperm must be >= 0");
@@ -391,6 +391,7 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     if (Nmax > 1000000) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "units longer than 1,000,000 markers are not supported");
     if (N > 2000000000LL) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "more than 2e9 markers per call are not supported");
     const bool mt = p->rng_mode == CBS_GPU_RNG_MT19937_64;
+    if (weighted && p->ibin) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "weighted CBS has no binary mode (cbs::segment_weighted takes no ibin)");
     if (weighted && p->hybrid && p->nmin < p->kmax + 2)
         return fail(c, CBS_GPU_ERR_UNSUPPORTED, "weighted hybrid CBS needs nmin >= kmax + 2");
 
@@ -603,6 +604,7 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     const size_t scan_smem = lay.bytes();
     const size_t wscan_smem = ((sizeof(WScanSmem) + 15) & ~(size_t)15) + (size_t)lay.nb_max * (2 * sizeof(double) + 3 * sizeof(int)) + 16;
     const int scan_grid = c->sm_count * scan_occ;
+    const size_t bscan_smem = ((sizeof(BinSmem) + 15) & ~(size_t)15) + (size_t)lay.nb_max * (2 * sizeof(double) + 3 * sizeof(int)) + 16;
 
     // shared-memory shuffle kernel, one launch per segment-length class present in this call
     int shuf_occ[SHUF_CL2]; bool shuf_on[SHUF_CL2];
@@ -724,6 +726,7 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
               k_wscan<0><<<c->sm_count * 4, 256, wscan_smem, st>>>(dD, lay.nb_max);   // permutation rows
               c->launches += 2;
           }
+          else if (p->ibin) k_scan_binary<<<c->sm_count * 4, 256, bscan_smem, st>>>(dD, lay.nb_max);
           else k_scan<<<scan_grid, lay.warps * 32, scan_smem, st>>>(dD, lay); }
         if (p->hybrid) {
             if (weighted) k_whscan<<<c->sm_count * 4, 256, 0, st>>>(dD); else k_hscan<<<c->sm_count * 4, 256, 0, st>>>(dD);
@@ -741,10 +744,11 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
         std::vector<unsigned char> key;
         auto put = [&](const void* v, size_t nbytes) { const unsigned char* b = (const unsigned char*)v; key.insert(key.end(), b, b + nbytes); };
 #define KEY_POD(v) put(&(v), sizeof(v))
-        const int flags[6] = {weighted ? 1 : 0, mt ? 1 : 0, shared_stream ? 1 : 0, hD.jump_polys ? 1 : 0, p->hybrid ? 1 : 0, l2_shuffle_on ? 1 : 0};
+        const int flags[7] = {weighted ? 1 : 0, mt ? 1 : 0, shared_stream ? 1 : 0, hD.jump_polys ? 1 : 0, p->hybrid ? 1 : 0, l2_shuffle_on ? 1 : 0,
+                              p->ibin ? 1 : 0};
         KEY_POD(dD); KEY_POD(st); KEY_POD(flags); KEY_POD(n_chains); KEY_POD(shuf_occ); KEY_POD(shuf_on); KEY_POD(cl_R); KEY_POD(cl_grid);
         KEY_POD(cl2_grid); KEY_POD(cl_smem); KEY_POD(cl2_smem); KEY_POD(chain_occ); KEY_POD(scan_grid); KEY_POD(scan_smem);
-        KEY_POD(wscan_smem); KEY_POD(lay);
+        KEY_POD(wscan_smem); KEY_POD(bscan_smem); KEY_POD(lay);
         const void* tailp_ptr = c->tailp.p; KEY_POD(tailp_ptr);
 #undef KEY_POD
         if (c->call_exec && key == c->call_key) {

@@ -48,7 +48,7 @@ typedef struct cbs_gpu_params {
     int32_t nmin;
     double eta; /* accepted, unused -- as in the reference */
     double tol;
-    int32_t ibin;
+    int32_t ibin;          /* binary data (CBS.cpp:99-224, ibin branches); not with hybrid, not on the weighted entries */
     int32_t undo_prune;
     double undo_prune_cutoff;
     int32_t do_smooth;
