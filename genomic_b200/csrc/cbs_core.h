@@ -140,6 +140,16 @@ struct DrawSrc {
 // Block geometry (CBS.cpp:71,77)
 // ------------------------------------------------------------------------------------
 CBS_HD int block_count(int n) { return n >= 50 ? (int)lround(sqrt((double)n)) : 1; }
+
+// The observed scan of a pending segment (k_scan_obs) is spread over one CTA per OBS_SLICE_MARKERS markers, at most
+// `cap` CTAs: a round holds only a few observed rows, and one CTA per row leaves most SMs idle (round 0: 23 rows).
+enum { OBS_SLICE_MARKERS = 8192, OBS_SLICES_MAX = 24 };
+CBS_HD int obs_slices(int n, int cap) {
+    const int s = (n + OBS_SLICE_MARKERS - 1) / OBS_SLICE_MARKERS;
+    return s < 1 ? 1 : (s > cap ? (cap < 1 ? 1 : cap) : s);
+}
+// work-stealing counters of the plain scan kernels, and the most slices any observed row of the round takes
+enum { CTR_SCAN_PERM = 16, CTR_SCAN_OBS = 17, CTR_OBS_SLICES = 18 };
 CBS_HD int block_end(int n, int nb, int b) {  // 1-based b; block_end(.,.,0) == 0
     return (int)lround((double)n * ((double)b / (double)nb));
 }
@@ -217,6 +227,11 @@ struct Task {
     unsigned long long w_level, w_found;
     double w_init, w_corner, w_v;
     int w_q, w_phase, w_o1, w_o2, w_i, w_j, w_set, w_lock;
+    // observed scan spread over several CTAs (k_scan_obs): running level (bit pattern of a positive double), the best
+    // arc of the finished slices (o_stat ... o_j; o_found: exact maximum without location) and the slices finished
+    unsigned long long o_level, o_found;
+    double o_stat, o_corner;
+    int o_q, o_key, o_i, o_j, o_set, o_lock, o_done;
     int w_tie;           // the maximum was attained in two pairs with EQUAL corner statistics: k_wobs_fin walks the pairs in the reference's
                          // own (std::sort) order to get the location (weighted.cuh wtmaxo_ordered)
     double w_delta;      // weighted hybrid: min weight of a (kmax+1)-marker arc / total weight (getmncwt, CBS.cpp:602-607)
@@ -329,8 +344,8 @@ struct Dev {
     // shuffle work lists by segment-length class (shuffle_class below)
     int n_shuf[SHUF_NCLS_MAX]; int* shuf_item[SHUF_NCLS_MAX]; int* shuf_prefix[SHUF_NCLS_MAX];
     int* shuf_p0[SHUF_NCLS_MAX];   // first permutation of the item that the entry covers
-    // work-stealing counters (reset every round): 0 global shuffle, 1 scan, 2 edge, 3 prefix, 4 hscan,
-    // 8+cls shared-memory shuffle of class cls
+    // work-stealing counters (reset every round): 0 global shuffle, 1 binary / weighted scan, 2 edge, 3 prefix, 4 hscan,
+    // 8+cls shared-memory shuffle of class cls, CTR_SCAN_* (k_scan_perm / k_scan_obs); ctr[CTR_OBS_SLICES] is written by the scheduler
     unsigned ctr[24];
     // ---- status -----------------------------------------------------------------------
     int done;
@@ -353,6 +368,8 @@ struct Dev {
     int api_n1, api_n2;         // tpermp: sizes of the two sides
     int shuf_cl2;     // segments of 65536..SHUF_CL2_MAX markers have their own class (cluster of 2 CTAs)
     int shuf_arena;   // segments > 65535 markers are shuffled by k_perm on 32-bit index arrays in the arena (fallback of k_shuffle_cluster)
+    int obs_slices;   // most CTAs per observed row (CBS_GPU_OBS_SLICES; 1: one CTA per row)
+    int obs_noloc;    // observed rows need the exact maximum only (cbs::tmaxp through the low-level API)
     int no_early;     // CBS_GPU_NO_EARLY=1: decision-mode scans never stop at the first rejecting arc (A/B switch)
 };
 
@@ -560,6 +577,9 @@ struct Sched {
         t.off_bin = bx ? t.off_bs + bs_stride(t.nb) : -1;
         arena_used += need;
         t.off_rej = rej_used; rej_used += 1;
+        t.o_level = 0; t.o_found = 0; t.o_set = 0; t.o_lock = 0; t.o_done = 0;
+        const unsigned ns = (unsigned)obs_slices(t.n, D.obs_slices);
+        if (ns > D.ctr[CTR_OBS_SLICES]) D.ctr[CTR_OBS_SLICES] = ns;
         D.prep_task[D.n_prep++] = idx;
         PermItem& it = D.items[D.n_items];
         it.task = idx; it.P = 1; it.obs = 1;

@@ -279,9 +279,9 @@ int smooth_device(cbs_gpu_ctx* c, const double* xin, const long long* goff, cons
     return CBS_GPU_OK;
 }
 
-// warps per scan CTA: the block and extrema tables are per CTA; take the CTA shape that keeps the most warps
-// resident on an SM
-bool pick_scan_warps(cbs_gpu_ctx* c, ScanLayout& lay, int* occ_out) {
+// warps per scan CTA of kernel `kern` (k_scan_perm / k_scan_obs): the block and extrema tables are per CTA; take the CTA
+// shape that keeps the most warps resident on an SM
+bool pick_scan_warps(cbs_gpu_ctx* c, ScanLayout& lay, int* occ_out, const void* kern) {
     int best_w = 0, best_res = 0, best_occ = 1;
     const int forced = (int)env_ll("CBS_GPU_SCAN_WARPS", 0);  // experiments only
     for (int w : {8, 4, 2, 1}) {
@@ -289,7 +289,7 @@ bool pick_scan_warps(cbs_gpu_ctx* c, ScanLayout& lay, int* occ_out) {
         lay.warps = w;
         if (lay.bytes() > c->smem_optin) continue;
         int occ = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_scan, w * 32, lay.bytes()) != cudaSuccess) { cudaGetLastError(); continue; }
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, w * 32, lay.bytes()) != cudaSuccess) { cudaGetLastError(); continue; }
         if (occ * w > best_res || (occ * w == best_res && w == 8)) { best_res = occ * w; best_w = w; best_occ = occ; }
     }
     if (!best_w) return false;
@@ -297,6 +297,13 @@ bool pick_scan_warps(cbs_gpu_ctx* c, ScanLayout& lay, int* occ_out) {
     if (occ_out) *occ_out = std::max(1, best_occ);
     return true;
 }
+// the scan of the round's observed rows or of its permutation rows; the counting instantiations only when D->profile is set
+void launch_scan(bool obs, bool prof, int grid, const ScanLayout& lay, cudaStream_t s, Dev* dD) {
+    const unsigned threads = (unsigned)lay.warps * 32;
+    if (obs) { if (prof) k_scan_obs<true><<<grid, threads, lay.bytes(), s>>>(dD, lay); else k_scan_obs<false><<<grid, threads, lay.bytes(), s>>>(dD, lay); }
+    else { if (prof) k_scan_perm<true><<<grid, threads, lay.bytes(), s>>>(dD, lay); else k_scan_perm<false><<<grid, threads, lay.bytes(), s>>>(dD, lay); }
+}
+int obs_slice_cap() { return (int)std::min<long long>(64, std::max<long long>(1, env_ll("CBS_GPU_OBS_SLICES", OBS_SLICES_MAX))); }
 
 // shared-memory shuffle classes (cbs_core.h): dynamic shared memory of a CTA = claim table + last[] of the longest segment
 size_t shuffle_smem_bytes(int cls) { return ((size_t)4 << shuffle_class_hbits(cls)) + (((size_t)shuffle_class_max(cls) + 2) * 2 + 15) / 16 * 16; }
@@ -560,6 +567,7 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     hD.profile = c->counting ? 1 : 0;
     hD.shuf_arena = 1;  // decided below (cluster shuffle available?) and patched on the device before the first round
     hD.no_early = env_ll("CBS_GPU_NO_EARLY", 0) ? 1 : 0;
+    hD.obs_slices = obs_slice_cap();
     if (weighted) {
         hD.w = c->wts.as<double>(); hD.rw = c->rw.as<double>(); hD.cw = c->cw.as<double>(); hD.ycur = c->ycur.as<double>();
         CUDA_TRY(c, cudaMemsetAsync(c->flag.p, 0, sizeof(int), st));
@@ -599,9 +607,13 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     ScanLayout lay;
     lay.nb_max = block_count((int)std::max<long long>(Nmax, 1)) + 2;
     lay.set_table(std::max<long long>(Nmax, 1));
-    int scan_occ = 1;
-    if (!pick_scan_warps(c, lay, &scan_occ)) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "segment too long for the scan kernel's shared memory");
-    const size_t scan_smem = lay.bytes();
+    int scan_occ = 1, obs_occ = 1;
+    ScanLayout lay_obs = lay;
+    if (!pick_scan_warps(c, lay, &scan_occ, (const void*)k_scan_perm<false>) ||
+        !pick_scan_warps(c, lay_obs, &obs_occ, (const void*)k_scan_obs<false>))
+        return fail(c, CBS_GPU_ERR_UNSUPPORTED, "segment too long for the scan kernel's shared memory");
+    const bool scan_prof = hD.profile != 0;
+    const int obs_grid = c->sm_count * obs_occ;
     const size_t wscan_smem = ((sizeof(WScanSmem) + 15) & ~(size_t)15) + (size_t)lay.nb_max * (2 * sizeof(double) + 3 * sizeof(int)) + 16;
     const int scan_grid = c->sm_count * scan_occ;
     const size_t bscan_smem = ((sizeof(BinSmem) + 15) & ~(size_t)15) + (size_t)lay.nb_max * (2 * sizeof(double) + 3 * sizeof(int)) + 16;
@@ -661,14 +673,18 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     auto enqueue_round = [&]() {
         bool ahead_pending = false;
         // One round.  Dependencies: everything after k_sched; shuffles after the generator;
-        // k_prefix after the shuffles; k_scan after k_prefix and k_prep; next k_sched after all.
-        //   main : sched, gen, [shuffle classes], prefix, scan
-        //   side0: prep            side1: edgeprep, edgeperm
+        // k_prefix after the shuffles; k_scan_perm after k_prefix; k_scan_obs after k_prep; next k_sched after all.
+        // A task's permutations are planned in a later round than its observed scan (Sched::step), so neither scan
+        // of a round reads what the other writes, and the observed scans run beside the shuffles.
+        //   main : sched, gen, [shuffle classes], prefix, scan_perm
+        //   side0: prep, scan_obs  side1: edgeprep, edgeperm
         //   side2, side3: other shuffle classes      side4: shuffle of segments > 65535 markers
         { LaunchTimer t(c, K_SCHED); k_sched<<<1, 256, 0, st>>>(dD, c->d_done, loop_handle, looped); }
         cudaEventRecord(c->ev_sched, st);
         cudaStreamWaitEvent(side[0], c->ev_sched, 0);
         { LaunchTimer t(c, K_PREP, side[0]); k_tables<<<dim3(16, 64), 256, 0, side[0]>>>(dD); if (weighted) { k_wprep<<<c->sm_count * 8, 32, 0, side[0]>>>(dD); k_wtables<<<c->sm_count * 2, 256, 0, side[0]>>>(dD); c->launches++; if (p->hybrid) { k_wdelta<<<c->sm_count * 2, 32, 0, side[0]>>>(dD); c->launches++; } } else k_prep<<<c->sm_count * 8, 32, 0, side[0]>>>(dD); c->launches++; }
+        const bool scan_split = !weighted && !p->ibin;
+        if (scan_split) { LaunchTimer t(c, K_SCAN, side[0]); launch_scan(true, scan_prof, obs_grid, lay_obs, side[0], dD); }
         cudaEventRecord(c->ev_side[0], side[0]);
         cudaStreamWaitEvent(side[1], c->ev_sched, 0);
         { LaunchTimer t(c, K_EDGEPREP, side[1]); if (weighted) k_wedgeprep<<<c->sm_count * 4, 32, 0, side[1]>>>(dD); else k_edgeprep<<<c->sm_count * 4, 32, 0, side[1]>>>(dD); }
@@ -718,7 +734,7 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
         }
         for (int k = 2; k < 5; ++k) if (used_side[k]) { cudaEventRecord(c->ev_side[k], side[k]); cudaStreamWaitEvent(st, c->ev_side[k], 0); }
         { LaunchTimer t(c, K_PREFIX); if (weighted && p->hybrid) { k_wssq<<<c->sm_count * 8, 128, 0, st>>>(dD); c->launches++; } if (weighted) k_chain<true><<<c->sm_count * chain_occ, 32 * (1 + CP_STAT_WARPS), 0, st>>>(dD); else k_chain<false><<<c->sm_count * chain_occ, 32 * (1 + CP_STAT_WARPS), 0, st>>>(dD); }
-        cudaStreamWaitEvent(st, c->ev_side[0], 0);
+        if (!scan_split) cudaStreamWaitEvent(st, c->ev_side[0], 0);
         { LaunchTimer t(c, K_SCAN);
           if (weighted) {
               k_wscan<1><<<c->sm_count * 4, 256, wscan_smem, st>>>(dD, lay.nb_max);   // observed rows, sliced over CTAs
@@ -727,7 +743,8 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
               c->launches += 2;
           }
           else if (p->ibin) k_scan_binary<<<c->sm_count * 4, 256, bscan_smem, st>>>(dD, lay.nb_max);
-          else k_scan<<<scan_grid, lay.warps * 32, scan_smem, st>>>(dD, lay); }
+          else launch_scan(false, scan_prof, scan_grid, lay, st, dD); }
+        if (scan_split) cudaStreamWaitEvent(st, c->ev_side[0], 0);  // the tail probabilities read the observed statistics
         if (p->hybrid) {
             if (weighted) k_whscan<<<c->sm_count * 4, 256, 0, st>>>(dD); else k_hscan<<<c->sm_count * 4, 256, 0, st>>>(dD);
             k_tailp_terms<<<c->sm_count * 8, 128, 0, st>>>(dD, c->tailp.as<double>());
@@ -747,8 +764,8 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
         const int flags[7] = {weighted ? 1 : 0, mt ? 1 : 0, shared_stream ? 1 : 0, hD.jump_polys ? 1 : 0, p->hybrid ? 1 : 0, l2_shuffle_on ? 1 : 0,
                               p->ibin ? 1 : 0};
         KEY_POD(dD); KEY_POD(st); KEY_POD(flags); KEY_POD(n_chains); KEY_POD(shuf_occ); KEY_POD(shuf_on); KEY_POD(cl_R); KEY_POD(cl_grid);
-        KEY_POD(cl2_grid); KEY_POD(cl_smem); KEY_POD(cl2_smem); KEY_POD(chain_occ); KEY_POD(scan_grid); KEY_POD(scan_smem);
-        KEY_POD(wscan_smem); KEY_POD(bscan_smem); KEY_POD(lay);
+        KEY_POD(cl2_grid); KEY_POD(cl_smem); KEY_POD(cl2_smem); KEY_POD(chain_occ); KEY_POD(scan_grid); KEY_POD(obs_grid); KEY_POD(scan_prof);
+        KEY_POD(wscan_smem); KEY_POD(bscan_smem); KEY_POD(lay); KEY_POD(lay_obs);
         const void* tailp_ptr = c->tailp.p; KEY_POD(tailp_ptr);
 #undef KEY_POD
         if (c->call_exec && key == c->call_key) {
@@ -1006,7 +1023,8 @@ int cbs_gpu_create(const int* device_ids, int ndev, cbs_gpu_ctx** out) {
     // function attributes are process-wide per device: set them once to the device maximum, never per call
     // (concurrent lanes with different needs would otherwise shrink each other's limit)
     const int mx = (int)c->smem_optin;
-    if (!set_max_smem(k_scan, mx) ||
+    if (!set_max_smem(k_scan_perm<false>, mx) || !set_max_smem(k_scan_perm<true>, mx) || !set_max_smem(k_scan_obs<false>, mx) ||
+        !set_max_smem(k_scan_obs<true>, mx) ||
         !set_max_smem(k_shuffle<128, 2, true>, mx) || !set_max_smem(k_shuffle<256, 2, true>, mx) || !set_max_smem(k_shuffle<512, 2, true>, mx) ||
         !set_max_smem(k_shuffle<1024, 2, true>, mx) || !set_max_smem(k_shuffle<128, 2, false>, mx) || !set_max_smem(k_shuffle<256, 2, false>, mx) ||
         !set_max_smem(k_shuffle<512, 2, false>, mx) || !set_max_smem(k_shuffle<1024, 2, false>, mx) ||
@@ -1168,6 +1186,8 @@ static int run_raw_scan(cbs_gpu_ctx* c, const double* xh, int n, int count, doub
     hD.arena = c->arena.as<double>(); hD.arena_cap = per * count; hD.rej = c->rej.as<int>(); hD.rej_cap = count;
     hD.n_prep = count; hD.prep_task = c->prep_task.as<int>();
     hD.n_items = count; hD.items = c->items.as<PermItem>(); hD.item_prefix = c->item_prefix.as<int>();
+    hD.obs_slices = obs_slice_cap(); hD.obs_noloc = obs == 2 ? 1 : 0;
+    hD.ctr[CTR_OBS_SLICES] = (unsigned)obs_slices(n, hD.obs_slices);
     CUDA_TRY(c, cudaMemcpyAsync(c->x.p, xh, sizeof(double) * (size_t)N, cudaMemcpyHostToDevice, st));
     CUDA_TRY(c, cudaMemcpyAsync(c->unit_off.p, off.data(), sizeof(long long) * off.size(), cudaMemcpyHostToDevice, st));
     CUDA_TRY(c, cudaMemcpyAsync(c->tasks.p, tasks.data(), sizeof(Task) * tasks.size(), cudaMemcpyHostToDevice, st));
@@ -1178,11 +1198,12 @@ static int run_raw_scan(cbs_gpu_ctx* c, const double* xh, int n, int count, doub
     ScanLayout lay;
     lay.nb_max = nb + 2;
     lay.set_table(n);
-    if (!pick_scan_warps(c, lay, nullptr)) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "vector too long for the scan kernel's shared memory");
+    int occ = 1;
+    if (!pick_scan_warps(c, lay, &occ, (const void*)k_scan_obs<false>)) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "vector too long for the scan kernel's shared memory");
     Dev* dD = c->dev.as<Dev>();
     k_tables<<<dim3(16, 64), 256, 0, st>>>(dD);
     k_prep<<<std::min(count, c->sm_count * 8), 32, 0, st>>>(dD);
-    k_scan<<<std::min(count, c->sm_count * 2), lay.warps * 32, lay.bytes(), st>>>(dD, lay);
+    launch_scan(true, false, (int)std::min<long long>((long long)count * hD.ctr[CTR_OBS_SLICES], (long long)c->sm_count * occ), lay, st, dD);
     CUDA_TRY(c, cudaGetLastError());
     tasks_out.resize((size_t)count);
     CUDA_TRY(c, cudaMemcpyAsync(tasks_out.data(), c->tasks.p, sizeof(Task) * tasks_out.size(), cudaMemcpyDeviceToHost, st));
