@@ -371,6 +371,7 @@ struct Dev {
     int obs_slices;   // most CTAs per observed row (CBS_GPU_OBS_SLICES; 1: one CTA per row)
     int obs_noloc;    // observed rows need the exact maximum only (cbs::tmaxp through the low-level API)
     int no_early;     // CBS_GPU_NO_EARLY=1: decision-mode scans never stop at the first rejecting arc (A/B switch)
+    int err_unit, err_lo, err_hi;  // ERR_SELF_SPLIT: the segment whose decision would have re-created it
 };
 
 // shared MT stream (ring + mirror): store one word / linear read pointer for a run of <= stream_mirror positions
@@ -385,7 +386,8 @@ CBS_HD const uint64_t* draw_window(const Dev& D, long long off) {
     return D.shared_stream ? D.stream + (off & D.stream_mask) : D.draws[D.round & 1] + off;
 }
 
-enum { ERR_TASK_CAP = 101, ERR_SEG_CAP = 102, ERR_ARENA = 103, ERR_SPLIT_CAP = 104, ERR_INTERNAL = 105, ERR_STALL = 106, ERR_STREAM_CAP = 107 };
+enum { ERR_TASK_CAP = 101, ERR_SEG_CAP = 102, ERR_ARENA = 103, ERR_SPLIT_CAP = 104, ERR_INTERNAL = 105, ERR_STALL = 106, ERR_STREAM_CAP = 107,
+       ERR_SELF_SPLIT = 108 };
 
 // Shuffle classes (shuffle.cuh).  0..5: one CTA per permutation, last[] (16 bit per marker) and the claim table in
 // shared memory; the class fixes the CTA size and the array size, hence how many permutations an SM holds at once
@@ -519,6 +521,13 @@ struct Sched {
         const int c1 = lo + icpt0 + 1;
         const int c2 = (ncpt == 2) ? lo + icpt1 + 1 : hi;
         free_task(idx);
+        // A child equal to its parent would be decided again with the same outcome, forever.  Only weighted CBS can get
+        // here: a weight that carries nearly all of the total leaves cw flat, an arc of weight 0 has an infinite
+        // statistic, ostat is NaN and the change point falls on the segment's last marker (DESIGN §2).
+        if (c1 == hi || (c1 == lo && c2 == hi) || c2 == lo) {
+            D.error = ERR_SELF_SPLIT; D.err_unit = unit; D.err_lo = lo; D.err_hi = hi;
+            return;
+        }
         int kids[3]; int nk = 0;
         kids[nk++] = new_task(unit, lo, c1);
         if (ncpt == 2) kids[nk++] = new_task(unit, c1, c2);

@@ -852,6 +852,10 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
         case ERR_STALL: return fail(c, CBS_GPU_ERR_CUDA, "scheduler stalled: live segments but no work could be planned");
         case ERR_STREAM_CAP: return fail(c, CBS_GPU_ERR_CAPACITY, "MT stream window smaller than one permutation (raise CBS_GPU_STREAM_MB)");
         case ERR_ARENA: return fail(c, CBS_GPU_ERR_OOM, "permutation arena too small for one segment (raise CBS_GPU_ARENA_MB)");
+        case ERR_SELF_SPLIT:
+            return fail(c, CBS_GPU_ERR_UNSUPPORTED, "unit " + std::to_string(hD.err_unit) + ", segment [" + std::to_string(hD.err_lo) + ", " +
+                        std::to_string(hD.err_hi) + "): the split decision would re-create the segment (weights so uneven that "
+                        "the statistic is not finite); the reference would not terminate");
         default: return fail(c, CBS_GPU_ERR_CUDA, "internal scheduler error " + std::to_string(hD.error));
         }
     }

@@ -333,7 +333,9 @@ __device__ __forceinline__ void warc_eval(const WPair& p, int q, WScanSmem* sm, 
             atomicMax(&sm->found, (unsigned long long)__double_as_longlong(v));
             atomicMax(&sm->level, (unsigned long long)__double_as_longlong(v));
             if (sm->gfound) { atomicMax(sm->gfound, (unsigned long long)__double_as_longlong(v)); atomicMax(sm->glevel, (unsigned long long)__double_as_longlong(v)); }
-            if (v >= sm->rej_at) sm->decided = 1;
+            // rej_at is +inf when the early decision is off; an infinite arc (weight 0, only where cw is not strictly
+            // increasing) must not match it: the reference's statistic is then NaN, which never rejects (CBS.cpp:933)
+            if (v >= sm->rej_at && sm->rej_at < __longlong_as_double(0x7ff0000000000000LL)) sm->decided = 1;
         }
     }
 }
@@ -599,7 +601,8 @@ __global__ void __launch_bounds__(256) k_wscan(Dev* D, int nb_max) {
                 if (!(ci > cp) || isinf(ci)) bad = 1;
             }
             bad = __syncthreads_or(bad);
-            if (tid == 0) { t.w_ok = bad ? 0 : 1; t.tmaxi = fi; t.tmaxj = fj; }  // location: the seed arc unless MODE 2 finds better
+            // location: the seed arc unless MODE 2 finds better; without spread the reference reports it unshifted (:642-645)
+            if (tid == 0) { t.w_ok = bad ? 0 : 1; t.tmaxi = psdiff > 0.0 ? fi : fi + 1; t.tmaxj = psdiff > 0.0 ? fj : fj + 1; }
         }
         if (psdiff > 0.0) {  // else CBS.cpp:642-645
             r.psrn = r.cw[n - 1];

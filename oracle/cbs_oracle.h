@@ -140,12 +140,33 @@ double orc_wtmaxp(const double* px, const double* w, const double* cw, int n, in
 void orc_wxperm(const double* x, const double* rw, int n, double* px, orc_rng* rng);
 double orc_wtpermp(int n1, int n2, int n, const double* x, const double* w, const double* rw, int nperm, orc_rng* rng,
                    double* scratch);
-/* segments, or -needed-16 if cap is too small, or -3 when the weighted hybrid method would be reached */
+void orc_getmncwt(const double* cw, int n, int k, double* mn, double* delta);
+double orc_hwtmaxp(const double* px, const double* w, const double* cw, const double* mn, int n, int k, int al0);
+/* one wfindcpt decision on x as given (centred, with the caller's tss); rw = sqrt(w) and cw are derived from w as
+ * segment_weighted derives them */
+orc_cpt orc_wfindcpt(const double* x, const double* w, int n, double tss, int nperm, double cpval, int hybrid, int al0,
+                     int hk, int ngrid, double tol, orc_rng* rng);
+/* segments, or -needed-16 if cap is too small, or -4 (ORC_W_SELF_SPLIT) when a decision would re-create its own segment.
+ *
+ * -4 is the one place where this restatement knowingly departs from the reference.  When one weight carries nearly all of
+ * the total, cw is not strictly increasing, an arc of weight 0 has an infinite statistic and ostat becomes NaN; no
+ * permutation rejects and the change point lands on the segment's last marker, so [lo,hi) splits into [lo,hi) and
+ * [hi,hi).  The reference (CBS.cpp:996-1004) then tests [lo,hi) again, with the same outcome, forever.  Here the driver
+ * stops at the first decision that would re-create its own segment and returns -4; the split log ends with that decision.
+ * The _log forms also fill a split log in processing order, as orc_segment does. */
 int orc_segment_weighted(const double* x, const double* w, int n, const orc_seg_opts* o, orc_rng* rng, uint64_t seed,
                          uint64_t unit_id, int cap, int* lengths, double* means);
+int orc_segment_weighted_log(const double* x, const double* w, int n, const orc_seg_opts* o, orc_rng* rng, uint64_t seed,
+                             uint64_t unit_id, int cap, int* lengths, double* means, orc_split_rec* log, int log_cap,
+                             int* log_n);
+/* total segments, -1 if cap is too small, -4 as above */
 int64_t orc_segment_weighted_units(const double* values, const double* weights, const int64_t* unit_off,
                                    const uint64_t* unit_ids, int n_units, const orc_cohort_opts* o, int64_t cap,
                                    int* seg_count, int* lengths, double* means, uint64_t* draws_out);
+int64_t orc_segment_weighted_units_log(const double* values, const double* weights, const int64_t* unit_off,
+                                       const uint64_t* unit_ids, int n_units, const orc_cohort_opts* o, int64_t cap,
+                                       int* seg_count, int* lengths, double* means, uint64_t* draws_out,
+                                       orc_split_rec* log, int64_t log_cap, int64_t* log_n, int* log_unit);
 
 #ifdef __cplusplus
 }

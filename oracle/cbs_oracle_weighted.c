@@ -15,6 +15,7 @@
  */
 
 #define ORC_W_UNSUPPORTED (-3) /* kept for the ABI of the python wrapper; no longer returned */
+#define ORC_W_SELF_SPLIT (-4)  /* see cbs_oracle.h: a decision that would re-create its own segment */
 
 /* ---- wtmaxo / wtmaxp ------------------------------------------------------------ */
 typedef struct {
@@ -373,9 +374,31 @@ static orc_cpt orc_wfndcpt(const double* x, int n, double tss, const double* w, 
     return r;
 }
 
+/* wfindcpt on a segment as given (the low-level entry): rw and cw derived from w as segment_weighted does (:1056-1066) */
+orc_cpt orc_wfindcpt(const double* x, const double* w, int n, double tss, int nperm, double cpval, int hybrid, int al0,
+                     int hk, int ngrid, double tol, orc_rng* rng) {
+    const size_t nn = (size_t)(n > 0 ? n : 1);
+    double* rw = (double*)malloc(sizeof(double) * nn);
+    double* cw = (double*)malloc(sizeof(double) * nn);
+    double wsum = 0.0;
+    for (int i = 0; i < n; ++i) { rw[i] = sqrt(w[i]); wsum += w[i]; }
+    const double scale = sqrt(wsum);
+    double run = 0.0;
+    for (int i = 0; i < n; ++i) { run += w[i]; cw[i] = run / scale; }
+    const orc_cpt r = orc_wfndcpt(x, n, tss, w, rw, cw, nperm, cpval, hybrid, al0, hk, ngrid, tol, rng);
+    free(rw); free(cw);
+    return r;
+}
+
 /* ---- recursive driver (segment_weighted :1026-1099) ---------------------------------- */
 int orc_segment_weighted(const double* x, const double* w, int n, const orc_seg_opts* o, orc_rng* rng, uint64_t seed,
                          uint64_t unit_id, int cap, int* lengths, double* means) {
+    return orc_segment_weighted_log(x, w, n, o, rng, seed, unit_id, cap, lengths, means, NULL, 0, NULL);
+}
+
+int orc_segment_weighted_log(const double* x, const double* w, int n, const orc_seg_opts* o, orc_rng* rng, uint64_t seed,
+                             uint64_t unit_id, int cap, int* lengths, double* means, orc_split_rec* log, int log_cap,
+                             int* log_n) {
     int ends_cap = 64, nends = 2;
     int* ends = (int*)malloc(sizeof(int) * (size_t)ends_cap);
     ends[0] = 0; ends[1] = n;
@@ -385,12 +408,13 @@ int orc_segment_weighted(const double* x, const double* w, int n, const orc_seg_
     double* cur = (double*)malloc(sizeof(double) * nn);
     double* rw = (double*)malloc(sizeof(double) * nn);
     double* cw = (double*)malloc(sizeof(double) * nn);
-    int unsupported = 0;
+    int unsupported = 0, self_split = 0, nlog = 0;
     while (nends > 1) {
         const int k = nends - 1;
         const int lo = ends[k - 1], hi = ends[k], len = hi - lo;
         orc_cpt z;
         memset(&z, 0, sizeof(z));
+        int called = 0;
         if (len >= 2 * o->min_width) {
             const int use_hybrid = o->hybrid && (o->nmin < len);
             int flat = 1;
@@ -409,7 +433,20 @@ int orc_segment_weighted(const double* x, const double* w, int n, const orc_seg_
                 }
                 orc_rng_set_task(rng, seed, unit_id, (uint32_t)lo, (uint32_t)hi);
                 z = orc_wfndcpt(cur, len, wxx, ws, rw, cw, o->nperm, o->alpha, use_hybrid, o->min_width, o->kmax, 100, o->tol, rng);
+                called = 1;
             }
+        }
+        if (log && nlog < log_cap) {
+            orc_split_rec* e = &log[nlog];
+            e->lo = lo; e->hi = hi; e->ostat = z.ostat; e->iseg0 = z.iseg[0]; e->iseg1 = z.iseg[1];
+            e->ncpt = z.ncpt; e->icpt0 = z.icpt[0]; e->icpt1 = z.icpt[1];
+            e->perms_run = z.perms_run; e->nrej = z.nrej; e->exit_code = z.exit_code; e->called = called;
+            e->edge_p0 = called ? z.edge_p[0] : -1.0; e->edge_p1 = called ? z.edge_p[1] : -1.0;
+        }
+        ++nlog;
+        if (z.ncpt > 0) {  /* children [lo,c1) [c1,c2) [c2,hi): one equal to [lo,hi) would be tested again, forever */
+            const int c1 = lo + z.icpt[0] + 1, c2 = (z.ncpt == 2) ? lo + z.icpt[1] + 1 : hi;
+            if (c1 == hi || (c1 == lo && c2 == hi) || c2 == lo) { self_split = 1; break; }
         }
         if (nends + 2 > ends_cap) { ends_cap *= 2; ends = (int*)realloc(ends, sizeof(int) * (size_t)ends_cap); }
         if (z.ncpt == 0) {
@@ -427,8 +464,10 @@ int orc_segment_weighted(const double* x, const double* w, int n, const orc_seg_
             nends += 2;
         }
     }
+    if (log_n) *log_n = nlog;
     int ret;
     if (unsupported) ret = ORC_W_UNSUPPORTED;
+    else if (self_split) ret = ORC_W_SELF_SPLIT;
     else {
         int nseg = ndone;
         int* lseg = (int*)malloc(sizeof(int) * (size_t)(nseg > 0 ? nseg + 2 : 2));
@@ -454,13 +493,22 @@ int orc_segment_weighted(const double* x, const double* w, int n, const orc_seg_
 }
 
 /* cohort form: every unit through orc_segment_weighted; rng handling as orc_segment_units.
- * Returns total segments, -1 if cap too small, -3 unsupported (weighted hybrid). */
+ * Returns total segments, -1 if cap too small, -3 unsupported (weighted hybrid), -4 self split. */
 int64_t orc_segment_weighted_units(const double* values, const double* weights, const int64_t* unit_off,
                                    const uint64_t* unit_ids, int n_units, const orc_cohort_opts* o, int64_t cap,
                                    int* seg_count, int* lengths, double* means, uint64_t* draws_out) {
+    return orc_segment_weighted_units_log(values, weights, unit_off, unit_ids, n_units, o, cap, seg_count, lengths, means,
+                                          draws_out, NULL, 0, NULL, NULL);
+}
+
+int64_t orc_segment_weighted_units_log(const double* values, const double* weights, const int64_t* unit_off,
+                                       const uint64_t* unit_ids, int n_units, const orc_cohort_opts* o, int64_t cap,
+                                       int* seg_count, int* lengths, double* means, uint64_t* draws_out,
+                                       orc_split_rec* log, int64_t log_cap, int64_t* log_n, int* log_unit) {
     orc_rng rng;
     if (o->rng_kind == 0) orc_rng_seed_mt(&rng, o->seed); else orc_rng_seed_philox(&rng, o->seed);
-    int64_t total = 0;
+    int64_t total = 0, nlog = 0;
+    if (log_n) *log_n = 0;
     for (int u = 0; u < n_units; ++u) {
         const int64_t lo = unit_off[u], hi = unit_off[u + 1];
         seg_count[u] = 0;
@@ -470,10 +518,17 @@ int64_t orc_segment_weighted_units(const double* values, const double* weights, 
         if (o->rng_kind == 0 && !o->chain) orc_rng_seed_mt(&rng, o->seed);
         const uint64_t d0 = rng.draws;
         const int64_t room = cap - total;
-        const int k = orc_segment_weighted(values + lo, weights + lo, n, &o->seg, &rng, o->seed,
-                                           unit_ids ? unit_ids[u] : (uint64_t)u,
-                                           room > 2147483647 ? 2147483647 : (int)room, lengths + total, means + total);
+        int this_log = 0;
+        const int k = orc_segment_weighted_log(values + lo, weights + lo, n, &o->seg, &rng, o->seed,
+                                               unit_ids ? unit_ids[u] : (uint64_t)u,
+                                               room > 2147483647 ? 2147483647 : (int)room, lengths + total, means + total,
+                                               log ? log + nlog : NULL,
+                                               (int)((log_cap - nlog) > 2147483647 ? 2147483647 : (log_cap - nlog)), &this_log);
+        if (log_unit) for (int i = 0; i < this_log && nlog + i < log_cap; ++i) log_unit[nlog + i] = u;
+        nlog += this_log;
+        if (log_n) *log_n = nlog;
         if (k == ORC_W_UNSUPPORTED) return -3;
+        if (k == ORC_W_SELF_SPLIT) return -4;
         if (k < 0) return -1;
         seg_count[u] = k;
         total += k;

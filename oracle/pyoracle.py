@@ -118,6 +118,18 @@ class OrcCohortOpts(C.Structure):
     ]
 
 
+class SplitIntoItself(RuntimeError):
+    """The weighted driver reached a decision that would re-create its own segment (oracle/cbs_oracle.h, code -4): the
+    reference would test that segment again forever."""
+
+
+def weight_tables(w):
+    """rw = sqrt(w) and cw = cumsum(w)/sqrt(sum w), summed in order as cbs::segment_weighted (and the device) does."""
+    w = np.ascontiguousarray(w, dtype=np.float64)
+    csum = np.cumsum(w)  # sequential
+    return np.sqrt(w), csum / np.sqrt(csum[-1])
+
+
 @dataclass
 class SegParams:
     """Mirror of the `cna segment` options (src/cna_segment.hpp:67-79)."""
@@ -207,6 +219,24 @@ class Oracle:
         L.orc_segment_weighted_units.argtypes = [c_double_p, c_double_p, c_i64_p, c_u64_p, C.c_int,
                                                  C.POINTER(OrcCohortOpts), C.c_int64, c_int_p, c_int_p, c_double_p,
                                                  c_u64_p]
+        L.orc_segment_weighted_units_log.restype = C.c_int64
+        L.orc_segment_weighted_units_log.argtypes = [c_double_p, c_double_p, c_i64_p, c_u64_p, C.c_int,
+                                                     C.POINTER(OrcCohortOpts), C.c_int64, c_int_p, c_int_p, c_double_p,
+                                                     c_u64_p, C.POINTER(OrcSplitRec), C.c_int64, c_i64_p, c_int_p]
+        L.orc_wtmaxo.restype = OrcTmax
+        L.orc_wtmaxo.argtypes = [c_double_p, c_double_p, c_double_p, C.c_int, C.c_double, C.c_int]
+        L.orc_wtmaxp.restype = C.c_double
+        L.orc_wtmaxp.argtypes = [c_double_p, c_double_p, c_double_p, C.c_int, C.c_int]
+        L.orc_wxperm.argtypes = [c_double_p, c_double_p, C.c_int, c_double_p, C.POINTER(OrcRng)]
+        L.orc_wtpermp.restype = C.c_double
+        L.orc_wtpermp.argtypes = [C.c_int, C.c_int, C.c_int, c_double_p, c_double_p, c_double_p, C.c_int,
+                                  C.POINTER(OrcRng), c_double_p]
+        L.orc_getmncwt.argtypes = [c_double_p, C.c_int, C.c_int, c_double_p, c_double_p]
+        L.orc_hwtmaxp.restype = C.c_double
+        L.orc_hwtmaxp.argtypes = [c_double_p, c_double_p, c_double_p, c_double_p, C.c_int, C.c_int, C.c_int]
+        L.orc_wfindcpt.restype = OrcCpt
+        L.orc_wfindcpt.argtypes = [c_double_p, c_double_p, C.c_int, C.c_double, C.c_int, C.c_double, C.c_int, C.c_int,
+                                   C.c_int, C.c_int, C.c_double, C.POINTER(OrcRng)]
 
     # -- rng ---------------------------------------------------------------
     def rng_mt(self, seed: int) -> OrcRng:
@@ -311,7 +341,9 @@ class Oracle:
         assert k >= 0, k
         return lengths[:k].copy(), means[:k].copy()
 
-    def segment_weighted_units(self, values, weights, unit_off, p: SegParams, unit_ids=None):
+    def segment_weighted_units(self, values, weights, unit_off, p: SegParams, unit_ids=None, want_log=False):
+        """Weighted segmentation of every unit; with want_log, also the split log as segment_units returns it.
+        Raises SplitIntoItself where the reference would not terminate."""
         values = np.ascontiguousarray(values, dtype=np.float64)
         weights = np.ascontiguousarray(weights, dtype=np.float64)
         unit_off = np.ascontiguousarray(unit_off, dtype=np.int64)
@@ -322,15 +354,76 @@ class Oracle:
         means = np.zeros(cap, dtype=np.float64)
         draws = np.zeros(n_units, dtype=np.uint64)
         uid = None if unit_ids is None else np.ascontiguousarray(unit_ids, dtype=np.uint64)
+        log_cap = (4 * cap) if want_log else 0
+        log = (OrcSplitRec * max(1, log_cap))()
+        log_unit = np.zeros(max(1, log_cap), dtype=np.int32)
+        nlog = C.c_int64(0)
         opts = p.cohort_opts()
-        tot = self.lib.orc_segment_weighted_units(
+        tot = self.lib.orc_segment_weighted_units_log(
             _dp(values), _dp(weights), unit_off.ctypes.data_as(c_i64_p),
             uid.ctypes.data_as(c_u64_p) if uid is not None else None, n_units, C.byref(opts), cap, _ip(seg_count),
-            _ip(lengths), _dp(means), draws.ctypes.data_as(c_u64_p))
+            _ip(lengths), _dp(means), draws.ctypes.data_as(c_u64_p), log if want_log else None, log_cap,
+            C.byref(nlog), _ip(log_unit))
         if tot == -3:
             raise NotImplementedError("weighted hybrid method is not restated")
+        if tot == -4:
+            last = log[nlog.value - 1] if want_log and nlog.value else None
+            raise SplitIntoItself("a weighted split decision would re-create its own segment"
+                                  + (f" (unit {log_unit[nlog.value - 1]}, [{last.lo}, {last.hi}))" if last else ""))
         assert tot >= 0, tot
-        return dict(seg_count=seg_count, lengths=lengths[:tot].copy(), means=means[:tot].copy(), draws=draws)
+        res = dict(seg_count=seg_count, lengths=lengths[:tot].copy(), means=means[:tot].copy(), draws=draws)
+        if want_log:
+            res["log"] = [(int(log_unit[i]), log[i]) for i in range(nlog.value)]
+        return res
+
+    # -- weighted low-level functions (CBS.cpp:538-957); rw and cw derived from w by weight_tables() ----------------
+    def wtmaxo(self, x, w, tss, al0=2):
+        x = np.ascontiguousarray(x, dtype=np.float64)
+        w = np.ascontiguousarray(w, dtype=np.float64)
+        _, cw = weight_tables(w)
+        r = self.lib.orc_wtmaxo(_dp(x), _dp(w), _dp(cw), len(x), tss, al0)
+        return r.stat, r.start, r.end
+
+    def wtmaxp(self, px, w, al0=2):
+        px = np.ascontiguousarray(px, dtype=np.float64)
+        w = np.ascontiguousarray(w, dtype=np.float64)
+        _, cw = weight_tables(w)
+        return self.lib.orc_wtmaxp(_dp(px), _dp(w), _dp(cw), len(px), al0)
+
+    def wxperm(self, x, w, rng: OrcRng):
+        x = np.ascontiguousarray(x, dtype=np.float64)
+        rw, _ = weight_tables(w)
+        px = np.empty_like(x)
+        self.lib.orc_wxperm(_dp(x), _dp(rw), len(x), _dp(px), C.byref(rng))
+        return px
+
+    def wtpermp(self, n1, n2, x, w, nperm, rng: OrcRng):
+        x = np.ascontiguousarray(x, dtype=np.float64)
+        w = np.ascontiguousarray(w, dtype=np.float64)
+        rw, _ = weight_tables(w)
+        scratch = np.empty(max(1, n1 + n2), dtype=np.float64)
+        return self.lib.orc_wtpermp(n1, n2, n1 + n2, _dp(x), _dp(w), _dp(rw), nperm, C.byref(rng), _dp(scratch))
+
+    def getmncwt(self, w, k):
+        """(mn[0..k], delta) of the weighted hybrid method"""
+        _, cw = weight_tables(w)
+        mn = np.zeros(k + 1, dtype=np.float64)
+        delta = C.c_double()
+        self.lib.orc_getmncwt(_dp(cw), len(cw), k, _dp(mn), C.byref(delta))
+        return mn, delta.value
+
+    def hwtmaxp(self, px, w, k, al0=2):
+        px = np.ascontiguousarray(px, dtype=np.float64)
+        w = np.ascontiguousarray(w, dtype=np.float64)
+        _, cw = weight_tables(w)
+        mn, _ = self.getmncwt(w, k)
+        return self.lib.orc_hwtmaxp(_dp(px), _dp(w), _dp(cw), _dp(mn), len(px), k, al0)
+
+    def wfindcpt(self, x, w, tss, nperm, cpval, rng: OrcRng, hybrid=False, al0=2, hk=25, ngrid=100, tol=1e-6) -> OrcCpt:
+        x = np.ascontiguousarray(x, dtype=np.float64)
+        w = np.ascontiguousarray(w, dtype=np.float64)
+        return self.lib.orc_wfindcpt(_dp(x), _dp(w), len(x), tss, nperm, cpval, int(hybrid), al0, hk, ngrid, tol,
+                                     C.byref(rng))
 
     def smooth(self, values, chrom, smooth_region=10, outlier_sd_scale=4.0, smooth_sd_scale=2.0, trim=0.025):
         values = np.ascontiguousarray(values, dtype=np.float64)

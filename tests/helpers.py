@@ -1,4 +1,6 @@
 """Shared input builders for the parity tests."""
+import ctypes as C
+
 import numpy as np
 
 
@@ -43,3 +45,37 @@ def equal_arrays(got, want):
     if isinstance(want, Digest):
         return want.matches(got)
     return np.array_equal(got, want)
+
+
+def weighted_centre(x, w):
+    """centred segment and weighted tss, each sum taken in order as segment_weighted does (CBS.cpp:1053-1063)"""
+    avg = np.cumsum(w * x)[-1] / np.cumsum(w)[-1]
+    cur = x - avg
+    return cur, float(np.cumsum(w * cur * cur)[-1])
+
+
+def untemper(y):
+    """mt19937_64 output -> the raw state word it was tempered from"""
+    y = int(y)
+    M = (1 << 64) - 1
+    y ^= y >> 43
+    y ^= (y << 37) & 0xFFF7EEE000000000 & M
+    z = y
+    for _ in range(4):
+        z = y ^ ((z << 17) & 0x71D67FFFEDA60000 & M)
+    y = z
+    z = y
+    for _ in range(3):
+        z = y ^ ((z >> 29) & 0x5555555555555555)
+    return z
+
+
+def engine_after(oracle, seed, skip):
+    """an oracle engine that has already handed out `skip` draws, and the same engine as its next 312 raw words (the
+    caller-owned engine state of the single-call entry points)"""
+    eng = oracle.rng_mt(seed)
+    oracle.lib.orc_rng_discard(C.byref(eng), skip)
+    probe = oracle.rng_mt(seed)
+    oracle.lib.orc_rng_discard(C.byref(probe), skip)
+    outs = [oracle.lib.orc_rng_u64(C.byref(probe)) for _ in range(312)]
+    return eng, np.array([untemper(v) for v in outs], dtype=np.uint64)

@@ -1,14 +1,13 @@
 """-m gpu: binary segmentation (ibin = true) through the device worklist against the oracle restatement (oracle/cbs_oracle.c,
 pinned to the compiled reference for tmaxo(ibin=true)).  The permutations decide with the scan of binary.cuh: the decision
 scan when the reject level Lstar lies above fac_max/4, the reference's ordered walk below it (DESIGN 4c)."""
-import ctypes as C
 import os
 import subprocess
 
 import numpy as np
 import pytest
 
-from helpers import pack
+from helpers import engine_after, pack
 from oracle.pyoracle import SegParams
 import genomic_b200
 from genomic_b200 import CbsGpuError, Params, RNG_MT19937_64, RNG_PHILOX
@@ -172,30 +171,6 @@ def test_binary_long_units(ctx, oracle, mode):
     p = SegParams(nperm=20, alpha=0.05, min_width=2, ibin=True, do_smooth=False, rng_kind=1 if mode == "philox" else 0,
                   chain=False, seed=4)
     check_batch(ctx, oracle, vals, off, p, first_batch=20, max_batch=20)
-
-
-def untemper(y):
-    y = int(y)
-    M = (1 << 64) - 1
-    y ^= y >> 43
-    y ^= (y << 37) & 0xFFF7EEE000000000 & M
-    z = y
-    for _ in range(4):
-        z = y ^ ((z << 17) & 0x71D67FFFEDA60000 & M)
-    y = z
-    z = y
-    for _ in range(3):
-        z = y ^ ((z >> 29) & 0x5555555555555555)
-    return z
-
-
-def engine_after(oracle, seed, skip):
-    eng = oracle.rng_mt(seed)
-    oracle.lib.orc_rng_discard(C.byref(eng), skip)
-    probe = oracle.rng_mt(seed)
-    oracle.lib.orc_rng_discard(C.byref(probe), skip)
-    outs = [oracle.lib.orc_rng_u64(C.byref(probe)) for _ in range(312)]
-    return eng, np.array([untemper(v) for v in outs], dtype=np.uint64)
 
 
 def test_binary_single_calls(ctx, oracle):

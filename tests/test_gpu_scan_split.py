@@ -18,9 +18,9 @@ def gparams(p: SegParams, **kw) -> Params:
                   rng_mode=RNG_PHILOX if p.rng_kind else RNG_MT19937_64, chain=p.chain, seed=p.seed, **kw)
 
 
-def tied_vectors():
+def tied_vectors(sizes=(20000, 61003)):
     """Vectors long enough for several slices whose maximum is attained by many arcs in different slices."""
-    for n in (20000, 61003):
+    for n in sizes:
         yield n, "runs", np.tile([1.0] * 700 + [-1.0] * 700, n // 1400 + 1)[:n]
         yield n, "motif", np.tile([0.5, 0.5, -1.0, 0.25, 0.25, -0.5], n // 6 + 1)[:n]
         x = np.zeros(n); x[n // 5: 3 * n // 5] = 1.0
