@@ -88,6 +88,7 @@ int fail(cbs_gpu_ctx* c, int code, const std::string& msg) {
     if (c) c->err = msg;
     return code;
 }
+const char* const kTooLong = "units and vectors longer than 8,388,608 (CBS_GPU_MAX_UNIT) markers are not supported";
 
 #define CUDA_TRY(c, expr)                                                                                   \
     do {                                                                                                    \
@@ -284,7 +285,7 @@ int smooth_device(cbs_gpu_ctx* c, const double* xin, const long long* goff, cons
 bool pick_scan_warps(cbs_gpu_ctx* c, ScanLayout& lay, int* occ_out, const void* kern) {
     int best_w = 0, best_res = 0, best_occ = 1;
     const int forced = (int)env_ll("CBS_GPU_SCAN_WARPS", 0);  // experiments only
-    for (int w : {8, 4, 2, 1}) {
+    for (int w : {SCAN_WARPS_MAX, 4, 2, 1}) {
         if (forced && w != forced) continue;
         lay.warps = w;
         if (lay.bytes() > c->smem_optin) continue;
@@ -395,7 +396,7 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     const long long N = off[n_units];
     long long Nmax = 0;
     for (int u = 0; u < n_units; ++u) Nmax = std::max(Nmax, off[u + 1] - off[u]);
-    if (Nmax > 1000000) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "units longer than 1,000,000 markers are not supported");
+    if (Nmax > CBS_GPU_MAX_UNIT) return fail(c, CBS_GPU_ERR_UNSUPPORTED, kTooLong);
     if (N > 2000000000LL) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "more than 2e9 markers per call are not supported");
     const bool mt = p->rng_mode == CBS_GPU_RNG_MT19937_64;
     if (weighted && p->ibin) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "weighted CBS has no binary mode (cbs::segment_weighted takes no ibin)");
@@ -606,8 +607,9 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     // ---- scan kernel configuration ------------------------------------------------------------
     ScanLayout lay;
     lay.nb_max = block_count((int)std::max<long long>(Nmax, 1)) + 2;
-    lay.set_table(std::max<long long>(Nmax, 1));
     int scan_occ = 1, obs_occ = 1;
+    if (!lay.set_table(std::max<long long>(Nmax, 1), c->smem_optin))
+        return fail(c, CBS_GPU_ERR_UNSUPPORTED, "segment too long for the scan kernel's shared memory");
     ScanLayout lay_obs = lay;
     if (!pick_scan_warps(c, lay, &scan_occ, (const void*)k_scan_perm<false>) ||
         !pick_scan_warps(c, lay_obs, &obs_occ, (const void*)k_scan_obs<false>))
@@ -617,6 +619,8 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     const size_t wscan_smem = ((sizeof(WScanSmem) + 15) & ~(size_t)15) + (size_t)lay.nb_max * (2 * sizeof(double) + 3 * sizeof(int)) + 16;
     const int scan_grid = c->sm_count * scan_occ;
     const size_t bscan_smem = ((sizeof(BinSmem) + 15) & ~(size_t)15) + (size_t)lay.nb_max * (2 * sizeof(double) + 3 * sizeof(int)) + 16;
+    if ((weighted && wscan_smem > c->smem_optin) || (p->ibin && bscan_smem > c->smem_optin))
+        return fail(c, CBS_GPU_ERR_UNSUPPORTED, "segment too long for the scan kernel's shared memory");
 
     // shared-memory shuffle kernel, one launch per segment-length class present in this call
     int shuf_occ[SHUF_CL2]; bool shuf_on[SHUF_CL2];
@@ -1034,7 +1038,8 @@ int cbs_gpu_create(const int* device_ids, int ndev, cbs_gpu_ctx** out) {
         !set_max_smem(k_shuffle<512, 2, false>, mx) || !set_max_smem(k_shuffle<1024, 2, false>, mx) ||
         !set_max_smem(k_shuffle_cluster<1024, 4, 2, true>, mx) || !set_max_smem(k_shuffle_cluster<1024, 4, 4, true>, mx) ||
         !set_max_smem(k_shuffle_cluster<1024, 4, 8, true>, mx) || !set_max_smem(k_shuffle_cluster<1024, 4, 2, false>, mx) ||
-        !set_max_smem(k_shuffle_cluster<1024, 4, 4, false>, mx) || !set_max_smem(k_shuffle_cluster<1024, 4, 8, false>, mx)) {
+        !set_max_smem(k_shuffle_cluster<1024, 4, 4, false>, mx) || !set_max_smem(k_shuffle_cluster<1024, 4, 8, false>, mx) ||
+        !set_max_smem(k_wscan<0>, mx) || !set_max_smem(k_wscan<1>, mx) || !set_max_smem(k_scan_binary, mx)) {
         delete c;
         return CBS_GPU_ERR_CUDA;
     }
@@ -1148,7 +1153,7 @@ static int run_raw_scan(cbs_gpu_ctx* c, const double* xh, int n, int count, doub
     if (ibin) return fail(c, CBS_GPU_ERR_CUDA, "internal: binary data takes run_bin_scan");
     if (n < 2 || count < 1 || !xh) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
     if (al0 < 1 || n < 2 * al0) return fail(c, CBS_GPU_ERR_INVALID, "need n >= 2*al0, al0 >= 1");
-    if (n > 1000000) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "vectors longer than 1,000,000 are not supported");
+    if (n > CBS_GPU_MAX_UNIT) return fail(c, CBS_GPU_ERR_UNSUPPORTED, kTooLong);
     if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
     cudaStream_t st = c->stream;
     const long long N = (long long)n * count;
@@ -1201,9 +1206,8 @@ static int run_raw_scan(cbs_gpu_ctx* c, const double* xh, int n, int count, doub
     CUDA_TRY(c, cudaMemcpyAsync(c->dev.p, &hD, sizeof(Dev), cudaMemcpyHostToDevice, st));
     ScanLayout lay;
     lay.nb_max = nb + 2;
-    lay.set_table(n);
     int occ = 1;
-    if (!pick_scan_warps(c, lay, &occ, (const void*)k_scan_obs<false>)) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "vector too long for the scan kernel's shared memory");
+    if (!lay.set_table(n, c->smem_optin) || !pick_scan_warps(c, lay, &occ, (const void*)k_scan_obs<false>)) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "vector too long for the scan kernel's shared memory");
     Dev* dD = c->dev.as<Dev>();
     k_tables<<<dim3(16, 64), 256, 0, st>>>(dD);
     k_prep<<<std::min(count, c->sm_count * 8), 32, 0, st>>>(dD);
@@ -1221,7 +1225,7 @@ static int run_bin_scan(cbs_gpu_ctx* c, const double* xh, int n, int count, doub
     if (!c) return CBS_GPU_ERR_INVALID;
     if (n < 2 || count < 1 || !xh) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
     if (al0 < 1 || n < 2 * al0) return fail(c, CBS_GPU_ERR_INVALID, "need n >= 2*al0, al0 >= 1");
-    if (n > 1000000) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "vectors longer than 1,000,000 are not supported");
+    if (n > CBS_GPU_MAX_UNIT) return fail(c, CBS_GPU_ERR_UNSUPPORTED, kTooLong);
     if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
     cudaStream_t st = c->stream;
     const long long N = (long long)n * count, per = bin_scratch_doubles(n);
@@ -1699,7 +1703,7 @@ int cbs_gpu_xperm(cbs_gpu_ctx* c, const double* x, const double* rwts, int32_t n
                   double* px) {
     if (!c) return CBS_GPU_ERR_INVALID;
     if (n < 1 || !x || !px) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
-    if (n > 1000000) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "vectors longer than 1,000,000 are not supported");
+    if (n > CBS_GPU_MAX_UNIT) return fail(c, CBS_GPU_ERR_UNSUPPORTED, kTooLong);
     if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
     cudaStream_t st = c->stream;
     std::vector<uint64_t> words((size_t)n + 312);
@@ -1771,7 +1775,7 @@ int cbs_gpu_htmaxp(cbs_gpu_ctx* c, const double* px, int32_t n, int32_t count, d
     if (ibin) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "htmaxp with ibin=true is not implemented");
     if (n < 2 || count < 1 || !px || !statistics) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
     if (al0 < 1 || k < al0 || k > 128 || n <= 2 * k) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "need al0 <= k <= 128 and n > 2k");
-    if (n > 1000000) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "vectors longer than 1,000,000 are not supported");
+    if (n > CBS_GPU_MAX_UNIT) return fail(c, CBS_GPU_ERR_UNSUPPORTED, kTooLong);
     if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
     cudaStream_t st = c->stream;
     const long long N = (long long)n * count;

@@ -1059,6 +1059,7 @@ __device__ __forceinline__ bool cand_better(const Cand& a, const Cand& b) {
 #define SCAN_QUEUE 256  // per-warp ring of surviving units (entries)
 #define SCAN_GRING 64   // per-warp ring of surviving groups of 128 arc lengths (entries)
 #define SCAN_LIST 2048  // per-CTA list of block pairs that reach the level (entries)
+#define SCAN_WARPS_MAX 8  // widest scan CTA that pick_scan_warps tries
 #define SCAN_LSMALL 128 // arcs shorter than this are swept row by row over the whole segment, not pair by pair
 #define PCODE_FLAT 0xffffffffu  // unit of the short-arc sweep: the block pair is looked up per arc
 
@@ -1274,6 +1275,21 @@ __device__ __forceinline__ float window_bound(const ScanCtx& c, int i0, int js, 
     return fmaxf(__fsub_ru(wmax, rmin), __fsub_ru(rmax, wmin));
 }
 
+// A unit (rows 32a .. 32a+31, arc lengths L0 .. L0+7, L0 a multiple of 8) is queued as 32 bits next to its pair code.
+// A unit of a block pair keeps its row group relative to the pair's first one: ((a - a0) << 20) | (L0 >> 3), a0 =
+// ilo >> 5 of block bi; a block spans fewer than 2^17 rows and arc lengths stay below 2^23 (CBS_GPU_MAX_UNIT).  A unit
+// of the short-arc sweep (PCODE_FLAT, L0 < SCAN_LSMALL) keeps its whole row group: (a << 4) | (L0 >> 3).
+__device__ __forceinline__ unsigned unit_code_pair(int a0, int a, int L0) { return ((unsigned)(a - a0) << 20) | (unsigned)(L0 >> 3); }
+__device__ __forceinline__ unsigned unit_code_flat(int a, int L0) { return ((unsigned)a << 4) | (unsigned)(L0 >> 3); }
+__device__ __forceinline__ void unit_decode(const ScanCtx& c, unsigned code, unsigned pcode, int& i0, int& L0) {
+    if (pcode == PCODE_FLAT) {
+        i0 = (int)(code >> 4) << 5; L0 = (int)(code & 15u) << 3;
+    } else {
+        const int a0 = (c.bb[(pcode >> 16) - 1] + 1) >> 5;  // ilo >> 5 of block bi (pair_lengths)
+        i0 = (a0 + (int)(code >> 20)) << 5; L0 = (int)(code & 0xfffffu) << 3;
+    }
+}
+
 // per-warp ring of units that survived the pruning tests; it lives across the pairs of a permutation so that the
 // arcs are (almost) always examined by 32 busy lanes
 struct UnitQueue {
@@ -1286,7 +1302,8 @@ struct UnitQueue {
 // (finite padding), can only produce a spurious hit, which the exact re-evaluation discards.
 template <bool OBS>
 __device__ __forceinline__ void scan_unit(const ScanCtx& c, unsigned code, unsigned pcode, ScanSmem* sm) {
-    const int i0 = (int)(code >> 17) << 5, L0 = (int)(code & 0x1ffffu) << 3;
+    int i0, L0;
+    unit_decode(c, code, pcode, i0, L0);
     // Thresholds for the 8 lengths.  The fast path never compares doubles (DSETP issues at a quarter of the DADD
     // rate on B200): an arc can only beat the level if |S_j - S_i| > th, and then the high word of |S_j - S_i|
     // is >= the high word of th.  Per length the maximum of (hi << 1) (the shift drops the sign) is kept with one
@@ -1397,7 +1414,7 @@ __device__ void sweep_short(const ScanCtx& c, UnitQueue& uq, ScanSmem* sm, int w
         unsigned keep4 = 0, code0 = 0;
         if (idx < total) {
             const int a = idx / ngs, Ls = (idx - a * ngs) << 5;
-            code0 = ((unsigned)a << 17) | (unsigned)(Ls >> 3);
+            code0 = unit_code_flat(a, Ls);
             if (group_may_reach(c, gs, sm, a, Ls, 32, La, Lb)) {
 #pragma unroll
                 for (int t = 0; t < 4; ++t)
@@ -1443,7 +1460,7 @@ __device__ void scan_band(const ScanCtx& c, const PairGeo& g, unsigned pcode, Un
                 const int ar = idx / ncg;
                 const int a = a0 + ar, Lc = (c0 + (idx - ar * ncg)) << 7;
                 keep = group_may_reach(c, g, sm, a, Lc, 128, La, Lb);
-                code = ((unsigned)a << 17) | (unsigned)(Lc >> 3);
+                code = unit_code_pair(a0, a, Lc);
             }
             const unsigned mask = __ballot_sync(FULL, keep);
             if (mask) {
@@ -1458,8 +1475,8 @@ __device__ void scan_band(const ScanCtx& c, const PairGeo& g, unsigned pcode, Un
             unsigned keep4 = 0, code0 = 0;  // surviving 8-length units of this lane's 32-length group
             if ((unsigned)(lane >> 2) < gtake) {
                 const unsigned gc = (unsigned)gring[(ghead + (lane >> 2)) & (SCAN_GRING - 1)];
-                const int a = (int)(gc >> 17), Ls = ((int)(gc & 0x1ffffu) << 3) + 32 * (lane & 3);
-                code0 = ((unsigned)a << 17) | (unsigned)(Ls >> 3);
+                const int a = a0 + (int)(gc >> 20), Ls = ((int)(gc & 0xfffffu) << 3) + 32 * (lane & 3);
+                code0 = unit_code_pair(a0, a, Ls);
                 if (group_may_reach(c, g, sm, a, Ls, 32, La, Lb)) {
 #pragma unroll
                     for (int t = 0; t < 4; ++t)
@@ -1518,11 +1535,19 @@ struct ScanLayout {
         return ((sizeof(ScanSmem) + 15) & ~(size_t)15) + 2 * (size_t)nb_max * 8 + 3 * (size_t)nb_max * 4 + 2 * (size_t)nt * 4 +
                (size_t)warps * (2 * SCAN_QUEUE + SCAN_GRING) * 4 + (size_t)SCAN_LIST * 4 + 64;
     }
-    // table geometry for units of up to nmax markers: at most 16384 entries (128 KB)
-    CBS_HD void set_table(long long nmax) {
-        tsh = 5;
-        while (((nmax >> tsh) + 2) > 16384) ++tsh;
-        nt = (int)(nmax >> tsh) + 2;
+    // table geometry for units of up to nmax markers (nb_max set): at most 16384 entries (128 KB), and coarser still until
+    // the layout with the most warps fits in `optin` bytes next to the block arrays and queues.  False when even 1024
+    // prefix sums per entry do not fit: the observed scan merges at most one warp's 1024 prefix sums into an entry.
+    CBS_HD bool set_table(long long nmax, size_t optin) {
+        const int w = warps;
+        warps = SCAN_WARPS_MAX;
+        bool fits = false;
+        for (tsh = 5; tsh <= 10 && !fits; tsh += fits ? 0 : 1) {
+            nt = (int)(nmax >> tsh) + 2;
+            fits = nt <= 16384 && bytes() <= optin;
+        }
+        warps = w;
+        return fits;
     }
 };
 
@@ -1603,7 +1628,7 @@ __device__ __forceinline__ void scan_rows(Dev* D, const ScanLayout& lay) {
             __syncthreads();
         // ---- phase 0a: extrema table.  A warp takes 1024 consecutive prefix sums (coalesced loads); a
             // reduce-scatter over the lanes leaves lane l with the extrema of run l of 32, in single precision
-            // rounded outwards; runs are merged 2 or 4 to an entry when the table is coarser (tsh 6, 7).
+            // rounded outwards; runs are merged 2, 4, .. 32 to an entry when the table is coarser (tsh 6 .. 10).
             for (int c0 = warp * 1024; c0 <= n; c0 += nwarps * 1024) {
                 float lo[32], hi[32];
     #pragma unroll
@@ -1658,7 +1683,7 @@ __device__ __forceinline__ void scan_rows(Dev* D, const ScanLayout& lay) {
             __syncthreads();
         } else {
             // ---- phase 0: the statistics of the row were written next to it by k_chain: the extrema of every
-            // aligned run of 32 prefix sums (merged 2 or 4 to an entry when the table is coarser) and the per-block
+            // aligned run of 32 prefix sums (merged 2, 4, .. 32 to an entry when the table is coarser) and the per-block
             // extrema with their first occurrence (CBS.cpp:88-94)
             {
                 const float* gmin = (const float*)(c.sx + Sched::tbl_offset(n));

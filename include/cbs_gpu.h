@@ -30,6 +30,10 @@ extern "C" {
 #define CBS_GPU_RNG_MT19937_64 0   /* bit-exact replay of std::mt19937_64 + generate_canonical */
 #define CBS_GPU_RNG_PHILOX 1       /* Philox4x32-10 counter mode, keyed per (seed, unit, segment) */
 
+/* Longest unit (one chromosome of one sample) and longest vector that any entry point takes, in markers.  Longer ones
+ * are rejected with CBS_GPU_ERR_UNSUPPORTED; a call takes at most 2e9 markers in all. */
+#define CBS_GPU_MAX_UNIT 8388608
+
 #define CBS_GPU_F32 0
 #define CBS_GPU_F64 1
 #define CBS_GPU_HOST 0
