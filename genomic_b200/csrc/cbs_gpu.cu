@@ -402,6 +402,11 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     if (weighted && p->ibin) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "weighted CBS has no binary mode (cbs::segment_weighted takes no ibin)");
     if (weighted && p->hybrid && p->nmin < p->kmax + 2)
         return fail(c, CBS_GPU_ERR_UNSUPPORTED, "weighted hybrid CBS needs nmin >= kmax + 2");
+    // A hybrid segment has n > nmin markers.  The reference is undefined below n = kmax + 2: with n < kmax htmaxp has no
+    // block (nb = int(n/kmax) = 0) and reads past its block tables (CBS.cpp:387-485); with n <= kmax + 1, delta =
+    // (kmax+1)/n >= 1 makes tailp NaN or -inf and nrejc = (int)((alpha - pval1) * nperm) an out-of-range conversion.
+    if (!weighted && !api.mode && p->hybrid && p->nmin < p->kmax + 1)
+        return fail(c, CBS_GPU_ERR_UNSUPPORTED, "hybrid CBS needs nmin >= kmax + 1 (the reference's hybrid p-value is undefined on segments of kmax + 1 markers or fewer)");
 
     RunCaps cap;
     cap.task_cap = (int)std::min<long long>(std::max<long long>(4096, 64LL * n_units + 1024), 1 << 22);
@@ -1611,6 +1616,11 @@ static int decision_impl(cbs_gpu_ctx* c, const double* x, const double* weights,
     p.do_smooth = 0; p.undo_prune = 0; p.chain = 0; p.record_splits = 1;
     int rc = validate_params(c, &p);
     if (rc) return rc;
+    if (!weights && api.mode == 1 && p.hybrid) {  // cbs_gpu_fndcpt; see the nmin rule in run_cbs
+        const double delta = api.delta > 0.0 ? api.delta : (double)(p.kmax + 1) / (double)n;
+        if (n < p.kmax || !(delta < 1.0))
+            return fail(c, CBS_GPU_ERR_UNSUPPORTED, "hybrid fndcpt needs n >= hk and delta < 1 (the reference's htmaxp or tailp is undefined otherwise)");
+    }
     for (int i = 0; i < n; ++i) if (!std::isfinite(x[i])) return fail(c, CBS_GPU_ERR_NONFINITE, "non-finite values reach CBS");
     cudaStream_t st = c->stream;
     ENSURE(c, c->x, sizeof(double) * (size_t)(n + 1));
@@ -1774,7 +1784,8 @@ int cbs_gpu_htmaxp(cbs_gpu_ctx* c, const double* px, int32_t n, int32_t count, d
     if (!c) return CBS_GPU_ERR_INVALID;
     if (ibin) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "htmaxp with ibin=true is not implemented");
     if (n < 2 || count < 1 || !px || !statistics) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
-    if (al0 < 1 || k < al0 || k > 128 || n <= 2 * k) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "need al0 <= k <= 128 and n > 2k");
+    // n < k leaves the reference's htmaxp without a block (nb = int(n/k) = 0): undefined there, as for the segmenter
+    if (al0 < 1 || k < al0 || k > 128 || n < k) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "need al0 <= k <= 128 and n >= k");
     if (n > CBS_GPU_MAX_UNIT) return fail(c, CBS_GPU_ERR_UNSUPPORTED, kTooLong);
     if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
     cudaStream_t st = c->stream;

@@ -1971,7 +1971,8 @@ __global__ void __launch_bounds__(256, 2) k_scan_obs(Dev* D, ScanLayout lay) { s
 //             fac(j)*d*d over ALL arcs of length al0..k (inside its ~k-wide blocks, straddling
 //             adjacent blocks, and wrapping around the end), plus the per-block (argmin,argmax)
 //             candidates, which use the other rounding fac*(d*d) (:415-416).  It is evaluated
-//             here by brute force, 25 arcs per marker.
+//             here by brute force, 25 arcs per marker.  That holds for n >= 2k; a segment with
+//             k > n/2 follows htmaxp's own loops instead (htmaxp_one_block).
 // ------------------------------------------------------------------------------------
 __device__ double dev_fpnorm(double x) { return 0.5 * erfc(-x / sqrt(2.0)); }
 __device__ double dev_nu(double x, double tol) {
@@ -2094,6 +2095,41 @@ __global__ void k_btailp_sum(double b, int m, int ng, const double* vals, double
     *out = acc;
 }
 
+// htmaxp (CBS.cpp:387-485) as written, for k > n/2 (so n < 2k and one block, nb = int(n/k) = 1).  Its pruning stops the
+// loop over arc lengths j at the first j with fac(j)*spread^2 < max, which is exact only while fac(j) = n/(j(n-j))
+// decreases, i.e. for j <= n/2; past n/2 it skips arcs, and its value is then not the all-arcs maximum k_hscan computes.
+__device__ double htmaxp_one_block(const double* __restrict__ sx, int n, int k, int al0) {
+    const double rn = (double)n;
+    double lo = sx[1], hi = lo, out = 0.0;
+    int ilo = 1, ihi = 1;
+    for (int i = 2; i <= n; ++i) {
+        const double v = sx[i];
+        if (v < lo) { lo = v; ilo = i; }
+        if (v > hi) { hi = v; ihi = i; }
+    }
+    const int d = abs(ilo - ihi);
+    if (d <= k && d >= al0) {
+        const double rj = (double)d;
+        const double fac = rn / (rj * (rn - rj));
+        const double v = fac * ((hi - lo) * (hi - lo));
+        if (out < v) out = v;
+    }
+    const double spread_sq = (hi - lo) * (hi - lo);  // also the wrap-around spread when nb = 1 (:441-443)
+    for (int wrap = 0; wrap < 2; ++wrap) {
+        for (int j = al0; j <= k; ++j) {
+            const double rj = (double)j;
+            const double fac = rn / (rj * (rn - rj));
+            if (fac * spread_sq < out) break;
+            double widest = 0.0;
+            if (!wrap) { for (int i = 1; i <= n - j; ++i) { const double w = fabs(sx[i + j] - sx[i]); if (widest < w) widest = w; } }
+            else       { for (int i = 1; i <= j; ++i) { const double w = fabs(sx[i + n - j] - sx[i]); if (widest < w) widest = w; } }
+            const double v = fac * widest * widest;
+            if (out < v) out = v;
+        }
+    }
+    return out;
+}
+
 __global__ void __launch_bounds__(256) k_hscan(Dev* D) {
     __shared__ double s_fac[132];
     __shared__ double s_red[8];
@@ -2122,6 +2158,9 @@ __global__ void __launch_bounds__(256) k_hscan(Dev* D) {
         }
         __syncthreads();
         double best = 0.0;
+        if (2 * kk > n) {  // fac(j) grows again past j = n/2: htmaxp's own loops, one thread (n < 2k <= 256)
+            if (tid == 0) best = htmaxp_one_block(sx, n, kk, al0);
+        } else
         // all arcs (i, i+j), 1 <= i <= n-j, and the wrap-around arcs i = 1..j against i+n-j
         for (int i = 1 + tid; i <= n; i += blockDim.x) {
             const double si = sx[i];

@@ -46,7 +46,7 @@ typedef struct cbs_gpu_ctx cbs_gpu_ctx;
 typedef struct cbs_gpu_params {
     double alpha;
     int32_t nperm;
-    int32_t hybrid;
+    int32_t hybrid;        /* needs kmax in 1..128 and nmin >= kmax + 1 (weighted: nmin >= kmax + 2) */
     int32_t min_width;
     int32_t kmax;
     int32_t nmin;
@@ -164,7 +164,9 @@ int cbs_gpu_tmaxp(cbs_gpu_ctx* ctx, const double* px, int32_t n, int32_t count, 
  * hybrid method's argument (0: (kmax+1)/n), ngrid must be 100.  sbdry is not an argument: `cna segment` disables the
  * sequential boundary (src/cna_segment.hpp:130) and so does this library.  The result comes back as a split record:
  * ncpt, icpt0/icpt1, iseg0/iseg1 (0-based, as cbs::ChangePointResult), ostat, plus perms_run, nrej and the edge tests'
- * counts for diagnostics.  mt_next312 / draws_consumed as in cbs_gpu_segment. */
+ * counts for diagnostics.  mt_next312 / draws_consumed as in cbs_gpu_segment.  hybrid with n < hk, or
+ * with delta >= 1 (with delta = 0: n <= hk + 1), is CBS_GPU_ERR_UNSUPPORTED: the reference's htmaxp has no block there, or
+ * its tailp is NaN or -inf, and its result is undefined. */
 int cbs_gpu_fndcpt(cbs_gpu_ctx* ctx, const double* x, int32_t n, double tss, const cbs_gpu_params* params, double delta,
                    int32_t ngrid, const uint64_t* mt_next312, cbs_gpu_split* out, uint64_t* draws_consumed);
 /* cbs::wfindcpt (CBS.hpp:81-97, CBS.cpp:894-957).  The reference also takes rwts = sqrt(wts) and cwts =
@@ -187,7 +189,8 @@ int cbs_gpu_wtmaxo(cbs_gpu_ctx* ctx, const double* x, const double* weights, int
  * engine advances by exactly n draws. */
 int cbs_gpu_xperm(cbs_gpu_ctx* ctx, const double* x, const double* rwts, int32_t n, const uint64_t* mt_next312, uint64_t seed,
                   double* px);
-/* cbs::htmaxp (CBS.hpp:34, CBS.cpp:387-485) for `count` vectors of length n laid end to end; ibin must be 0 */
+/* cbs::htmaxp (CBS.hpp:34, CBS.cpp:387-485) for `count` vectors of length n laid end to end; ibin must be 0,
+ * al0 <= k <= 128 and n >= k (with n < k the reference's htmaxp has no block and is undefined) */
 int cbs_gpu_htmaxp(cbs_gpu_ctx* ctx, const double* px, int32_t n, int32_t count, double tss, int32_t k, int32_t al0,
                    int32_t ibin, double* statistics);
 /* cbs::tailp (CBS.hpp:29, CBS.cpp:324-339); ngrid must be 100.  Evaluated with the CUDA erfc/log/exp/pow (<= 4 ulp each), so

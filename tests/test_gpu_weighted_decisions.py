@@ -10,19 +10,13 @@ import re
 import numpy as np
 import pytest
 
-from helpers import engine_after, f32, make_unit, pack, weighted_centre
+from helpers import check_edge_p, check_split_log, engine_after, f32, gparams, make_unit, pack, weighted_centre
 from oracle.pyoracle import SegParams, SplitIntoItself, weight_tables
 from test_gpu_scan_split import tied_vectors
-from genomic_b200 import CbsGpuError, Params, RNG_MT19937_64, RNG_PHILOX
+from genomic_b200 import CbsGpuError, Params
 from genomic_b200.binding import ERR_UNSUPPORTED
 
 pytestmark = pytest.mark.gpu
-
-
-def gparams(p: SegParams, **kw) -> Params:
-    return Params(alpha=p.alpha, nperm=p.nperm, hybrid=p.hybrid, min_width=p.min_width, kmax=p.kmax, nmin=p.nmin,
-                  do_smooth=False, rng_mode=RNG_PHILOX if p.rng_kind else RNG_MT19937_64, chain=p.chain, seed=p.seed,
-                  undo_prune=p.undo_prune, undo_prune_cutoff=p.undo_prune_cutoff, **kw)
 
 
 def weight_sets(rng, n):
@@ -88,15 +82,6 @@ def decision_input(rng, kind, n):
     return f32(x)
 
 
-def check_edge_p(status, nrej, want_p, nperm, msg):
-    """tpermp p-values of both boundaries: the device reports the rejection counts and the shortcut status"""
-    for side in (0, 1):
-        if want_p[side] < 0:
-            continue  # not run
-        got_p = 1.0 if status[side] == 1 else 0.0 if status[side] == 2 else nrej[side] / nperm
-        assert got_p == want_p[side], (msg, side, status, nrej, want_p)
-
-
 def test_wfindcpt_single_calls(ctx, oracle):
     """cbs::wfindcpt with a caller-owned engine that has already been used: every field of the decision and the draws."""
     rng = np.random.default_rng(501)
@@ -153,32 +138,10 @@ def step_unit(rng, n):
 
 
 def check_weighted_log(got, want, p, exact_draws):
-    """every logged decision of the device equals the oracle's, matched by (unit, lo, hi); returns coverage counts"""
-    assert np.array_equal(got.seg_count, want["seg_count"])
-    assert np.array_equal(got.lengths, want["lengths"])
-    if p.hybrid:  # as in the other hybrid tests
-        assert np.allclose(got.means, want["means"], rtol=1e-9, atol=0)
-    else:
-        assert np.array_equal(got.means, want["means"])
-    if exact_draws:
-        assert np.array_equal(got.draws, want["draws"])
-    assert len(got.splits) == len(want["log"])
-    by_key = {(g["unit"], g["lo"], g["hi"]): g for g in got.splits}
-    assert len(by_key) == len(got.splits)
-    edge_mid = nrej_mid = 0
-    for u, w in want["log"]:
-        key = (u, w.lo, w.hi)
-        g = by_key[key]
-        assert (g["called"], g["ncpt"]) == (w.called, w.ncpt), key
-        if not w.called:
-            continue
-        assert np.array_equal(g["ostat"], w.ostat, equal_nan=True), key
-        assert (g["iseg0"], g["iseg1"], g["perms_run"], g["nrej"], g["exit_code"]) == \
-            (w.iseg0, w.iseg1, w.perms_run, w.nrej, w.exit_code), key
-        assert (g["icpt0"], g["icpt1"])[:w.ncpt] == (w.icpt0, w.icpt1)[:w.ncpt], key
-        check_edge_p((g["e_status0"], g["e_status1"]), (g["e_nrej0"], g["e_nrej1"]), (w.edge_p0, w.edge_p1), p.nperm, key)
-        edge_mid += int(0.0 < w.edge_p0 < 1.0) + int(0.0 < w.edge_p1 < 1.0)
-        nrej_mid += int(w.exit_code != 3 and 0 < w.nrej)
+    """helpers.check_split_log; returns coverage counts: edge tests with 0 < p < 1, max-t tests run to the end with nrej > 0"""
+    called = check_split_log(got, want, p, exact_draws)
+    edge_mid = sum(int(0.0 < w.edge_p0 < 1.0) + int(0.0 < w.edge_p1 < 1.0) for _, w, _ in called)
+    nrej_mid = sum(int(w.exit_code != 3 and 0 < w.nrej) for _, w, _ in called)
     return edge_mid, nrej_mid
 
 
