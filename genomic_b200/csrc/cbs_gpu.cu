@@ -13,7 +13,6 @@
 #include <cstddef>
 #include <cstring>
 #include <string>
-#include <thread>
 #include <vector>
 
 #include "../../include/cbs_gpu.h"
@@ -40,6 +39,23 @@ struct DevBuf {
 
 enum KernelId { K_SCHED = 0, K_GEN, K_PREP, K_PERM, K_SCAN, K_EDGEPREP, K_EDGEPERM, K_MEANS, K_SMOOTH, K_SHUF0, K_SHUF1, K_SHUF2, K_SHUF3, K_PREFIX, K_COUNT };
 
+// Everything one scheduler round reads that can differ between calls: the round's launches are a function of this alone,
+// so it is also the key of the cached call graph.  Zeroed with memset before it is filled, so that padding compares equal.
+struct RoundConfig {
+    Dev* dD;
+    cudaStream_t st, side[5], gen;  // as resolved after `serial`
+    int weighted, mt, shared_stream, jump, hybrid, ibin, l2_shuffle_on, counting;
+    int n_chains;
+    int shuf_on[SHUF_CL2], shuf_occ[SHUF_CL2];
+    int cl_R, cl_grid, cl2_grid;
+    size_t cl_smem, cl2_smem;
+    int chain_occ;
+    int scan_grid, obs_grid;
+    ScanLayout lay, lay_obs;
+    size_t wscan_smem, bscan_smem;
+    const void* tailp;
+};
+
 }  // namespace
 
 struct cbs_gpu_ctx {
@@ -50,7 +66,7 @@ struct cbs_gpu_ctx {
     std::string err;
     int* h_done = nullptr;  // mapped pinned
     cudaGraphExec_t call_exec = nullptr;  // graph of a whole call: WHILE node around one scheduler round (run_cbs)
-    std::vector<unsigned char> call_key;  // the launch configuration it was captured with
+    RoundConfig call_cfg;                 // the round configuration it was captured with
     unsigned long long round_launches = 0;
     int* d_done = nullptr;  // device alias of h_done
     DevBuf x, cur, gtab, factab, bbtab, unit_off, unit_ids, tasks, ring, act0, act1, chains, segs, splits, udraws, arena,
@@ -58,12 +74,6 @@ struct cbs_gpu_ctx {
         dev, staging, fv, fidx, flab, lab, diffs, diffs_sorted, sm_keys, sm_gid, cn_scratch, gout, cubtmp, flag, goff, stream_buf, shuf, jump, tailp,
         wts, rw, cw, ycur;  // weighted CBS
     bool jump_ready = false;
-    // lanes: a call with independent units is split into contiguous unit ranges that run as separate
-    // worklists on their own streams (child contexts), so the latency-bound phases of one lane overlap
-    // the other's; results are merged in unit order
-    std::vector<cbs_gpu_ctx*> lanes;
-    double mem_fraction = 0.80;  // share of free device memory the arenas of this context may take
-    bool is_lane = false;
     bool profiling = false;   // per-launch CUDA events
     bool serial = false;      // all kernels of a round on one stream (non-overlapping per-kernel times)
     bool counting = false;    // scan work counters (atomics in the kernel: slows it, never combine with timing)
@@ -180,6 +190,34 @@ int validate_params(cbs_gpu_ctx* c, const cbs_gpu_params* p) {
     return CBS_GPU_OK;
 }
 
+// start of an entry point: a context, its device current, the kernel timings and launch count of the last call cleared
+int begin_call(cbs_gpu_ctx* c) {
+    if (!c) return CBS_GPU_ERR_INVALID;
+    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
+    for (double& ms : c->kms) ms = 0.0;
+    c->launches = 0;
+    return CBS_GPU_OK;
+}
+#define BEGIN_CALL(c)                                           \
+    do {                                                        \
+        const int rc__ = begin_call(c);                         \
+        if (rc__ != CBS_GPU_OK) return rc__;                    \
+    } while (0)
+
+// unit table of a batch: starts at 0 and never decreases
+int check_unit_offsets(cbs_gpu_ctx* c, const int64_t* unit_offsets, int n_units) {
+    if (unit_offsets[0] != 0) return fail(c, CBS_GPU_ERR_INVALID, "unit_offsets[0] must be 0");
+    for (int u = 0; u < n_units; ++u)
+        if (unit_offsets[u + 1] < unit_offsets[u]) return fail(c, CBS_GPU_ERR_INVALID, "unit_offsets must be non-decreasing");
+    return CBS_GPU_OK;
+}
+
+// CBS needs finite input (the reference has no defined behaviour otherwise): host vectors of the single-vector entry points
+int check_finite_host(cbs_gpu_ctx* c, const double* x, long long n) {
+    for (long long i = 0; i < n; ++i) if (!std::isfinite(x[i])) return fail(c, CBS_GPU_ERR_NONFINITE, "non-finite values reach CBS");
+    return CBS_GPU_OK;
+}
+
 // ---- smoothing on device buffers -------------------------------------------------------------
 // xin: values (double, device, N), goff: device group offsets [n_groups+1], dlab: labels or nullptr
 // (constant label per group), out: device N. host_off is the host copy of the offsets.
@@ -284,9 +322,7 @@ int smooth_device(cbs_gpu_ctx* c, const double* xin, const long long* goff, cons
 // shape that keeps the most warps resident on an SM
 bool pick_scan_warps(cbs_gpu_ctx* c, ScanLayout& lay, int* occ_out, const void* kern) {
     int best_w = 0, best_res = 0, best_occ = 1;
-    const int forced = (int)env_ll("CBS_GPU_SCAN_WARPS", 0);  // experiments only
     for (int w : {SCAN_WARPS_MAX, 4, 2, 1}) {
-        if (forced && w != forced) continue;
         lay.warps = w;
         if (lay.bytes() > c->smem_optin) continue;
         int occ = 0;
@@ -347,6 +383,8 @@ int shuffle_occupancy(int cls) {
 template <class F>
 bool set_max_smem(F* f, int bytes) { return cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes) == cudaSuccess; }
 
+const int kClusterHbits = 12;  // log2 of the claim-table entries of k_shuffle_cluster
+
 // resident clusters x R of k_shuffle_cluster for segments of up to nmax markers (0: does not fit / not schedulable)
 int cluster_fit(cbs_gpu_ctx* c, int R, long long nmax, int hbits, size_t* smem_out) {
     const size_t smem = ((size_t)4 << hbits) + 4 * ((size_t)nmax / R + 4);
@@ -365,9 +403,15 @@ int cluster_fit(cbs_gpu_ctx* c, int R, long long nmax, int hbits, size_t* smem_o
     return ncl * R;
 }
 
+// Sizes of one call (run_cbs stage 1): limits of the input, capacities of the worklist tables, the permutation arena, the
+// MT draw windows and the shared stream ring.
 struct RunCaps {
+    long long N, Nmax;
+    bool mt, shared_stream;
+    int n_chains;
     int task_cap, list_cap, seg_cap, split_cap, max_live;
     long long arena_cap, draws_cap, rej_cap;
+    long long stream_ring, stream_mirror;
 };
 
 // The core: x already resident (double, device, smoothed if requested) in c->x.
@@ -377,22 +421,10 @@ struct ApiMode {   // low-level entry points: ONE decision on the vector as give
     int n1 = 0, n2 = 0;
 };
 
-int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* unit_ids, int n_units,
-            const cbs_gpu_params* p, const uint64_t* mt_next312, bool weighted /* weights resident in c->wts */, Dev& hD,
-            const ApiMode& api = ApiMode()) {
-    cudaStream_t st = c->stream;
-    // CBS_GPU_DEBUG_SETUP=1: host wall clock of the set-up phases on stderr
-    const bool setup_debug = getenv("CBS_GPU_DEBUG_SETUP") != nullptr;
-    auto setup_t0 = std::chrono::steady_clock::now();
-    auto setup_mark = [&](const char* what) {
-        if (!setup_debug) return;
-        const auto now = std::chrono::steady_clock::now();
-        fprintf(stderr, "[setup] %s %.3f ms\n", what, std::chrono::duration<double, std::milli>(now - setup_t0).count());
-        setup_t0 = now;
-    };
-    // profiling bit 2: every kernel on the one stream, so that per-launch event times do not overlap (roofline time base)
-    cudaStream_t side[5], gen_stream = c->serial ? st : c->gen_stream;
-    for (int k = 0; k < 5; ++k) side[k] = c->serial ? st : c->side[k];
+const double kMemFraction = 0.80;  // share of free device memory the arenas of a context may take
+
+int size_call(cbs_gpu_ctx* c, const std::vector<long long>& off, int n_units, const cbs_gpu_params* p, bool weighted,
+              const ApiMode& api, RunCaps& cap) {
     const long long N = off[n_units];
     long long Nmax = 0;
     for (int u = 0; u < n_units; ++u) Nmax = std::max(Nmax, off[u + 1] - off[u]);
@@ -407,8 +439,8 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     // (kmax+1)/n >= 1 makes tailp NaN or -inf and nrejc = (int)((alpha - pval1) * nperm) an out-of-range conversion.
     if (!weighted && !api.mode && p->hybrid && p->nmin < p->kmax + 1)
         return fail(c, CBS_GPU_ERR_UNSUPPORTED, "hybrid CBS needs nmin >= kmax + 1 (the reference's hybrid p-value is undefined on segments of kmax + 1 markers or fewer)");
+    cap.N = N; cap.Nmax = Nmax; cap.mt = mt;
 
-    RunCaps cap;
     cap.task_cap = (int)std::min<long long>(std::max<long long>(4096, 64LL * n_units + 1024), 1 << 22);
     cap.task_cap = (int)std::max<long long>(64, std::min<long long>(env_ll("CBS_GPU_TASK_CAP", cap.task_cap), 1 << 24));  // env overrides: sane range only
     cap.list_cap = 4 * cap.task_cap + n_units + 16;
@@ -437,8 +469,8 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     ENSURE(c, c->ring, sizeof(int) * (size_t)cap.task_cap);
     ENSURE(c, c->act0, sizeof(int) * (size_t)cap.list_cap);
     ENSURE(c, c->act1, sizeof(int) * (size_t)cap.list_cap);
-    const int n_chains = mt ? (p->chain ? 1 : n_units) : 0;
-    ENSURE(c, c->chains, sizeof(Chain) * (size_t)std::max(1, n_chains));
+    cap.n_chains = mt ? (p->chain ? 1 : n_units) : 0;
+    ENSURE(c, c->chains, sizeof(Chain) * (size_t)std::max(1, cap.n_chains));
     ENSURE(c, c->segs, sizeof(SegRec) * (size_t)cap.seg_cap);
     ENSURE(c, c->splits, sizeof(SplitRec) * (size_t)cap.split_cap);
     ENSURE(c, c->udraws, sizeof(uint64_t) * (size_t)(n_units + 1));
@@ -449,20 +481,20 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     ENSURE(c, c->edgeprep_task, sizeof(int) * (size_t)cap.list_cap);
     ENSURE(c, c->edges, sizeof(EdgeItem) * (size_t)cap.list_cap);
     ENSURE(c, c->edge_prefix, sizeof(int) * (size_t)(cap.list_cap + 1));
-    ENSURE(c, c->gen_chain, sizeof(int) * (size_t)(n_chains + 1));
+    ENSURE(c, c->gen_chain, sizeof(int) * (size_t)(cap.n_chains + 1));
     ENSURE(c, c->shuf, sizeof(int) * (3 * SHUF_NCLS + 1) * (size_t)(cap.list_cap + 1));
     ENSURE(c, c->means, sizeof(double) * (size_t)cap.seg_cap);
     ENSURE(c, c->seed312, sizeof(uint64_t) * 312);
     ENSURE(c, c->dev, sizeof(Dev));
     if (p->hybrid) ENSURE(c, c->tailp, sizeof(double) * 100 * (size_t)cap.list_cap);  // tailp quadrature terms per new segment
 
-    setup_mark("buffers");
     // arenas: sized from the workload, bounded by what the device has left
     const long long per_perm_max = 3 * Nmax + 64;
     long long want_arena = std::min<long long>(24LL * 4096 * std::max<long long>(N, 1), 32LL << 30) / 8;
     want_arena = std::max<long long>(want_arena, 16 * per_perm_max);
     want_arena = std::max<long long>(want_arena, (64LL << 20) / 8);
     const bool shared_stream = mt && !p->chain;
+    cap.shared_stream = shared_stream;
     long long want_draws = (mt && !shared_stream) ? std::max<long long>(want_arena / 3, 8 * (Nmax + 312)) : 1;
     // shared raw MT stream (chain == 0): as long as the largest consumption of any one unit
     // shared raw MT stream (chain == 0): a ring of 2^k words (default 16 GB, CBS_GPU_STREAM_MB) + a mirror of its first words
@@ -488,7 +520,7 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
         size_t free_b = 0, total_b = 0;
         CUDA_TRY(c, cudaMemGetInfo(&free_b, &total_b));
         const size_t have = c->arena.cap + c->draws0.cap + c->draws1.cap + c->stream_buf.cap;
-        const double budget = c->mem_fraction * (double)(free_b + have);
+        const double budget = kMemFraction * (double)(free_b + have);
         const double need = 8.0 * ((double)want_arena + 2.0 * (double)want_draws + (double)want_stream);
         if (need > budget) {
             const double f = budget / need;
@@ -510,9 +542,16 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     }
     cap.arena_cap = (long long)(c->arena.cap / 8);
     cap.draws_cap = (mt && !shared_stream) ? (long long)(std::min(c->draws0.cap, c->draws1.cap) / 8) : 0;
+    cap.stream_ring = stream_ring; cap.stream_mirror = stream_mirror;
+    return CBS_GPU_OK;
+}
 
-    setup_mark("arenas");
-    // ---- device state ---------------------------------------------------------------------
+// run_cbs stage 2: the device state of the call (Dev), its upload, the weights check and the MT engines
+int init_device_state(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* unit_ids, int n_units,
+                      const cbs_gpu_params* p, const uint64_t* mt_next312, bool weighted, const ApiMode& api, const RunCaps& cap,
+                      Dev& hD) {
+    cudaStream_t st = c->stream;
+    const long long N = cap.N;
     memset(&hD, 0, sizeof(hD));
     hD.x = c->x.as<double>();
     hD.unit_off = c->unit_off.as<long long>();
@@ -520,7 +559,7 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     hD.n_units = n_units;
     hD.prm.alpha = p->alpha; hD.prm.nperm = p->nperm; hD.prm.hybrid = p->hybrid; hD.prm.min_width = p->min_width;
     hD.prm.kmax = p->kmax; hD.prm.nmin = p->nmin; hD.prm.eta = p->eta; hD.prm.tol = p->tol; hD.prm.ibin = p->ibin;
-    hD.prm.rng_mode = mt ? RNG_MT : RNG_PHILOX; hD.prm.chain = p->chain ? 1 : 0; hD.prm.seed = p->seed;
+    hD.prm.rng_mode = cap.mt ? RNG_MT : RNG_PHILOX; hD.prm.chain = p->chain ? 1 : 0; hD.prm.seed = p->seed;
     hD.prm.first_batch = p->first_batch > 0 ? p->first_batch : 256;
     hD.prm.max_batch = p->max_batch > 0 ? p->max_batch : 4096;
     // a batch needs one rejection flag per permutation: never ask for more than the flag table holds (it would be deferred forever)
@@ -534,7 +573,7 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     hD.tasks = c->tasks.as<Task>(); hD.task_cap = cap.task_cap; hD.free_ring = c->ring.as<int>();
     hD.free_head = 0; hD.free_tail = (unsigned)cap.task_cap;
     hD.active[0] = c->act0.as<int>(); hD.active[1] = c->act1.as<int>(); hD.list_cap = cap.list_cap;
-    hD.chains = c->chains.as<Chain>(); hD.n_chains = n_chains;
+    hD.chains = c->chains.as<Chain>(); hD.n_chains = cap.n_chains;
     hD.units_started = 0; hD.max_live = cap.max_live;
     hD.segs = c->segs.as<SegRec>(); hD.seg_cap = cap.seg_cap;
     hD.splits = c->splits.as<SplitRec>(); hD.split_cap = cap.split_cap;
@@ -551,13 +590,13 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     }
     hD.item_uprefix = c->shuf.as<int>() + (size_t)(2 * SHUF_NCLS) * (cap.list_cap + 1);
     for (int k = 0; k < SHUF_NCLS; ++k) hD.shuf_p0[k] = c->shuf.as<int>() + (size_t)(2 * SHUF_NCLS + 1 + k) * (cap.list_cap + 1);
-    hD.shared_stream = shared_stream ? 1 : 0;
+    hD.shared_stream = cap.shared_stream ? 1 : 0;
     hD.stream = c->stream_buf.as<uint64_t>();
-    hD.stream_cap = stream_ring; hD.stream_mask = stream_ring - 1; hD.stream_mirror = stream_mirror; hD.stream_lo = 0;
+    hD.stream_cap = cap.stream_ring; hD.stream_mask = cap.stream_ring - 1; hD.stream_mirror = cap.stream_mirror; hD.stream_lo = 0;
     hD.stream_len = 312; hD.stream_target = 312; hD.stream_target_prev = 312;
     hD.jump_polys = nullptr;
     hD.span_max = 1LL << 40;
-    if (shared_stream && (long long)Nmax * hD.prm.first_batch > mtjump::SEG && !env_ll("CBS_GPU_NO_JUMP", 0)) {
+    if (cap.shared_stream && (long long)cap.Nmax * hD.prm.first_batch > mtjump::SEG) {
         // parallel generation of the one stream: table of x^(c*S) mod phi, built once per process
         if (!c->jump_ready) {
             const mtjump::Table& T = mtjump::table();
@@ -571,7 +610,7 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
         if (c->jump_ready) { hD.jump_polys = c->jump.as<uint64_t>(); hD.span_max = (long long)mtjump::NSEG * mtjump::SEG; }
     }
     hD.profile = c->counting ? 1 : 0;
-    hD.shuf_arena = 1;  // decided below (cluster shuffle available?) and patched on the device before the first round
+    hD.shuf_arena = 1;  // decided by configure_round (cluster shuffle available?) and patched on the device before the first round
     hD.no_early = env_ll("CBS_GPU_NO_EARLY", 0) ? 1 : 0;
     hD.obs_slices = obs_slice_cap();
     if (weighted) {
@@ -595,21 +634,36 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     }
     Dev* dD = c->dev.as<Dev>();
     if (api.mode == 2 && N) CUDA_TRY(c, cudaMemcpyAsync(c->cur.p, c->x.p, sizeof(double) * (size_t)N, cudaMemcpyDeviceToDevice, st));  // no k_prep in this mode
-    if (mt) {
+    if (cap.mt) {
         uint64_t next[312];
         if (mt_next312) memcpy(next, mt_next312, sizeof(next)); else mt_seed_next312(p->seed, next);
         CUDA_TRY(c, cudaMemcpyAsync(c->seed312.p, next, sizeof(next), cudaMemcpyHostToDevice, st));
         CUDA_TRY(c, cudaStreamSynchronize(st));
-        k_init_chains<<<std::min(std::max(1, n_chains), 1024), 128, 0, st>>>(dD, c->seed312.as<uint64_t>());
-        if (shared_stream) {  // positions 0..311 (and their mirror)
+        k_init_chains<<<std::min(std::max(1, cap.n_chains), 1024), 128, 0, st>>>(dD, c->seed312.as<uint64_t>());
+        if (cap.shared_stream) {  // positions 0..311 (and their mirror)
             CUDA_TRY(c, cudaMemcpyAsync(c->stream_buf.p, next, sizeof(next), cudaMemcpyHostToDevice, st));
-            CUDA_TRY(c, cudaMemcpyAsync(c->stream_buf.as<uint64_t>() + stream_ring, next, sizeof(next), cudaMemcpyHostToDevice, st));
+            CUDA_TRY(c, cudaMemcpyAsync(c->stream_buf.as<uint64_t>() + cap.stream_ring, next, sizeof(next), cudaMemcpyHostToDevice, st));
         }
         CUDA_TRY(c, cudaStreamSynchronize(st));
     }
+    return CBS_GPU_OK;
+}
 
-    setup_mark("device state");
-    // ---- scan kernel configuration ------------------------------------------------------------
+// run_cbs stage 3: every launch configuration of the round, fixed for the call
+int configure_round(cbs_gpu_ctx* c, const cbs_gpu_params* p, bool weighted, const RunCaps& cap, Dev& hD, RoundConfig& r) {
+    memset(&r, 0, sizeof(r));
+    r.dD = c->dev.as<Dev>();
+    // profiling bit 2: every kernel on the one stream, so that per-launch event times do not overlap (roofline time base)
+    r.st = c->stream;
+    r.gen = c->serial ? r.st : c->gen_stream;
+    for (int k = 0; k < 5; ++k) r.side[k] = c->serial ? r.st : c->side[k];
+    r.weighted = weighted; r.mt = cap.mt; r.shared_stream = cap.shared_stream; r.jump = hD.jump_polys != nullptr;
+    r.hybrid = p->hybrid != 0; r.ibin = p->ibin != 0; r.counting = c->counting;
+    r.n_chains = cap.n_chains;
+    r.tailp = c->tailp.p;
+    const long long Nmax = cap.Nmax;
+
+    // scan kernels
     ScanLayout lay;
     lay.nb_max = block_count((int)std::max<long long>(Nmax, 1)) + 2;
     int scan_occ = 1, obs_occ = 1;
@@ -619,213 +673,203 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     if (!pick_scan_warps(c, lay, &scan_occ, (const void*)k_scan_perm<false>) ||
         !pick_scan_warps(c, lay_obs, &obs_occ, (const void*)k_scan_obs<false>))
         return fail(c, CBS_GPU_ERR_UNSUPPORTED, "segment too long for the scan kernel's shared memory");
-    const bool scan_prof = hD.profile != 0;
-    const int obs_grid = c->sm_count * obs_occ;
-    const size_t wscan_smem = ((sizeof(WScanSmem) + 15) & ~(size_t)15) + (size_t)lay.nb_max * (2 * sizeof(double) + 3 * sizeof(int)) + 16;
-    const int scan_grid = c->sm_count * scan_occ;
-    const size_t bscan_smem = ((sizeof(BinSmem) + 15) & ~(size_t)15) + (size_t)lay.nb_max * (2 * sizeof(double) + 3 * sizeof(int)) + 16;
-    if ((weighted && wscan_smem > c->smem_optin) || (p->ibin && bscan_smem > c->smem_optin))
+    r.lay = lay; r.lay_obs = lay_obs;
+    r.obs_grid = c->sm_count * obs_occ;
+    r.scan_grid = c->sm_count * scan_occ;
+    r.wscan_smem = ((sizeof(WScanSmem) + 15) & ~(size_t)15) + (size_t)lay.nb_max * (2 * sizeof(double) + 3 * sizeof(int)) + 16;
+    r.bscan_smem = ((sizeof(BinSmem) + 15) & ~(size_t)15) + (size_t)lay.nb_max * (2 * sizeof(double) + 3 * sizeof(int)) + 16;
+    if ((weighted && r.wscan_smem > c->smem_optin) || (p->ibin && r.bscan_smem > c->smem_optin))
         return fail(c, CBS_GPU_ERR_UNSUPPORTED, "segment too long for the scan kernel's shared memory");
 
     // shared-memory shuffle kernel, one launch per segment-length class present in this call
-    int shuf_occ[SHUF_CL2]; bool shuf_on[SHUF_CL2];
     for (int cls = 0; cls < SHUF_CL2; ++cls) {
-        shuf_on[cls] = (cls == 0) || Nmax > shuffle_class_max(cls - 1);  // no unit is long enough otherwise
-        shuf_occ[cls] = shuf_on[cls] ? shuffle_occupancy(cls) : 1;
+        r.shuf_on[cls] = (cls == 0) || Nmax > shuffle_class_max(cls - 1);  // no unit is long enough otherwise
+        r.shuf_occ[cls] = r.shuf_on[cls] ? shuffle_occupancy(cls) : 1;
     }
-    const bool l2_shuffle_on = Nmax > shuffle_class_max(SHUF_CL2 - 1);
+    r.l2_shuffle_on = Nmax > shuffle_class_max(SHUF_CL2 - 1);
     // segments > 65535 markers: a cluster of 2, 4 or 8 CTAs per permutation shares last[] through distributed shared
-    // memory; units too long even for that (or CBS_GPU_SHUF_CLUSTER=0) fall back to k_perm (index arrays in the arena)
-    int cl_R = 0, cl_grid = 0, cl2_grid = 0;
-    const int cl_hbits = 12;
-    size_t cl_smem = 0, cl2_smem = 0;
-    auto cluster_fit_l = [&](int R, long long nmax, size_t* smem_out) -> int { return cluster_fit(c, R, nmax, cl_hbits, smem_out); };
-    if (l2_shuffle_on && env_ll("CBS_GPU_SHUF_CLUSTER", 1)) {
+    // memory; units too long even for that fall back to k_perm (index arrays in the arena)
+    if (r.l2_shuffle_on) {
         if (Nmax > SHUF_CL2_MAX) {
-            for (int R : {4, 8}) { cl_grid = cluster_fit_l(R, Nmax, &cl_smem); if (cl_grid) { cl_R = R; break; } }
-        } else cl_R = -1;  // nothing longer than the cluster-of-2 class
-        if (cl_R) cl2_grid = cluster_fit_l(2, std::min<long long>(Nmax, SHUF_CL2_MAX), &cl2_smem);
-        if (cl_R < 0) { cl_R = cl2_grid ? 2 : 0; }
+            for (int R : {4, 8}) { r.cl_grid = cluster_fit(c, R, Nmax, kClusterHbits, &r.cl_smem); if (r.cl_grid) { r.cl_R = R; break; } }
+        } else r.cl_R = -1;  // nothing longer than the cluster-of-2 class
+        if (r.cl_R) r.cl2_grid = cluster_fit(c, 2, std::min<long long>(Nmax, SHUF_CL2_MAX), kClusterHbits, &r.cl2_smem);
+        if (r.cl_R < 0) { r.cl_R = r.cl2_grid ? 2 : 0; }
     }
-    static const int kShufTimer[SHUF_CL2] = {K_SHUF0, K_SHUF1, K_SHUF2, K_SHUF2, K_SHUF3, K_SHUF3};
-
-    if (cl_R) {
+    if (r.cl_R) {
         hD.shuf_arena = 0;
-        hD.shuf_cl2 = cl2_grid ? 1 : 0;
-        CUDA_TRY(c, cudaMemcpyAsync((char*)dD + offsetof(Dev, shuf_arena), &hD.shuf_arena, sizeof(int), cudaMemcpyHostToDevice, st));
-        CUDA_TRY(c, cudaMemcpyAsync((char*)dD + offsetof(Dev, shuf_cl2), &hD.shuf_cl2, sizeof(int), cudaMemcpyHostToDevice, st));
+        hD.shuf_cl2 = r.cl2_grid ? 1 : 0;
+        cudaStream_t st = c->stream;
+        CUDA_TRY(c, cudaMemcpyAsync((char*)r.dD + offsetof(Dev, shuf_arena), &hD.shuf_arena, sizeof(int), cudaMemcpyHostToDevice, st));
+        CUDA_TRY(c, cudaMemcpyAsync((char*)r.dD + offsetof(Dev, shuf_cl2), &hD.shuf_cl2, sizeof(int), cudaMemcpyHostToDevice, st));
         CUDA_TRY(c, cudaStreamSynchronize(st));
     }
 
     int chain_occ = 4;
     if ((weighted ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(&chain_occ, k_chain<true>, 32 * (1 + CP_STAT_WARPS), 0)
                   : cudaOccupancyMaxActiveBlocksPerMultiprocessor(&chain_occ, k_chain<false>, 32 * (1 + CP_STAT_WARPS), 0)) != cudaSuccess) { cudaGetLastError(); chain_occ = 4; }
-    chain_occ = std::max(1, chain_occ);
+    r.chain_occ = std::max(1, chain_occ);
+    return CBS_GPU_OK;
+}
 
-    setup_mark("launch configuration");
-    // ---- rounds -------------------------------------------------------------------------------
-    *c->h_done = 0;
-    const int G = (int)std::min<long long>(64, std::max<long long>(1, env_ll("CBS_GPU_ROUND_GROUP", 16)));
-    // rounds per group; two groups are kept in flight, so the host is 16-32 rounds ahead of the device and its scheduling
-    // jitter cannot starve the GPU; the rounds enqueued beyond the last one find D->done set and every kernel returns at once
-    const bool debug = env_ll("CBS_GPU_DEBUG", 0) != 0;
-    int groups_in_flight = 0, rounds = 0;
-    int gi = 0;
-    // One round = one fork-join of launches over the main stream, the side streams and the generator stream, and every launch
-    // configuration is fixed for the call.  The round is therefore captured ONCE as the body of a WHILE node of a CUDA graph
-    // whose condition the scheduler kernel keeps at 1 until the work list is empty: the whole call is one graph launch, the
-    // device runs exactly the rounds it needs and the host plays no part between them.  The instantiated graph is kept in
-    // the context and reused by later calls with the same configuration.  Event-timed profiling, CBS_GPU_DEBUG and
-    // CBS_GPU_GRAPH=0 enqueue the rounds from the host instead, in groups with a done flag polled in between.
-    cudaGraphConditionalHandle loop_handle = 0;
-    int looped = 0;
-    auto enqueue_round = [&]() {
-        bool ahead_pending = false;
-        // One round.  Dependencies: everything after k_sched; shuffles after the generator;
-        // k_prefix after the shuffles; k_scan_perm after k_prefix; k_scan_obs after k_prep; next k_sched after all.
-        // A task's permutations are planned in a later round than its observed scan (Sched::step), so neither scan
-        // of a round reads what the other writes, and the observed scans run beside the shuffles.
-        //   main : sched, gen, [shuffle classes], prefix, scan_perm
-        //   side0: prep, scan_obs  side1: edgeprep, edgeperm
-        //   side2, side3: other shuffle classes      side4: shuffle of segments > 65535 markers
-        { LaunchTimer t(c, K_SCHED); k_sched<<<1, 256, 0, st>>>(dD, c->d_done, loop_handle, looped); }
-        cudaEventRecord(c->ev_sched, st);
-        cudaStreamWaitEvent(side[0], c->ev_sched, 0);
-        { LaunchTimer t(c, K_PREP, side[0]); k_tables<<<dim3(16, 64), 256, 0, side[0]>>>(dD); if (weighted) { k_wprep<<<c->sm_count * 8, 32, 0, side[0]>>>(dD); k_wtables<<<c->sm_count * 2, 256, 0, side[0]>>>(dD); c->launches++; if (p->hybrid) { k_wdelta<<<c->sm_count * 2, 32, 0, side[0]>>>(dD); c->launches++; } } else k_prep<<<c->sm_count * 8, 32, 0, side[0]>>>(dD); c->launches++; }
-        const bool scan_split = !weighted && !p->ibin;
-        if (scan_split) { LaunchTimer t(c, K_SCAN, side[0]); launch_scan(true, scan_prof, obs_grid, lay_obs, side[0], dD); }
-        cudaEventRecord(c->ev_side[0], side[0]);
-        cudaStreamWaitEvent(side[1], c->ev_sched, 0);
-        { LaunchTimer t(c, K_EDGEPREP, side[1]); if (weighted) k_wedgeprep<<<c->sm_count * 4, 32, 0, side[1]>>>(dD); else k_edgeprep<<<c->sm_count * 4, 32, 0, side[1]>>>(dD); }
-        if (mt) {
-            LaunchTimer t(c, K_GEN);
-            if (shared_stream) {
-                k_gen_lead<<<1, 192, 0, st>>>(dD, 0);
-                if (hD.jump_polys) { k_gen_par<<<GEN_NSEG, 320, 0, st>>>(dD); c->launches++; }
-            } else k_gen<<<std::min(std::max(1, n_chains), c->sm_count * 4), 192, 0, st>>>(dD);
+// run_cbs stage 4: one round = one fork-join of launches over the main stream, the side streams and the generator stream.
+// `looped`: the round is being captured as the body of the call graph's WHILE node (k_sched sets its condition).
+void enqueue_round(cbs_gpu_ctx* c, const RoundConfig& r, cudaGraphConditionalHandle loop_handle, int looped) {
+    static const int kShufTimer[SHUF_CL2] = {K_SHUF0, K_SHUF1, K_SHUF2, K_SHUF2, K_SHUF3, K_SHUF3};
+    cudaStream_t st = r.st;
+    const cudaStream_t* side = r.side;
+    Dev* dD = r.dD;
+    const int sm = c->sm_count;
+    bool ahead_pending = false;
+    // Dependencies: everything after k_sched; shuffles after the generator;
+    // k_prefix after the shuffles; k_scan_perm after k_prefix; k_scan_obs after k_prep; next k_sched after all.
+    // A task's permutations are planned in a later round than its observed scan (Sched::step), so neither scan
+    // of a round reads what the other writes, and the observed scans run beside the shuffles.
+    //   main : sched, gen, [shuffle classes], prefix, scan_perm
+    //   side0: prep, scan_obs  side1: edgeprep, edgeperm
+    //   side2, side3: other shuffle classes      side4: shuffle of segments > 65535 markers
+    { LaunchTimer t(c, K_SCHED); k_sched<<<1, 256, 0, st>>>(dD, c->d_done, loop_handle, looped); }
+    cudaEventRecord(c->ev_sched, st);
+    cudaStreamWaitEvent(side[0], c->ev_sched, 0);
+    { LaunchTimer t(c, K_PREP, side[0]); k_tables<<<dim3(16, 64), 256, 0, side[0]>>>(dD); if (r.weighted) { k_wprep<<<sm * 8, 32, 0, side[0]>>>(dD); k_wtables<<<sm * 2, 256, 0, side[0]>>>(dD); c->launches++; if (r.hybrid) { k_wdelta<<<sm * 2, 32, 0, side[0]>>>(dD); c->launches++; } } else k_prep<<<sm * 8, 32, 0, side[0]>>>(dD); c->launches++; }
+    const bool scan_split = !r.weighted && !r.ibin;
+    if (scan_split) { LaunchTimer t(c, K_SCAN, side[0]); launch_scan(true, r.counting, r.obs_grid, r.lay_obs, side[0], dD); }
+    cudaEventRecord(c->ev_side[0], side[0]);
+    cudaStreamWaitEvent(side[1], c->ev_sched, 0);
+    { LaunchTimer t(c, K_EDGEPREP, side[1]); if (r.weighted) k_wedgeprep<<<sm * 4, 32, 0, side[1]>>>(dD); else k_edgeprep<<<sm * 4, 32, 0, side[1]>>>(dD); }
+    if (r.mt) {
+        LaunchTimer t(c, K_GEN);
+        if (r.shared_stream) {
+            k_gen_lead<<<1, 192, 0, st>>>(dD, 0);
+            if (r.jump) { k_gen_par<<<GEN_NSEG, 320, 0, st>>>(dD); c->launches++; }
+        } else k_gen<<<std::min(std::max(1, r.n_chains), sm * 4), 192, 0, st>>>(dD);
+    }
+    cudaEventRecord(c->ev_gen, st);
+    // the edge permutations read this round's draws (plan_edge asked the generator for them): after the generator
+    if (r.mt) cudaStreamWaitEvent(side[1], c->ev_gen, 0);
+    { LaunchTimer t(c, K_EDGEPERM, side[1]); if (r.weighted) k_wedgeperm<<<sm * 4, 128, 0, side[1]>>>(dD); else k_edgeperm<<<sm * 4, 128, 0, side[1]>>>(dD); }
+    cudaEventRecord(c->ev_side[1], side[1]);
+    if (r.mt && r.shared_stream && r.jump) {
+        // generate ahead for the next round, next to this round's shuffles and scan
+        cudaStreamWaitEvent(r.gen, c->ev_gen, 0);
+        k_gen_lead<<<1, 192, 0, r.gen>>>(dD, 1);
+        k_gen_par<<<GEN_NSEG, 320, 0, r.gen>>>(dD);
+        c->launches += 2;
+        cudaEventRecord(c->ev_ahead, r.gen);
+        ahead_pending = true;
+    }
+    // shuffles: classes alternate between the main stream and three side streams so that they run
+    // concurrently (each class is latency bound on its own); the longest present class goes first
+    bool used_side[5] = {false, false, false, false, false};
+    {
+        int slot = 0;
+        if (r.l2_shuffle_on) {
+            cudaStream_t ss = side[4];
+            cudaStreamWaitEvent(ss, c->ev_gen, 0);
+            used_side[4] = true;
+            LaunchTimer t(c, K_PERM, ss);
+            if (r.cl_R == 4 || r.cl_R == 8) launch_shuffle_cluster(dD, r.cl_R, SHUF_GLOBAL, kClusterHbits, r.cl_grid, r.cl_smem, ss, r.mt);
+            else if (r.cl_R == 0) k_perm<<<sm * 8, 128, 0, ss>>>(dD);
+            if (r.cl2_grid) { launch_shuffle_cluster(dD, 2, SHUF_CL2, kClusterHbits, r.cl2_grid, r.cl2_smem, ss, r.mt); c->launches++; }
         }
-        cudaEventRecord(c->ev_gen, st);
-        // the edge permutations read this round's draws (plan_edge asked the generator for them): after the generator
-        if (mt) cudaStreamWaitEvent(side[1], c->ev_gen, 0);
-        { LaunchTimer t(c, K_EDGEPERM, side[1]); if (weighted) k_wedgeperm<<<c->sm_count * 4, 128, 0, side[1]>>>(dD); else k_edgeperm<<<c->sm_count * 4, 128, 0, side[1]>>>(dD); }
-        cudaEventRecord(c->ev_side[1], side[1]);
-        if (mt && shared_stream && hD.jump_polys) {
-            // generate ahead for the next round, next to this round's shuffles and scan
-            cudaStreamWaitEvent(gen_stream, c->ev_gen, 0);
-            k_gen_lead<<<1, 192, 0, gen_stream>>>(dD, 1);
-            k_gen_par<<<GEN_NSEG, 320, 0, gen_stream>>>(dD);
-            c->launches += 2;
-            cudaEventRecord(c->ev_ahead, gen_stream);
-            ahead_pending = true;
-        }
-        // shuffles: classes alternate between the main stream and three side streams so that they run
-        // concurrently (each class is latency bound on its own); the longest present class goes first
-        bool used_side[5] = {false, false, false, false, false};
-        {
-            int slot = 0;
-            if (l2_shuffle_on) {
-                cudaStream_t ss = side[4];
-                cudaStreamWaitEvent(ss, c->ev_gen, 0);
-                used_side[4] = true;
-                LaunchTimer t(c, K_PERM, ss);
-                if (cl_R == 4 || cl_R == 8) launch_shuffle_cluster(dD, cl_R, SHUF_GLOBAL, cl_hbits, cl_grid, cl_smem, ss, mt);
-                else if (cl_R == 0) k_perm<<<c->sm_count * 8, 128, 0, ss>>>(dD);
-                if (cl2_grid) { launch_shuffle_cluster(dD, 2, SHUF_CL2, cl_hbits, cl2_grid, cl2_smem, ss, mt); c->launches++; }
-            }
-            for (int cls = SHUF_CL2 - 1; cls >= 0; --cls) {
-                if (!shuf_on[cls]) continue;
-                const int where = slot++ % 3;  // 0 = main stream, 1,2 = side[2], side[3]
-                cudaStream_t ss = where == 0 ? st : side[1 + where];
-                if (where != 0 && !used_side[1 + where]) { cudaStreamWaitEvent(ss, c->ev_gen, 0); used_side[1 + where] = true; }
-                LaunchTimer t(c, kShufTimer[cls], ss);
-                launch_shuffle(dD, cls, c->sm_count * shuf_occ[cls], ss, mt);
-            }
-        }
-        for (int k = 2; k < 5; ++k) if (used_side[k]) { cudaEventRecord(c->ev_side[k], side[k]); cudaStreamWaitEvent(st, c->ev_side[k], 0); }
-        { LaunchTimer t(c, K_PREFIX); if (weighted && p->hybrid) { k_wssq<<<c->sm_count * 8, 128, 0, st>>>(dD); c->launches++; } if (weighted) k_chain<true><<<c->sm_count * chain_occ, 32 * (1 + CP_STAT_WARPS), 0, st>>>(dD); else k_chain<false><<<c->sm_count * chain_occ, 32 * (1 + CP_STAT_WARPS), 0, st>>>(dD); }
-        if (!scan_split) cudaStreamWaitEvent(st, c->ev_side[0], 0);
-        { LaunchTimer t(c, K_SCAN);
-          if (weighted) {
-              k_wscan<1><<<c->sm_count * 4, 256, wscan_smem, st>>>(dD, lay.nb_max);   // observed rows, sliced over CTAs
-              k_wobs_fin<<<8, 128, 0, st>>>(dD);
-              k_wscan<0><<<c->sm_count * 4, 256, wscan_smem, st>>>(dD, lay.nb_max);   // permutation rows
-              c->launches += 2;
-          }
-          else if (p->ibin) k_scan_binary<<<c->sm_count * 4, 256, bscan_smem, st>>>(dD, lay.nb_max);
-          else launch_scan(false, scan_prof, scan_grid, lay, st, dD); }
-        if (scan_split) cudaStreamWaitEvent(st, c->ev_side[0], 0);  // the tail probabilities read the observed statistics
-        if (p->hybrid) {
-            if (weighted) k_whscan<<<c->sm_count * 4, 256, 0, st>>>(dD); else k_hscan<<<c->sm_count * 4, 256, 0, st>>>(dD);
-            k_tailp_terms<<<c->sm_count * 8, 128, 0, st>>>(dD, c->tailp.as<double>());
-            k_tailp_sum<<<c->sm_count, 64, 0, st>>>(dD, c->tailp.as<double>());
-            c->launches += 3;
-        }
-        cudaStreamWaitEvent(st, c->ev_side[1], 0);
-        if (ahead_pending) cudaStreamWaitEvent(st, c->ev_ahead, 0);  // the next k_sched plans on the extended stream
-    };
-    const bool use_graph = !c->profiling && !debug && env_ll("CBS_GPU_GRAPH", 1) != 0;
-    unsigned long long launches_per_round = 0;
-    cudaGraphExec_t call_exec = nullptr;
-    if (use_graph) {
-        std::vector<unsigned char> key;
-        auto put = [&](const void* v, size_t nbytes) { const unsigned char* b = (const unsigned char*)v; key.insert(key.end(), b, b + nbytes); };
-#define KEY_POD(v) put(&(v), sizeof(v))
-        const int flags[7] = {weighted ? 1 : 0, mt ? 1 : 0, shared_stream ? 1 : 0, hD.jump_polys ? 1 : 0, p->hybrid ? 1 : 0, l2_shuffle_on ? 1 : 0,
-                              p->ibin ? 1 : 0};
-        KEY_POD(dD); KEY_POD(st); KEY_POD(flags); KEY_POD(n_chains); KEY_POD(shuf_occ); KEY_POD(shuf_on); KEY_POD(cl_R); KEY_POD(cl_grid);
-        KEY_POD(cl2_grid); KEY_POD(cl_smem); KEY_POD(cl2_smem); KEY_POD(chain_occ); KEY_POD(scan_grid); KEY_POD(obs_grid); KEY_POD(scan_prof);
-        KEY_POD(wscan_smem); KEY_POD(bscan_smem); KEY_POD(lay); KEY_POD(lay_obs);
-        const void* tailp_ptr = c->tailp.p; KEY_POD(tailp_ptr);
-#undef KEY_POD
-        if (c->call_exec && key == c->call_key) {
-            call_exec = c->call_exec;
-            launches_per_round = c->round_launches;
-        } else {
-            if (c->call_exec) { cudaGraphExecDestroy(c->call_exec); c->call_exec = nullptr; }
-            const unsigned long long before = c->launches;
-            cudaGraph_t graph = nullptr;
-            cudaError_t ce = cudaGraphCreate(&graph, 0);
-            if (ce == cudaSuccess) ce = cudaGraphConditionalHandleCreate(&loop_handle, graph, 1, cudaGraphCondAssignDefault);
-            cudaGraphNodeParams wp = {cudaGraphNodeTypeConditional};
-            wp.conditional.handle = loop_handle;
-            wp.conditional.type = cudaGraphCondTypeWhile;
-            wp.conditional.size = 1;
-            cudaGraphNode_t wnode = nullptr;
-            if (ce == cudaSuccess) ce = cudaGraphAddNode(&wnode, graph, nullptr, 0, &wp);
-            if (ce == cudaSuccess) {
-                looped = 1;
-                ce = cudaStreamBeginCaptureToGraph(st, wp.conditional.phGraph_out[0], nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed);
-                if (ce == cudaSuccess) {
-                    enqueue_round();
-                    ce = cudaStreamEndCapture(st, nullptr);
-                }
-                looped = 0;
-            }
-            launches_per_round = c->launches - before;
-            c->launches = before;
-            if (ce == cudaSuccess) ce = cudaGraphInstantiate(&call_exec, graph, 0);
-            if (graph) cudaGraphDestroy(graph);
-            if (ce != cudaSuccess) {
-                // (a driver without conditional nodes, or a capture that could not be closed: rounds are enqueued by the host)
-                cudaGetLastError();
-                call_exec = nullptr;
-                if (env_ll("CBS_GPU_GRAPH", 1) == 2) return fail(c, CBS_GPU_ERR_CUDA, std::string("call graph: ") + cudaGetErrorString(ce));
-            } else {
-                c->call_exec = call_exec;
-                c->call_key = key;
-                c->round_launches = launches_per_round;
-            }
+        for (int cls = SHUF_CL2 - 1; cls >= 0; --cls) {
+            if (!r.shuf_on[cls]) continue;
+            const int where = slot++ % 3;  // 0 = main stream, 1,2 = side[2], side[3]
+            cudaStream_t ss = where == 0 ? st : side[1 + where];
+            if (where != 0 && !used_side[1 + where]) { cudaStreamWaitEvent(ss, c->ev_gen, 0); used_side[1 + where] = true; }
+            LaunchTimer t(c, kShufTimer[cls], ss);
+            launch_shuffle(dD, cls, sm * r.shuf_occ[cls], ss, r.mt);
         }
     }
-    setup_mark("graph");
-    if (call_exec) {
-        CUDA_TRY(c, cudaGraphLaunch(call_exec, st));
+    for (int k = 2; k < 5; ++k) if (used_side[k]) { cudaEventRecord(c->ev_side[k], side[k]); cudaStreamWaitEvent(st, c->ev_side[k], 0); }
+    { LaunchTimer t(c, K_PREFIX); if (r.weighted && r.hybrid) { k_wssq<<<sm * 8, 128, 0, st>>>(dD); c->launches++; } if (r.weighted) k_chain<true><<<sm * r.chain_occ, 32 * (1 + CP_STAT_WARPS), 0, st>>>(dD); else k_chain<false><<<sm * r.chain_occ, 32 * (1 + CP_STAT_WARPS), 0, st>>>(dD); }
+    if (!scan_split) cudaStreamWaitEvent(st, c->ev_side[0], 0);
+    { LaunchTimer t(c, K_SCAN);
+      if (r.weighted) {
+          k_wscan<1><<<sm * 4, 256, r.wscan_smem, st>>>(dD, r.lay.nb_max);   // observed rows, sliced over CTAs
+          k_wobs_fin<<<8, 128, 0, st>>>(dD);
+          k_wscan<0><<<sm * 4, 256, r.wscan_smem, st>>>(dD, r.lay.nb_max);   // permutation rows
+          c->launches += 2;
+      }
+      else if (r.ibin) k_scan_binary<<<sm * 4, 256, r.bscan_smem, st>>>(dD, r.lay.nb_max);
+      else launch_scan(false, r.counting, r.scan_grid, r.lay, st, dD); }
+    if (scan_split) cudaStreamWaitEvent(st, c->ev_side[0], 0);  // the tail probabilities read the observed statistics
+    if (r.hybrid) {
+        double* tailp = (double*)r.tailp;
+        if (r.weighted) k_whscan<<<sm * 4, 256, 0, st>>>(dD); else k_hscan<<<sm * 4, 256, 0, st>>>(dD);
+        k_tailp_terms<<<sm * 8, 128, 0, st>>>(dD, tailp);
+        k_tailp_sum<<<sm, 64, 0, st>>>(dD, tailp);
+        c->launches += 3;
+    }
+    cudaStreamWaitEvent(st, c->ev_side[1], 0);
+    if (ahead_pending) cudaStreamWaitEvent(st, c->ev_ahead, 0);  // the next k_sched plans on the extended stream
+}
+
+// run_cbs stage 5: the graph of the whole call.  Every launch configuration is fixed for the call, so the round is captured
+// ONCE as the body of a WHILE node of a CUDA graph whose condition the scheduler kernel keeps at 1 until the work list is
+// empty: the whole call is one graph launch, the device runs exactly the rounds it needs and the host plays no part between
+// them.  The instantiated graph is kept in the context and reused by later calls with the same round configuration.
+// *exec stays nullptr when the graph cannot be built: the rounds are then enqueued by the host.
+int call_graph(cbs_gpu_ctx* c, const RoundConfig& r, cudaGraphExec_t* exec) {
+    *exec = nullptr;
+    if (c->call_exec && memcmp(&r, &c->call_cfg, sizeof(r)) == 0) { *exec = c->call_exec; return CBS_GPU_OK; }
+    if (c->call_exec) { cudaGraphExecDestroy(c->call_exec); c->call_exec = nullptr; }
+    const unsigned long long before = c->launches;
+    cudaGraph_t graph = nullptr;
+    cudaGraphConditionalHandle loop_handle = 0;
+    cudaError_t ce = cudaGraphCreate(&graph, 0);
+    if (ce == cudaSuccess) ce = cudaGraphConditionalHandleCreate(&loop_handle, graph, 1, cudaGraphCondAssignDefault);
+    cudaGraphNodeParams wp = {cudaGraphNodeTypeConditional};
+    wp.conditional.handle = loop_handle;
+    wp.conditional.type = cudaGraphCondTypeWhile;
+    wp.conditional.size = 1;
+    cudaGraphNode_t wnode = nullptr;
+    if (ce == cudaSuccess) ce = cudaGraphAddNode(&wnode, graph, nullptr, 0, &wp);
+    if (ce == cudaSuccess) {
+        ce = cudaStreamBeginCaptureToGraph(r.st, wp.conditional.phGraph_out[0], nullptr, nullptr, 0, cudaStreamCaptureModeRelaxed);
+        if (ce == cudaSuccess) {
+            enqueue_round(c, r, loop_handle, 1);
+            ce = cudaStreamEndCapture(r.st, nullptr);
+        }
+    }
+    const unsigned long long launches_per_round = c->launches - before;
+    c->launches = before;
+    cudaGraphExec_t made = nullptr;
+    if (ce == cudaSuccess) ce = cudaGraphInstantiate(&made, graph, 0);
+    if (graph) cudaGraphDestroy(graph);
+    if (ce != cudaSuccess) {
+        // (a driver without conditional nodes, or a capture that could not be closed: rounds are enqueued by the host)
+        cudaGetLastError();
+        if (env_ll("CBS_GPU_GRAPH", 1) == 2) return fail(c, CBS_GPU_ERR_CUDA, std::string("call graph: ") + cudaGetErrorString(ce));
+        return CBS_GPU_OK;
+    }
+    c->call_exec = made;
+    memcpy(&c->call_cfg, &r, sizeof(r));  // padding included: the next call compares with memcmp
+    c->round_launches = launches_per_round;
+    *exec = made;
+    return CBS_GPU_OK;
+}
+
+// rounds per group of the host-enqueued path; two groups are kept in flight, so the host is 16-32 rounds ahead of the
+// device and its scheduling jitter cannot starve the GPU; the rounds enqueued beyond the last one find D->done set and
+// every kernel returns at once
+const int kRoundGroup = 16;
+
+// run_cbs stage 6: run the rounds until the scheduler is done, then read the device state back into hD.  With `exec` the
+// call is one graph launch; otherwise (event-timed profiling, CBS_GPU_DEBUG, CBS_GPU_GRAPH=0) the host enqueues the
+// rounds in groups and polls the done flag in between.
+int drive_rounds(cbs_gpu_ctx* c, const RoundConfig& r, cudaGraphExec_t exec, bool debug, Dev& hD) {
+    cudaStream_t st = r.st;
+    *c->h_done = 0;
+    if (exec) {
+        CUDA_TRY(c, cudaGraphLaunch(exec, st));
         CUDA_TRY(c, cudaStreamSynchronize(st));
         if (*(volatile int*)c->h_done == 0) return fail(c, CBS_GPU_ERR_CUDA, "the call graph ended before the scheduler was done");
     }
-    for (; !call_exec;) {
-        for (int r = 0; r < G; ++r) {
-            enqueue_round();
+    int groups_in_flight = 0, rounds = 0, gi = 0;
+    for (; !exec;) {
+        for (int k = 0; k < kRoundGroup; ++k) {
+            enqueue_round(c, r, 0, 0);
             ++rounds;
         }
         CUDA_TRY(c, cudaEventRecord(c->grp[gi], st));
@@ -837,7 +881,7 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
             if (*(volatile int*)c->h_done != 0) break;
             if (debug) {
                 Dev snap;
-                cudaMemcpy(&snap, dD, sizeof(Dev), cudaMemcpyDeviceToHost);  // synchronises: debugging only
+                cudaMemcpy(&snap, r.dD, sizeof(Dev), cudaMemcpyDeviceToHost);  // synchronises: debugging only
                 fprintf(stderr, "[cbs_gpu] enq=%d round=%d live=%d items=%d perms=%d prep=%d edgeprep=%d edge=%d gen=%d segs=%d perms_done=%llu err=%d\n",
                         rounds, snap.round, snap.n_active[snap.cur_list], snap.n_items, snap.item_prefix ? -1 : 0, snap.n_prep,
                         snap.n_edgeprep, snap.n_edge, snap.n_gen, snap.n_segs, snap.stat_perms, snap.error);
@@ -847,37 +891,76 @@ int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* u
     }
     // everything that was enqueued (up to two groups of rounds, on the main, generator and side streams) has to be over before
     // anything is read back or an error is reported
-    for (int k = 0; k < 5; ++k) cudaStreamSynchronize(side[k]);
-    CUDA_TRY(c, cudaStreamSynchronize(gen_stream));
+    for (int k = 0; k < 5; ++k) cudaStreamSynchronize(r.side[k]);
+    CUDA_TRY(c, cudaStreamSynchronize(r.gen));
     CUDA_TRY(c, cudaStreamSynchronize(st));
     CUDA_TRY(c, cudaGetLastError());
-    CUDA_TRY(c, cudaMemcpy(&hD, dD, sizeof(Dev), cudaMemcpyDeviceToHost));
-    if (call_exec) c->launches += launches_per_round * (unsigned long long)std::max(1, hD.round);  // one body per scheduler round
-    if (hD.error) {
-        switch (hD.error) {
-        case ERR_TASK_CAP: return fail(c, CBS_GPU_ERR_CAPACITY, "pending-segment pool exhausted (raise CBS_GPU_TASK_CAP)");
-        case ERR_SEG_CAP: return fail(c, CBS_GPU_ERR_CAPACITY, "segment table exhausted (raise CBS_GPU_SEG_CAP)");
-        case ERR_SPLIT_CAP: return fail(c, CBS_GPU_ERR_CAPACITY, "split log exhausted");
-        case ERR_STALL: return fail(c, CBS_GPU_ERR_CUDA, "scheduler stalled: live segments but no work could be planned");
-        case ERR_STREAM_CAP: return fail(c, CBS_GPU_ERR_CAPACITY, "MT stream window smaller than one permutation (raise CBS_GPU_STREAM_MB)");
-        case ERR_ARENA: return fail(c, CBS_GPU_ERR_OOM, "permutation arena too small for one segment (raise CBS_GPU_ARENA_MB)");
-        case ERR_SELF_SPLIT:
-            return fail(c, CBS_GPU_ERR_UNSUPPORTED, "unit " + std::to_string(hD.err_unit) + ", segment [" + std::to_string(hD.err_lo) + ", " +
-                        std::to_string(hD.err_hi) + "): the split decision would re-create the segment (weights so uneven that "
-                        "the statistic is not finite); the reference would not terminate");
-        default: return fail(c, CBS_GPU_ERR_CUDA, "internal scheduler error " + std::to_string(hD.error));
-        }
+    CUDA_TRY(c, cudaMemcpy(&hD, r.dD, sizeof(Dev), cudaMemcpyDeviceToHost));
+    if (exec) c->launches += c->round_launches * (unsigned long long)std::max(1, hD.round);  // one body per scheduler round
+    return CBS_GPU_OK;
+}
+
+// run_cbs stage 7: the scheduler's error codes (Dev::error) as status codes and messages
+int scheduler_error(cbs_gpu_ctx* c, const Dev& hD) {
+    static const struct { int error, status; const char* msg; } kErrors[] = {
+        {ERR_TASK_CAP, CBS_GPU_ERR_CAPACITY, "pending-segment pool exhausted (raise CBS_GPU_TASK_CAP)"},
+        {ERR_SEG_CAP, CBS_GPU_ERR_CAPACITY, "segment table exhausted (raise CBS_GPU_SEG_CAP)"},
+        {ERR_SPLIT_CAP, CBS_GPU_ERR_CAPACITY, "split log exhausted"},
+        {ERR_STALL, CBS_GPU_ERR_CUDA, "scheduler stalled: live segments but no work could be planned"},
+        {ERR_STREAM_CAP, CBS_GPU_ERR_CAPACITY, "MT stream window smaller than one permutation (raise CBS_GPU_STREAM_MB)"},
+        {ERR_ARENA, CBS_GPU_ERR_OOM, "permutation arena too small for one segment (raise CBS_GPU_ARENA_MB)"},
+    };
+    for (const auto& e : kErrors) if (e.error == hD.error) return fail(c, e.status, e.msg);
+    if (hD.error == ERR_SELF_SPLIT)
+        return fail(c, CBS_GPU_ERR_UNSUPPORTED, "unit " + std::to_string(hD.err_unit) + ", segment [" + std::to_string(hD.err_lo) + ", " +
+                    std::to_string(hD.err_hi) + "): the split decision would re-create the segment (weights so uneven that "
+                    "the statistic is not finite); the reference would not terminate");
+    return fail(c, CBS_GPU_ERR_CUDA, "internal scheduler error " + std::to_string(hD.error));
+}
+
+int run_cbs(cbs_gpu_ctx* c, const std::vector<long long>& off, const uint64_t* unit_ids, int n_units,
+            const cbs_gpu_params* p, const uint64_t* mt_next312, bool weighted /* weights resident in c->wts */, Dev& hD,
+            const ApiMode& api = ApiMode()) {
+    // CBS_GPU_DEBUG_SETUP=1: host wall clock of the set-up phases on stderr
+    const bool setup_debug = getenv("CBS_GPU_DEBUG_SETUP") != nullptr;
+    auto setup_t0 = std::chrono::steady_clock::now();
+    auto setup_mark = [&](const char* what) {
+        if (!setup_debug) return;
+        const auto now = std::chrono::steady_clock::now();
+        fprintf(stderr, "[setup] %s %.3f ms\n", what, std::chrono::duration<double, std::milli>(now - setup_t0).count());
+        setup_t0 = now;
+    };
+    RunCaps cap;
+    int rc = size_call(c, off, n_units, p, weighted, api, cap);
+    if (rc) return rc;
+    setup_mark("buffers and arenas");
+    rc = init_device_state(c, off, unit_ids, n_units, p, mt_next312, weighted, api, cap, hD);
+    if (rc) return rc;
+    setup_mark("device state");
+    RoundConfig r;
+    rc = configure_round(c, p, weighted, cap, hD, r);
+    if (rc) return rc;
+    setup_mark("launch configuration");
+    const bool debug = env_ll("CBS_GPU_DEBUG", 0) != 0;
+    cudaGraphExec_t exec = nullptr;
+    if (!c->profiling && !debug && env_ll("CBS_GPU_GRAPH", 1) != 0) {
+        rc = call_graph(c, r, &exec);
+        if (rc) return rc;
     }
+    setup_mark("graph");
+    rc = drive_rounds(c, r, exec, debug, hD);
+    if (rc) return rc;
+    if (hD.error) return scheduler_error(c, hD);
     if (getenv("CBS_GPU_DEBUG_ROUNDS")) {
         fprintf(stderr, "[rounds] planned perms / markers per round:");
-        for (int r = 0; r < std::min(hD.round, 64); ++r) fprintf(stderr, " %d:%llu/%.1fM", r, hD.round_perms[r], hD.round_elems[r] * 1e-6);
+        for (int k = 0; k < std::min(hD.round, 64); ++k) fprintf(stderr, " %d:%llu/%.1fM", k, hD.round_perms[k], hD.round_elems[k] * 1e-6);
         fprintf(stderr, "\n");
         if (hD.shared_stream) fprintf(stderr, "[stream] words generated %.1fM, furthest word asked for %.1fM\n", hD.stream_len * 1e-6, hD.stream_target * 1e-6);
     }
     if (hD.n_segs > 0) {
         LaunchTimer t(c, K_MEANS);
-        if (weighted) k_wmeans<<<std::min(hD.n_segs, c->sm_count * 8), 32, 0, st>>>(dD, c->means.as<double>());
-        else k_means<<<std::min(hD.n_segs, c->sm_count * 8), 32, 0, st>>>(dD, c->means.as<double>());
+        if (weighted) k_wmeans<<<std::min(hD.n_segs, c->sm_count * 8), 32, 0, c->stream>>>(r.dD, c->means.as<double>());
+        else k_means<<<std::min(hD.n_segs, c->sm_count * 8), 32, 0, c->stream>>>(r.dD, c->means.as<double>());
     }
     CUDA_TRY(c, cudaGetLastError());
     return CBS_GPU_OK;
@@ -891,6 +974,28 @@ struct ResultOwner {
     std::vector<uint64_t> draws;
     std::vector<cbs_gpu_split> splits;
 };
+
+// point the public view of R at its vectors
+void publish(ResultOwner* R, int n_units) {
+    R->pub.n_units = n_units;
+    R->pub.n_segments = (int64_t)R->lengths.size();
+    R->pub.seg_offsets = R->seg_offsets.data();
+    R->pub.lengths = R->lengths.data();
+    R->pub.means = R->means.data();
+    R->pub.draws_consumed = R->draws.data();
+    R->pub.n_splits = (int64_t)R->splits.size();
+    R->pub.splits = R->splits.empty() ? nullptr : R->splits.data();
+}
+
+cbs_gpu_split to_split(const SplitRec& s) {
+    cbs_gpu_split o;
+    memset(&o, 0, sizeof(o));
+    o.unit = s.unit; o.lo = s.lo; o.hi = s.hi; o.ostat = s.ostat; o.iseg0 = s.iseg0; o.iseg1 = s.iseg1;
+    o.ncpt = s.ncpt; o.icpt0 = s.icpt0; o.icpt1 = s.icpt1; o.perms_run = s.perms_run; o.nrej = s.nrej;
+    o.exit_code = s.exit_code; o.called = s.called; o.e_nrej0 = s.e_nrej0; o.e_nrej1 = s.e_nrej1;
+    o.e_status0 = s.e_status0; o.e_status1 = s.e_status1;
+    return o;
+}
 
 int fetch_results(cbs_gpu_ctx* c, const Dev& hD, int n_units, bool want_splits, ResultOwner* R, const cbs_gpu_params* prm = nullptr,
                   const std::vector<long long>* unit_off = nullptr, bool weighted = false) {
@@ -961,23 +1066,9 @@ int fetch_results(cbs_gpu_ctx* c, const Dev& hD, int n_units, bool want_splits, 
         }
         R->seg_offsets.swap(noff); R->lengths.swap(nlen); R->means.swap(nmean);
     }
-    R->splits.resize(sp.size());
-    for (size_t k = 0; k < sp.size(); ++k) {
-        cbs_gpu_split& o = R->splits[k];
-        const SplitRec& s = sp[k];
-        o.unit = s.unit; o.lo = s.lo; o.hi = s.hi; o.ostat = s.ostat; o.iseg0 = s.iseg0; o.iseg1 = s.iseg1;
-        o.ncpt = s.ncpt; o.icpt0 = s.icpt0; o.icpt1 = s.icpt1; o.perms_run = s.perms_run; o.nrej = s.nrej;
-        o.exit_code = s.exit_code; o.called = s.called; o.e_nrej0 = s.e_nrej0; o.e_nrej1 = s.e_nrej1;
-        o.e_status0 = s.e_status0; o.e_status1 = s.e_status1;
-    }
-    R->pub.n_units = n_units;
-    R->pub.n_segments = (int64_t)R->lengths.size();
-    R->pub.seg_offsets = R->seg_offsets.data();
-    R->pub.lengths = R->lengths.data();
-    R->pub.means = R->means.data();
-    R->pub.draws_consumed = R->draws.data();
-    R->pub.n_splits = (int64_t)R->splits.size();
-    R->pub.splits = R->splits.empty() ? nullptr : R->splits.data();
+    R->splits.clear();
+    for (const SplitRec& s : sp) R->splits.push_back(to_split(s));
+    publish(R, n_units);
     R->pub.rounds = hD.round;
     R->pub.perms_run = hD.stat_perms;
     R->pub.perm_elements = hD.stat_perm_elems;
@@ -1001,6 +1092,19 @@ int stage_values(cbs_gpu_ctx* c, const void* values, int dtype, int memspace, lo
         k_widen_f32<<<std::min<long long>((N + 255) / 256, c->sm_count * 16), 256, 0, st>>>(src, dst, N);
         c->launches++;
     }
+    return CBS_GPU_OK;
+}
+
+// CBS needs finite input (the reference has no defined behaviour otherwise): the N values staged in c->x
+int check_finite_device(cbs_gpu_ctx* c, long long N) {
+    cudaStream_t st = c->stream;
+    ENSURE(c, c->flag, sizeof(int));
+    CUDA_TRY(c, cudaMemsetAsync(c->flag.p, 0, sizeof(int), st));
+    if (N) { k_count_nonfinite<<<std::min<long long>((N + 255) / 256, c->sm_count * 8), 256, 0, st>>>(c->x.as<double>(), N, c->flag.as<int>()); c->launches++; }
+    int bad = 0;
+    CUDA_TRY(c, cudaMemcpyAsync(&bad, c->flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(c, cudaStreamSynchronize(st));
+    if (bad) return fail(c, CBS_GPU_ERR_NONFINITE, "non-finite values reach CBS; remove them first (DNAcopy drops missing values before segmenting)");
     return CBS_GPU_OK;
 }
 
@@ -1034,7 +1138,7 @@ int cbs_gpu_create(const int* device_ids, int ndev, cbs_gpu_ctx** out) {
     c->sm_count = prop.multiProcessorCount;
     c->smem_optin = prop.sharedMemPerBlockOptin - 1024;  // head room for the kernels' static shared memory
     // function attributes are process-wide per device: set them once to the device maximum, never per call
-    // (concurrent lanes with different needs would otherwise shrink each other's limit)
+    // (concurrent contexts with different needs would otherwise shrink each other's limit)
     const int mx = (int)c->smem_optin;
     if (!set_max_smem(k_scan_perm<false>, mx) || !set_max_smem(k_scan_perm<true>, mx) || !set_max_smem(k_scan_obs<false>, mx) ||
         !set_max_smem(k_scan_obs<true>, mx) ||
@@ -1070,8 +1174,6 @@ int cbs_gpu_create(const int* device_ids, int ndev, cbs_gpu_ctx** out) {
 
 void cbs_gpu_destroy(cbs_gpu_ctx* c) {
     if (!c) return;
-    for (auto* l : c->lanes) cbs_gpu_destroy(l);
-    c->lanes.clear();
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
     DevBuf* bufs[] = {&c->x, &c->cur, &c->gtab, &c->factab, &c->bbtab, &c->unit_off, &c->unit_ids, &c->tasks, &c->ring, &c->act0,
@@ -1131,7 +1233,7 @@ int cbs_gpu_selftest(void) {
 
 int cbs_gpu_measure_fp64(cbs_gpu_ctx* c, double* tera_inst_per_s) {
     if (!c || !tera_inst_per_s) return CBS_GPU_ERR_INVALID;
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
+    BEGIN_CALL(c);
     const int grid = c->sm_count * 8, block = 256, iters = 4096;
     ENSURE(c, c->staging, sizeof(double) * (size_t)grid * block);
     cudaStream_t st = c->stream;
@@ -1151,15 +1253,12 @@ int cbs_gpu_measure_fp64(cbs_gpu_ctx* c, double* tera_inst_per_s) {
     return CBS_GPU_OK;
 }
 
-// ---- low level: cbs::tmaxo / cbs::tmaxp on vectors as given ------------------------------------
-static int run_raw_scan(cbs_gpu_ctx* c, const double* xh, int n, int count, double tss, int al0, int ibin, int obs,
-                        std::vector<Task>& tasks_out) {
-    if (!c) return CBS_GPU_ERR_INVALID;
-    if (ibin) return fail(c, CBS_GPU_ERR_CUDA, "internal: binary data takes run_bin_scan");
-    if (n < 2 || count < 1 || !xh) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
-    if (al0 < 1 || n < 2 * al0) return fail(c, CBS_GPU_ERR_INVALID, "need n >= 2*al0, al0 >= 1");
-    if (n > CBS_GPU_MAX_UNIT) return fail(c, CBS_GPU_ERR_UNSUPPORTED, kTooLong);
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
+// ---- low level: cbs::tmaxo / cbs::tmaxp / cbs::htmaxp on vectors as given ------------------------------------
+// `count` vectors of n values laid end to end, staged without the scheduler: one raw task per vector (state `state`,
+// `use_hybrid`) with its prep entry and scan item (`obs`), the caller's hD (zeroed, with the fields only that caller sets)
+// completed and uploaded; then the tables and prefix sums of every vector (k_tables, k_prep)
+static int stage_raw_vectors(cbs_gpu_ctx* c, const double* xh, int n, int count, double tss, int al0, int state, int use_hybrid,
+                             int obs, Dev& hD) {
     cudaStream_t st = c->stream;
     const long long N = (long long)n * count;
     const int nb = block_count(n);
@@ -1182,17 +1281,15 @@ static int run_raw_scan(cbs_gpu_ctx* c, const double* xh, int n, int count, doub
     std::vector<int> prep((size_t)count), prefix((size_t)count + 1);
     std::vector<PermItem> items((size_t)count);
     memset(tasks.data(), 0, sizeof(Task) * tasks.size());
-    for (int u = 0; u <= count; ++u) off[u] = (long long)u * n;
+    for (int u = 0; u <= count; ++u) off[(size_t)u] = (long long)u * n;
     for (int u = 0; u < count; ++u) {
-        Task& t = tasks[u];
-        t.unit = u; t.lo = 0; t.hi = n; t.n = n; t.nb = nb; t.raw = 1; t.tss = tss; t.state = TS_OBS;
+        Task& t = tasks[(size_t)u];
+        t.unit = u; t.lo = 0; t.hi = n; t.n = n; t.nb = nb; t.raw = 1; t.tss = tss; t.state = state; t.use_hybrid = use_hybrid;
         t.off_sx = per * u; t.off_bs = per * u + Sched::sx_stride(n); t.off_rej = u; t.next = -1;
-        prep[u] = u; prefix[u] = u;
-        items[u].task = u; items[u].P = 1; items[u].obs = obs;
+        prep[(size_t)u] = u; prefix[(size_t)u] = u;
+        items[(size_t)u].task = u; items[(size_t)u].P = 1; items[(size_t)u].obs = obs;
     }
-    prefix[count] = count;
-    Dev hD;
-    memset(&hD, 0, sizeof(hD));
+    prefix[(size_t)count] = count;
     hD.x = c->x.as<double>(); hD.unit_off = c->unit_off.as<long long>(); hD.n_units = count;
     hD.prm.min_width = al0; hD.prm.nperm = 0; hD.prm.rng_mode = RNG_PHILOX;
     hD.cur = c->cur.as<double>(); hD.gtab = c->gtab.as<double>(); hD.factab = c->factab.as<double>(); hD.bbtab = c->bbtab.as<int>();
@@ -1200,8 +1297,6 @@ static int run_raw_scan(cbs_gpu_ctx* c, const double* xh, int n, int count, doub
     hD.arena = c->arena.as<double>(); hD.arena_cap = per * count; hD.rej = c->rej.as<int>(); hD.rej_cap = count;
     hD.n_prep = count; hD.prep_task = c->prep_task.as<int>();
     hD.n_items = count; hD.items = c->items.as<PermItem>(); hD.item_prefix = c->item_prefix.as<int>();
-    hD.obs_slices = obs_slice_cap(); hD.obs_noloc = obs == 2 ? 1 : 0;
-    hD.ctr[CTR_OBS_SLICES] = (unsigned)obs_slices(n, hD.obs_slices);
     CUDA_TRY(c, cudaMemcpyAsync(c->x.p, xh, sizeof(double) * (size_t)N, cudaMemcpyHostToDevice, st));
     CUDA_TRY(c, cudaMemcpyAsync(c->unit_off.p, off.data(), sizeof(long long) * off.size(), cudaMemcpyHostToDevice, st));
     CUDA_TRY(c, cudaMemcpyAsync(c->tasks.p, tasks.data(), sizeof(Task) * tasks.size(), cudaMemcpyHostToDevice, st));
@@ -1209,14 +1304,32 @@ static int run_raw_scan(cbs_gpu_ctx* c, const double* xh, int n, int count, doub
     CUDA_TRY(c, cudaMemcpyAsync(c->items.p, items.data(), sizeof(PermItem) * items.size(), cudaMemcpyHostToDevice, st));
     CUDA_TRY(c, cudaMemcpyAsync(c->item_prefix.p, prefix.data(), sizeof(int) * prefix.size(), cudaMemcpyHostToDevice, st));
     CUDA_TRY(c, cudaMemcpyAsync(c->dev.p, &hD, sizeof(Dev), cudaMemcpyHostToDevice, st));
-    ScanLayout lay;
-    lay.nb_max = nb + 2;
-    int occ = 1;
-    if (!lay.set_table(n, c->smem_optin) || !pick_scan_warps(c, lay, &occ, (const void*)k_scan_obs<false>)) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "vector too long for the scan kernel's shared memory");
     Dev* dD = c->dev.as<Dev>();
     k_tables<<<dim3(16, 64), 256, 0, st>>>(dD);
-    k_prep<<<std::min(count, c->sm_count * 8), 32, 0, st>>>(dD);
-    launch_scan(true, false, (int)std::min<long long>((long long)count * hD.ctr[CTR_OBS_SLICES], (long long)c->sm_count * occ), lay, st, dD);
+    k_prep<<<std::min(count, c->sm_count * 8), 32, 0, st>>>(dD);  // prefix sums of the vectors as given (CBS.cpp:396-398)
+    return CBS_GPU_OK;
+}
+
+// cbs::tmaxo (obs = 1) / cbs::tmaxp (obs = 2): the observed scan of each vector
+static int run_raw_scan(cbs_gpu_ctx* c, const double* xh, int n, int count, double tss, int al0, int obs,
+                        std::vector<Task>& tasks_out) {
+    if (!c) return CBS_GPU_ERR_INVALID;
+    if (n < 2 || count < 1 || !xh) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
+    if (al0 < 1 || n < 2 * al0) return fail(c, CBS_GPU_ERR_INVALID, "need n >= 2*al0, al0 >= 1");
+    if (n > CBS_GPU_MAX_UNIT) return fail(c, CBS_GPU_ERR_UNSUPPORTED, kTooLong);
+    BEGIN_CALL(c);
+    cudaStream_t st = c->stream;
+    ScanLayout lay;
+    lay.nb_max = block_count(n) + 2;
+    int occ = 1;
+    if (!lay.set_table(n, c->smem_optin) || !pick_scan_warps(c, lay, &occ, (const void*)k_scan_obs<false>)) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "vector too long for the scan kernel's shared memory");
+    Dev hD;
+    memset(&hD, 0, sizeof(hD));
+    hD.obs_slices = obs_slice_cap(); hD.obs_noloc = obs == 2 ? 1 : 0;
+    hD.ctr[CTR_OBS_SLICES] = (unsigned)obs_slices(n, hD.obs_slices);
+    const int rc = stage_raw_vectors(c, xh, n, count, tss, al0, TS_OBS, 0, obs, hD);
+    if (rc) return rc;
+    launch_scan(true, false, (int)std::min<long long>((long long)count * hD.ctr[CTR_OBS_SLICES], (long long)c->sm_count * occ), lay, st, c->dev.as<Dev>());
     CUDA_TRY(c, cudaGetLastError());
     tasks_out.resize((size_t)count);
     CUDA_TRY(c, cudaMemcpyAsync(tasks_out.data(), c->tasks.p, sizeof(Task) * tasks_out.size(), cudaMemcpyDeviceToHost, st));
@@ -1231,7 +1344,7 @@ static int run_bin_scan(cbs_gpu_ctx* c, const double* xh, int n, int count, doub
     if (n < 2 || count < 1 || !xh) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
     if (al0 < 1 || n < 2 * al0) return fail(c, CBS_GPU_ERR_INVALID, "need n >= 2*al0, al0 >= 1");
     if (n > CBS_GPU_MAX_UNIT) return fail(c, CBS_GPU_ERR_UNSUPPORTED, kTooLong);
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
+    BEGIN_CALL(c);
     cudaStream_t st = c->stream;
     const long long N = (long long)n * count, per = bin_scratch_doubles(n);
     ENSURE(c, c->x, sizeof(double) * (size_t)(N + 1));
@@ -1262,7 +1375,7 @@ int cbs_gpu_tmaxo(cbs_gpu_ctx* c, const double* x, int32_t n, double tss, int32_
         return CBS_GPU_OK;
     }
     std::vector<Task> t;
-    const int rc = run_raw_scan(c, x, n, 1, tss, al0, ibin, 1, t);
+    const int rc = run_raw_scan(c, x, n, 1, tss, al0, 1, t);
     if (rc) return rc;
     if (statistic) *statistic = t[0].ostat;
     if (start) *start = t[0].tmaxi - 1;  // CBS.cpp:380
@@ -1280,36 +1393,35 @@ int cbs_gpu_tmaxp(cbs_gpu_ctx* c, const double* px, int32_t n, int32_t count, do
         return CBS_GPU_OK;
     }
     std::vector<Task> t;
-    const int rc = run_raw_scan(c, px, n, count, tss, al0, ibin, 2, t);
+    const int rc = run_raw_scan(c, px, n, count, tss, al0, 2, t);
     if (rc) return rc;
     for (int k = 0; k < count; ++k) statistics[k] = t[k].ostat;
     return CBS_GPU_OK;
 }
 
-static int segment_batch_impl(cbs_gpu_ctx* c, const void* values, int dtype, int memspace, const int64_t* unit_offsets,
-                              const uint64_t* unit_ids, int32_t n_units, const cbs_gpu_params* params, cbs_gpu_result** out) {
+// One batch on this context: cbs_gpu_segment_batch (one sub-batch of it) and, with `weighted`, cbs_gpu_segment_weighted_batch
+// (cbs::segment_weighted, CBS.cpp:1026-1099, for every unit; weights float64, laid out like the values)
+static int segment_batch_impl(cbs_gpu_ctx* c, const void* values, const double* weights, bool weighted, int dtype, int memspace,
+                              const int64_t* unit_offsets, const uint64_t* unit_ids, int32_t n_units, const cbs_gpu_params* params,
+                              cbs_gpu_result** out) {
     if (!c) return CBS_GPU_ERR_INVALID;
     if (!out) return fail(c, CBS_GPU_ERR_INVALID, "out is NULL");
     *out = nullptr;
     const auto wall0 = std::chrono::steady_clock::now();
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
+    BEGIN_CALL(c);
     int rc = validate_params(c, params);
     if (rc) return rc;
     if (n_units < 0 || !unit_offsets) return fail(c, CBS_GPU_ERR_INVALID, "bad unit table");
     if (dtype != CBS_GPU_F32 && dtype != CBS_GPU_F64) return fail(c, CBS_GPU_ERR_INVALID, "bad dtype");
-    std::vector<long long> off((size_t)n_units + 1);
-    for (int u = 0; u <= n_units; ++u) {
-        off[u] = unit_offsets[u];
-        if (u && off[u] < off[u - 1]) return fail(c, CBS_GPU_ERR_INVALID, "unit_offsets must be non-decreasing");
-    }
-    if (off[0] != 0) return fail(c, CBS_GPU_ERR_INVALID, "unit_offsets[0] must be 0");
+    rc = check_unit_offsets(c, unit_offsets, n_units);
+    if (rc) return rc;
+    const std::vector<long long> off(unit_offsets, unit_offsets + n_units + 1);
     const long long N = off[n_units];
-    if (N > 0 && !values) return fail(c, CBS_GPU_ERR_INVALID, "values is NULL");
-    for (int k = 0; k < K_COUNT; ++k) c->kms[k] = 0.0;
-    c->launches = 0;
+    if (N > 0 && (!values || (weighted && !weights)))
+        return fail(c, CBS_GPU_ERR_INVALID, weighted ? "values / weights is NULL" : "values is NULL");
     cudaStream_t st = c->stream;
     ENSURE(c, c->x, sizeof(double) * (size_t)(N + 1));
-    ENSURE(c, c->flag, sizeof(int));
+    if (weighted) ENSURE(c, c->wts, sizeof(double) * (size_t)(N + 1));
     CUDA_TRY(c, cudaEventRecord(c->e0, st));
     double* xdst = c->x.as<double>();
     if (params->do_smooth) {
@@ -1319,6 +1431,10 @@ static int segment_batch_impl(cbs_gpu_ctx* c, const void* values, int dtype, int
     }
     rc = stage_values(c, values, dtype, memspace, N, xdst);
     if (rc) return rc;
+    if (weighted && N) {
+        const cudaMemcpyKind kind = memspace == CBS_GPU_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
+        CUDA_TRY(c, cudaMemcpyAsync(c->wts.p, weights, sizeof(double) * (size_t)N, kind, st));
+    }
     CUDA_TRY(c, cudaEventRecord(c->e1, st));
     if (params->do_smooth) {
         ENSURE(c, c->goff, sizeof(long long) * (size_t)(n_units + 1));
@@ -1328,20 +1444,15 @@ static int segment_batch_impl(cbs_gpu_ctx* c, const void* values, int dtype, int
         if (rc) return rc;
     }
     CUDA_TRY(c, cudaEventRecord(c->e2, st));
-    // CBS needs finite input (the reference has no defined behaviour otherwise)
-    CUDA_TRY(c, cudaMemsetAsync(c->flag.p, 0, sizeof(int), st));
-    if (N) { k_count_nonfinite<<<std::min<long long>((N + 255) / 256, c->sm_count * 8), 256, 0, st>>>(c->x.as<double>(), N, c->flag.as<int>()); c->launches++; }
-    int bad = 0;
-    CUDA_TRY(c, cudaMemcpyAsync(&bad, c->flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(c, cudaStreamSynchronize(st));
-    if (bad) return fail(c, CBS_GPU_ERR_NONFINITE, "non-finite values reach CBS; remove them first (DNAcopy drops missing values before segmenting)");
+    rc = check_finite_device(c, N);
+    if (rc) return rc;
     Dev hD;
-    rc = run_cbs(c, off, unit_ids, n_units, params, nullptr, false, hD);
+    rc = run_cbs(c, off, unit_ids, n_units, params, nullptr, weighted, hD);
     if (rc) return rc;
     CUDA_TRY(c, cudaEventRecord(c->e3, st));
     ResultOwner* R = new ResultOwner();
     memset(&R->pub, 0, sizeof(R->pub));
-    rc = fetch_results(c, hD, n_units, params->record_splits != 0, R, params, &off);
+    rc = fetch_results(c, hD, n_units, params->record_splits != 0, R, params, &off, weighted);
     if (rc) { delete R; return rc; }
     CUDA_TRY(c, cudaEventRecord(c->e4, st));
     CUDA_TRY(c, cudaEventSynchronize(c->e4));
@@ -1364,115 +1475,46 @@ int cbs_gpu_segment_batch(cbs_gpu_ctx* c, const void* values, int dtype, int mem
     if (!c) return CBS_GPU_ERR_INVALID;
     if (!out) return fail(c, CBS_GPU_ERR_INVALID, "out is NULL");
     *out = nullptr;
-    int want_lanes = (int)env_ll("CBS_GPU_LANES", 1);  // opt-in: measured no gain on B200 (persistent grids fill the SMs)
-    const bool serial_stream = params && params->rng_mode == CBS_GPU_RNG_MT19937_64 && params->chain;
-    bool splittable = !c->is_lane && params && unit_offsets && n_units >= 2 && !serial_stream && (dtype == CBS_GPU_F32 || dtype == CBS_GPU_F64);
-    if (splittable) {  // (malformed unit tables go to segment_batch_impl as they are: it reports them)
-        if (unit_offsets[0] != 0) splittable = false;
-        for (int u = 0; splittable && u < n_units; ++u) if (unit_offsets[u + 1] < unit_offsets[u]) splittable = false;
-    }
     // Large cohorts are segmented in consecutive sub-batches of about CBS_GPU_CHUNK_MARKERS markers (default 96 M, some 50
     // SNP6 samples) so that a call of any size runs in bounded device memory (~100 B per marker of per-call buffers besides
     // the arenas).  Units are independent (Philox keys and chain == 0 streams do not depend on the neighbours), and the cost
     // per sample does not depend on the batch size beyond a few samples per call (125 samples: 6.77 s in one batch, 6.81 s in
-    // five), so the split costs nothing.
+    // five), so the split costs nothing.  (Malformed unit tables go to segment_batch_impl as they are: it reports them.)
+    const bool serial_stream = params && params->rng_mode == CBS_GPU_RNG_MT19937_64 && params->chain;
+    const bool splittable = params && unit_offsets && n_units >= 2 && !serial_stream && (dtype == CBS_GPU_F32 || dtype == CBS_GPU_F64) &&
+                            check_unit_offsets(nullptr, unit_offsets, n_units) == CBS_GPU_OK;
     const long long chunk_max = std::max<long long>(1024, env_ll("CBS_GPU_CHUNK_MARKERS", 96LL << 20));
-    const long long N_all = splittable ? (long long)unit_offsets[n_units] : 0;
-    const bool parallel = splittable && want_lanes >= 2 && n_units >= 2 * want_lanes;
-    if (!parallel && (!splittable || N_all <= chunk_max))
-        return segment_batch_impl(c, values, dtype, memspace, unit_offsets, unit_ids, n_units, params, out);
-    if (want_lanes > 4) want_lanes = 4;
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
-    int L = want_lanes;
-    std::vector<int> cut;
-    if (parallel) {
-        while ((int)c->lanes.size() < L) {
-            cbs_gpu_ctx* child = nullptr;
-            const int ids[1] = {c->device};
-            if (cbs_gpu_create(ids, 1, &child) != CBS_GPU_OK) return fail(c, CBS_GPU_ERR_CUDA, "cannot create lane context");
-            child->is_lane = true;
-            c->lanes.push_back(child);
-        }
-        // contiguous ranges balanced by sum n^1.5 (the cost of the permutation scans)
-        std::vector<double> cost((size_t)n_units + 1, 0.0);
-        for (int u = 0; u < n_units; ++u) {
-            const double n = (double)(unit_offsets[u + 1] - unit_offsets[u]);
-            cost[u + 1] = cost[u] + (n > 0 ? n * std::sqrt(n) : 0.0);
-        }
-        cut.assign((size_t)L + 1, 0);
-        cut[L] = n_units;
-        for (int l = 1; l < L; ++l) {
-            const double target = cost[n_units] * l / L;
-            int u = cut[l - 1];
-            while (u < n_units && cost[u + 1] <= target) ++u;
-            cut[l] = std::max(u, cut[l - 1]);
-        }
-    } else {
-        // sub-batches of equal marker counts, cut at unit boundaries
-        const int want = (int)std::min<long long>((N_all + chunk_max - 1) / chunk_max, n_units);
-        cut.push_back(0);
-        for (int k = 1; k < want; ++k) {
-            const long long target = N_all * k / want;
-            int u = cut.back();
-            while (u < n_units && (long long)unit_offsets[u + 1] <= target) ++u;
-            if (u > cut.back() && u < n_units) cut.push_back(u);
-        }
-        cut.push_back(n_units);
-        L = (int)cut.size() - 1;
+    if (!splittable || (long long)unit_offsets[n_units] <= chunk_max)
+        return segment_batch_impl(c, values, nullptr, false, dtype, memspace, unit_offsets, unit_ids, n_units, params, out);
+    BEGIN_CALL(c);
+    // sub-batches of equal marker counts, cut at unit boundaries
+    const long long N_all = unit_offsets[n_units];
+    const int want = (int)std::min<long long>((N_all + chunk_max - 1) / chunk_max, n_units);
+    std::vector<int> cut = {0};
+    for (int k = 1; k < want; ++k) {
+        const long long target = N_all * k / want;
+        int u = cut.back();
+        while (u < n_units && (long long)unit_offsets[u + 1] <= target) ++u;
+        if (u > cut.back() && u < n_units) cut.push_back(u);
     }
-    // the input must be complete before other streams read it
-    if (memspace == CBS_GPU_DEVICE) cudaStreamSynchronize(c->stream);
+    cut.push_back(n_units);
     std::vector<uint64_t> ids_all((size_t)n_units);
     for (int u = 0; u < n_units; ++u) ids_all[u] = unit_ids ? unit_ids[u] : (uint64_t)u;  // keys must not depend on the split
-    std::vector<int> rcs((size_t)L, CBS_GPU_OK);
-    std::vector<cbs_gpu_result*> parts((size_t)L, nullptr);
-    std::vector<std::vector<int64_t>> offs((size_t)L);
-    std::vector<std::thread> th;
     const size_t esz = dtype == CBS_GPU_F32 ? 4 : 8;
-    std::vector<std::vector<double>> part_kms((size_t)L, std::vector<double>((size_t)K_COUNT, 0.0));
-    std::vector<unsigned long long> part_arcs((size_t)L, 0), part_slots((size_t)L, 0);
-    for (int l = 0; l < L; ++l) {
-        const int u0 = cut[l], u1 = cut[l + 1];
-        offs[l].resize((size_t)(u1 - u0) + 1);
-        for (int u = u0; u <= u1; ++u) offs[l][u - u0] = unit_offsets[u] - unit_offsets[u0];
-        const char* base = (const char*)values + (size_t)unit_offsets[u0] * esz;
-        if (parallel) {
-            cbs_gpu_ctx* child = c->lanes[l];
-            child->profiling = c->profiling; child->counting = c->counting; child->serial = c->serial;
-            child->mem_fraction = 0.80 / L;
-            th.emplace_back([=, &rcs, &parts, &offs, &ids_all]() {
-                rcs[l] = segment_batch_impl(child, base, dtype, memspace, offs[l].data(), ids_all.data() + u0, u1 - u0, params, &parts[l]);
-            });
-        } else {
-            rcs[l] = segment_batch_impl(c, base, dtype, memspace, offs[l].data(), ids_all.data() + u0, u1 - u0, params, &parts[l]);
-            if (rcs[l] != CBS_GPU_OK) {
-                for (auto* p : parts) if (p) cbs_gpu_result_free(p);
-                return rcs[l];  // the message is already in c
-            }
-            for (int k = 0; k < K_COUNT; ++k) part_kms[l][k] = c->kms[k];
-            part_arcs[l] = c->last_arcs; part_slots[l] = c->last_slots;
-        }
-    }
-    for (auto& t : th) t.join();
-    if (parallel)
-        for (int l = 0; l < L; ++l) {
-            if (rcs[l] != CBS_GPU_OK) {
-                const std::string msg = cbs_gpu_last_error(c->lanes[l]);
-                for (auto* p : parts) if (p) cbs_gpu_result_free(p);
-                return fail(c, rcs[l], msg);
-            }
-            for (int k = 0; k < K_COUNT; ++k) part_kms[l][k] = c->lanes[l]->kms[k];
-            part_arcs[l] = c->lanes[l]->last_arcs; part_slots[l] = c->lanes[l]->last_slots;
-        }
     ResultOwner* R = new ResultOwner();
     memset(&R->pub, 0, sizeof(R->pub));
     R->seg_offsets.assign((size_t)n_units + 1, 0);
     R->draws.assign((size_t)n_units, 0);
-    for (int k = 0; k < K_COUNT; ++k) c->kms[k] = 0.0;
-    c->last_arcs = 0; c->last_slots = 0;
-    for (int l = 0; l < L; ++l) {
-        const cbs_gpu_result* p = parts[l];
-        const int u0 = cut[l];
+    double kms[K_COUNT] = {0};
+    uint64_t arcs = 0, slots = 0;
+    for (size_t l = 0; l + 1 < cut.size(); ++l) {  // one after the other: times and rounds add up
+        const int u0 = cut[l], u1 = cut[l + 1];
+        std::vector<int64_t> offs((size_t)(u1 - u0) + 1);
+        for (int u = u0; u <= u1; ++u) offs[u - u0] = unit_offsets[u] - unit_offsets[u0];
+        const char* base = (const char*)values + (size_t)unit_offsets[u0] * esz;
+        cbs_gpu_result* p = nullptr;
+        const int rc = segment_batch_impl(c, base, nullptr, false, dtype, memspace, offs.data(), ids_all.data() + u0, u1 - u0, params, &p);
+        if (rc != CBS_GPU_OK) { delete R; return rc; }  // the message is already in c
         const int64_t shift = (int64_t)R->lengths.size();
         for (int u = 0; u < p->n_units; ++u) {
             R->seg_offsets[(size_t)u0 + u + 1] = shift + p->seg_offsets[u + 1];
@@ -1482,30 +1524,18 @@ int cbs_gpu_segment_batch(cbs_gpu_ctx* c, const void* values, int dtype, int mem
         R->means.insert(R->means.end(), p->means, p->means + p->n_segments);
         for (int64_t k = 0; k < p->n_splits; ++k) { cbs_gpu_split sp = p->splits[k]; sp.unit += u0; R->splits.push_back(sp); }
         R->pub.perms_run += p->perms_run; R->pub.perm_elements += p->perm_elements; R->pub.kernel_launches += p->kernel_launches;
-        if (parallel) {  // lanes run side by side, sub-batches one after the other
-            R->pub.rounds = std::max(R->pub.rounds, p->rounds);
-            R->pub.ms_h2d = std::max(R->pub.ms_h2d, p->ms_h2d); R->pub.ms_smooth = std::max(R->pub.ms_smooth, p->ms_smooth);
-            R->pub.ms_segment = std::max(R->pub.ms_segment, p->ms_segment); R->pub.ms_d2h = std::max(R->pub.ms_d2h, p->ms_d2h);
-            R->pub.ms_call = std::max(R->pub.ms_call, p->ms_call);
-        } else {
-            R->pub.rounds += p->rounds;
-            R->pub.ms_h2d += p->ms_h2d; R->pub.ms_smooth += p->ms_smooth; R->pub.ms_segment += p->ms_segment; R->pub.ms_d2h += p->ms_d2h;
-            R->pub.ms_call += p->ms_call;
-        }
-        for (int k = 0; k < K_COUNT; ++k) c->kms[k] += part_kms[l][k];
-        c->last_arcs += part_arcs[l]; c->last_slots += part_slots[l];
+        R->pub.rounds += p->rounds;
+        R->pub.ms_h2d += p->ms_h2d; R->pub.ms_smooth += p->ms_smooth; R->pub.ms_segment += p->ms_segment; R->pub.ms_d2h += p->ms_d2h;
+        R->pub.ms_call += p->ms_call;
+        for (int k = 0; k < K_COUNT; ++k) kms[k] += c->kms[k];
+        arcs += c->last_arcs; slots += c->last_slots;
+        cbs_gpu_result_free(p);
     }
+    for (int k = 0; k < K_COUNT; ++k) c->kms[k] = kms[k];
+    c->last_arcs = arcs; c->last_slots = slots;
     // empty leading/trailing units keep monotone offsets
     for (int u = 0; u < n_units; ++u) if (R->seg_offsets[u + 1] < R->seg_offsets[u]) R->seg_offsets[u + 1] = R->seg_offsets[u];
-    for (auto* p : parts) cbs_gpu_result_free(p);
-    R->pub.n_units = n_units;
-    R->pub.n_segments = (int64_t)R->lengths.size();
-    R->pub.seg_offsets = R->seg_offsets.data();
-    R->pub.lengths = R->lengths.data();
-    R->pub.means = R->means.data();
-    R->pub.draws_consumed = R->draws.data();
-    R->pub.n_splits = (int64_t)R->splits.size();
-    R->pub.splits = R->splits.empty() ? nullptr : R->splits.data();
+    publish(R, n_units);
     *out = &R->pub;
     return CBS_GPU_OK;
 }
@@ -1518,85 +1548,41 @@ int cbs_gpu_segment_weighted_batch(cbs_gpu_ctx* c, const double* values, const d
     if (!out) return fail(c, CBS_GPU_ERR_INVALID, "out is NULL");
     *out = nullptr;
     if (!params || !unit_offsets || n_units < 0) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
     cbs_gpu_params p = *params;
     p.do_smooth = 0;  // cbs::segment_weighted does not smooth
-    int rc = validate_params(c, &p);
-    if (rc) return rc;
-    std::vector<long long> off((size_t)n_units + 1);
-    for (int u = 0; u <= n_units; ++u) off[u] = unit_offsets[u];
-    if (off[0] != 0) return fail(c, CBS_GPU_ERR_INVALID, "unit_offsets[0] must be 0");
-    for (int u = 0; u < n_units; ++u) if (off[u + 1] < off[u]) return fail(c, CBS_GPU_ERR_INVALID, "unit_offsets must be non-decreasing");
-    const long long N = off[n_units];
-    if (N > 0 && (!values || !weights)) return fail(c, CBS_GPU_ERR_INVALID, "values / weights is NULL");
-    for (int k = 0; k < K_COUNT; ++k) c->kms[k] = 0.0;
-    c->launches = 0;
-    cudaStream_t st = c->stream;
-    ENSURE(c, c->x, sizeof(double) * (size_t)(N + 1));
-    ENSURE(c, c->wts, sizeof(double) * (size_t)(N + 1));
-    ENSURE(c, c->flag, sizeof(int));
-    CUDA_TRY(c, cudaEventRecord(c->e0, st));
-    const cudaMemcpyKind kind = memspace == CBS_GPU_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice;
-    if (N) {
-        CUDA_TRY(c, cudaMemcpyAsync(c->x.p, values, sizeof(double) * (size_t)N, kind, st));
-        CUDA_TRY(c, cudaMemcpyAsync(c->wts.p, weights, sizeof(double) * (size_t)N, kind, st));
-    }
-    CUDA_TRY(c, cudaEventRecord(c->e1, st));
-    CUDA_TRY(c, cudaMemsetAsync(c->flag.p, 0, sizeof(int), st));
-    if (N) { k_count_nonfinite<<<std::min<long long>((N + 255) / 256, c->sm_count * 8), 256, 0, st>>>(c->x.as<double>(), N, c->flag.as<int>()); c->launches++; }
-    int bad = 0;
-    CUDA_TRY(c, cudaMemcpyAsync(&bad, c->flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(c, cudaStreamSynchronize(st));
-    if (bad) return fail(c, CBS_GPU_ERR_NONFINITE, "non-finite values reach CBS");
-    CUDA_TRY(c, cudaEventRecord(c->e2, st));
-    Dev hD;
-    rc = run_cbs(c, off, unit_ids, n_units, &p, nullptr, true, hD);
-    if (rc) return rc;
-    CUDA_TRY(c, cudaEventRecord(c->e3, st));
-    ResultOwner* R = new ResultOwner();
-    memset(&R->pub, 0, sizeof(R->pub));
-    rc = fetch_results(c, hD, n_units, p.record_splits != 0, R, &p, &off, true);
-    if (rc) { delete R; return rc; }
-    CUDA_TRY(c, cudaEventRecord(c->e4, st));
-    CUDA_TRY(c, cudaEventSynchronize(c->e4));
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, c->e0, c->e1); R->pub.ms_h2d = ms;
-    cudaEventElapsedTime(&ms, c->e2, c->e3); R->pub.ms_segment = ms;
-    cudaEventElapsedTime(&ms, c->e3, c->e4); R->pub.ms_d2h = ms;
-    if (c->profiling) collect_timers(c);
-    R->pub.kernel_launches = c->launches;
-    *out = &R->pub;
-    return CBS_GPU_OK;
+    return segment_batch_impl(c, values, weights, true, CBS_GPU_F64, memspace, unit_offsets, unit_ids, n_units, &p, out);
 }
 
-// cbs::segment_weighted on one vector (CBS.hpp:115-128)
-int cbs_gpu_segment_weighted(cbs_gpu_ctx* c, const double* x, const double* weights, int32_t n, const cbs_gpu_params* params,
-                             const uint64_t* mt_next312, int32_t cap, int32_t* lengths, double* means, int32_t* n_segments,
-                             uint64_t* draws_consumed) {
+// cbs::segment (CBS.cpp:959-1024) and, with `weighted`, cbs::segment_weighted (CBS.hpp:115-128) on one vector
+static int segment_one(cbs_gpu_ctx* c, const double* x, const double* weights, bool weighted, int32_t n, const cbs_gpu_params* params,
+                       const uint64_t* mt_next312, int32_t cap, int32_t* lengths, double* means, int32_t* n_segments,
+                       uint64_t* draws_consumed) {
     if (!c) return CBS_GPU_ERR_INVALID;
-    if (n < 0 || (n > 0 && (!x || !weights)) || !n_segments || !params) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
+    if (n < 0 || (n > 0 && (!x || (weighted && !weights))) || !n_segments || !params) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
+    BEGIN_CALL(c);
     cbs_gpu_params p = *params;
-    p.do_smooth = 0;
+    p.do_smooth = 0;  // cbs::segment does not smooth
     int rc = validate_params(c, &p);
     if (rc) return rc;
     *n_segments = 0;
     if (draws_consumed) *draws_consumed = 0;
-    if (n == 0) return CBS_GPU_OK;
-    for (int i = 0; i < n; ++i) if (!std::isfinite(x[i])) return fail(c, CBS_GPU_ERR_NONFINITE, "non-finite values reach CBS");
+    if (n == 0) return CBS_GPU_OK;  // cbs::segment on an empty vector returns no segments
+    rc = check_finite_host(c, x, n);
+    if (rc) return rc;
     cudaStream_t st = c->stream;
     ENSURE(c, c->x, sizeof(double) * (size_t)(n + 1));
-    ENSURE(c, c->wts, sizeof(double) * (size_t)(n + 1));
     CUDA_TRY(c, cudaMemcpyAsync(c->x.p, x, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(c, cudaMemcpyAsync(c->wts.p, weights, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, st));
+    if (weighted) {
+        ENSURE(c, c->wts, sizeof(double) * (size_t)(n + 1));
+        CUDA_TRY(c, cudaMemcpyAsync(c->wts.p, weights, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, st));
+    }
     std::vector<long long> off = {0, (long long)n};
     Dev hD;
-    for (int k = 0; k < K_COUNT; ++k) c->kms[k] = 0.0;
-    rc = run_cbs(c, off, nullptr, 1, &p, mt_next312, true, hD);
+    rc = run_cbs(c, off, nullptr, 1, &p, mt_next312, weighted, hD);
     if (rc) return rc;
     ResultOwner R;
     memset(&R.pub, 0, sizeof(R.pub));
-    rc = fetch_results(c, hD, 1, false, &R, &p, &off, true);
+    rc = fetch_results(c, hD, 1, false, &R, &p, &off, weighted);
     if (rc) return rc;
     if (c->profiling) collect_timers(c);
     *n_segments = (int32_t)R.pub.n_segments;
@@ -1606,12 +1592,23 @@ int cbs_gpu_segment_weighted(cbs_gpu_ctx* c, const double* x, const double* weig
     return CBS_GPU_OK;
 }
 
+int cbs_gpu_segment(cbs_gpu_ctx* c, const double* x, int32_t n, const cbs_gpu_params* params, const uint64_t* mt_next312,
+                    int32_t cap, int32_t* lengths, double* means, int32_t* n_segments, uint64_t* draws_consumed) {
+    return segment_one(c, x, nullptr, false, n, params, mt_next312, cap, lengths, means, n_segments, draws_consumed);
+}
+
+int cbs_gpu_segment_weighted(cbs_gpu_ctx* c, const double* x, const double* weights, int32_t n, const cbs_gpu_params* params,
+                             const uint64_t* mt_next312, int32_t cap, int32_t* lengths, double* means, int32_t* n_segments,
+                             uint64_t* draws_consumed) {
+    return segment_one(c, x, weights, true, n, params, mt_next312, cap, lengths, means, n_segments, draws_consumed);
+}
+
 // ---- low level: one decision on a vector as given -------------------------------------------------------------
 static int decision_impl(cbs_gpu_ctx* c, const double* x, const double* weights, int32_t n, const cbs_gpu_params* params,
                          const ApiMode& api, const uint64_t* mt_next312, cbs_gpu_split* out, uint64_t* draws_consumed) {
     if (!c) return CBS_GPU_ERR_INVALID;
     if (n < 2 || !x || !params || !out) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
+    BEGIN_CALL(c);
     cbs_gpu_params p = *params;
     p.do_smooth = 0; p.undo_prune = 0; p.chain = 0; p.record_splits = 1;
     int rc = validate_params(c, &p);
@@ -1621,7 +1618,8 @@ static int decision_impl(cbs_gpu_ctx* c, const double* x, const double* weights,
         if (n < p.kmax || !(delta < 1.0))
             return fail(c, CBS_GPU_ERR_UNSUPPORTED, "hybrid fndcpt needs n >= hk and delta < 1 (the reference's htmaxp or tailp is undefined otherwise)");
     }
-    for (int i = 0; i < n; ++i) if (!std::isfinite(x[i])) return fail(c, CBS_GPU_ERR_NONFINITE, "non-finite values reach CBS");
+    rc = check_finite_host(c, x, n);
+    if (rc) return rc;
     cudaStream_t st = c->stream;
     ENSURE(c, c->x, sizeof(double) * (size_t)(n + 1));
     CUDA_TRY(c, cudaMemcpyAsync(c->x.p, x, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, st));
@@ -1631,7 +1629,6 @@ static int decision_impl(cbs_gpu_ctx* c, const double* x, const double* weights,
     }
     std::vector<long long> off = {0, (long long)n};
     Dev hD;
-    for (int k = 0; k < K_COUNT; ++k) c->kms[k] = 0.0;
     rc = run_cbs(c, off, nullptr, 1, &p, mt_next312, weights != nullptr, hD, api);
     if (rc) return rc;
     if (hD.n_splits < 1) return fail(c, CBS_GPU_ERR_CUDA, "internal: the decision was not recorded");
@@ -1641,11 +1638,8 @@ static int decision_impl(cbs_gpu_ctx* c, const double* x, const double* weights,
     CUDA_TRY(c, cudaMemcpyAsync(&draws, c->udraws.p, sizeof(uint64_t), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(c, cudaStreamSynchronize(st));
     if (c->profiling) collect_timers(c);
-    memset(out, 0, sizeof(*out));
-    out->unit = 0; out->lo = s.lo; out->hi = s.hi; out->ostat = s.ostat; out->iseg0 = s.iseg0; out->iseg1 = s.iseg1;
-    out->ncpt = s.ncpt; out->icpt0 = s.icpt0; out->icpt1 = s.icpt1; out->perms_run = s.perms_run; out->nrej = s.nrej;
-    out->exit_code = s.exit_code; out->called = s.called; out->e_nrej0 = s.e_nrej0; out->e_nrej1 = s.e_nrej1;
-    out->e_status0 = s.e_status0; out->e_status1 = s.e_status1;
+    *out = to_split(s);
+    out->unit = 0;
     if (draws_consumed) *draws_consumed = draws;
     return CBS_GPU_OK;
 }
@@ -1714,7 +1708,7 @@ int cbs_gpu_xperm(cbs_gpu_ctx* c, const double* x, const double* rwts, int32_t n
     if (!c) return CBS_GPU_ERR_INVALID;
     if (n < 1 || !x || !px) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
     if (n > CBS_GPU_MAX_UNIT) return fail(c, CBS_GPU_ERR_UNSUPPORTED, kTooLong);
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
+    BEGIN_CALL(c);
     cudaStream_t st = c->stream;
     std::vector<uint64_t> words((size_t)n + 312);
     if (mt_next312) memcpy(words.data(), mt_next312, sizeof(uint64_t) * 312); else mt_seed_next312(seed, words.data());
@@ -1738,7 +1732,7 @@ int cbs_gpu_xperm(cbs_gpu_ctx* c, const double* x, const double* rwts, int32_t n
     int cls = shuffle_class(n, false), cl_R = 0, cl_grid = 0;
     size_t cl_smem = 0;
     if (cls == SHUF_GLOBAL)
-        for (int R : {2, 4, 8}) { cl_grid = cluster_fit(c, R, n, 12, &cl_smem); if (cl_grid) { cl_R = R; break; } }
+        for (int R : {2, 4, 8}) { cl_grid = cluster_fit(c, R, n, kClusterHbits, &cl_smem); if (cl_grid) { cl_R = R; break; } }
     Task t;
     memset(&t, 0, sizeof(t));
     t.unit = 0; t.lo = 0; t.hi = n; t.n = n; t.nb = block_count(n); t.raw = 1; t.off_sx = 0; t.off_A = stride; t.off_draw = 0;
@@ -1770,7 +1764,7 @@ int cbs_gpu_xperm(cbs_gpu_ctx* c, const double* x, const double* rwts, int32_t n
     CUDA_TRY(c, cudaMemcpyAsync(c->dev.p, &hD, sizeof(Dev), cudaMemcpyHostToDevice, st));
     Dev* dD = c->dev.as<Dev>();
     if (cls < SHUF_CL2) launch_shuffle(dD, cls, 1, st, true);
-    else if (cl_R) launch_shuffle_cluster(dD, cl_R, SHUF_GLOBAL, 12, cl_R, cl_smem, st, true);
+    else if (cl_R) launch_shuffle_cluster(dD, cl_R, SHUF_GLOBAL, kClusterHbits, cl_R, cl_smem, st, true);
     else k_perm<<<1, 128, 0, st>>>(dD);
     CUDA_TRY(c, cudaGetLastError());
     CUDA_TRY(c, cudaMemcpyAsync(px, c->arena.as<double>() + 1, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, st));
@@ -1787,59 +1781,17 @@ int cbs_gpu_htmaxp(cbs_gpu_ctx* c, const double* px, int32_t n, int32_t count, d
     // n < k leaves the reference's htmaxp without a block (nb = int(n/k) = 0): undefined there, as for the segmenter
     if (al0 < 1 || k < al0 || k > 128 || n < k) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "need al0 <= k <= 128 and n >= k");
     if (n > CBS_GPU_MAX_UNIT) return fail(c, CBS_GPU_ERR_UNSUPPORTED, kTooLong);
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
+    BEGIN_CALL(c);
     cudaStream_t st = c->stream;
-    const long long N = (long long)n * count;
-    const int nb = block_count(n);
-    const long long per = Sched::sx_stride(n) + Sched::bs_stride(nb);
-    ENSURE(c, c->x, sizeof(double) * (size_t)(N + 1));
-    ENSURE(c, c->cur, sizeof(double) * (size_t)(N + 1));
-    ENSURE(c, c->gtab, sizeof(double) * (size_t)(N + 1));
-    ENSURE(c, c->factab, sizeof(double) * (size_t)(N + 1));
-    ENSURE(c, c->bbtab, sizeof(int) * (size_t)(N + 1));
-    ENSURE(c, c->unit_off, sizeof(long long) * (size_t)(count + 1));
-    ENSURE(c, c->tasks, sizeof(Task) * (size_t)count);
-    ENSURE(c, c->arena, sizeof(double) * (size_t)(per * count));
-    ENSURE(c, c->rej, sizeof(int) * (size_t)count);
-    ENSURE(c, c->prep_task, sizeof(int) * (size_t)count);
-    ENSURE(c, c->items, sizeof(PermItem) * (size_t)count);
-    ENSURE(c, c->item_prefix, sizeof(int) * (size_t)(count + 1));
-    ENSURE(c, c->dev, sizeof(Dev));
-    std::vector<long long> off((size_t)count + 1);
-    std::vector<Task> tasks((size_t)count);
-    std::vector<int> prep((size_t)count), prefix((size_t)count + 1);
-    std::vector<PermItem> items((size_t)count);
-    memset(tasks.data(), 0, sizeof(Task) * tasks.size());
-    for (int u = 0; u <= count; ++u) off[(size_t)u] = (long long)u * n;
-    for (int u = 0; u < count; ++u) {
-        Task& t = tasks[(size_t)u];
-        t.unit = u; t.lo = 0; t.hi = n; t.n = n; t.nb = nb; t.raw = 1; t.tss = tss; t.state = TS_PERM; t.use_hybrid = 1;
-        t.off_sx = per * u; t.off_bs = per * u + Sched::sx_stride(n); t.off_rej = u; t.next = -1;
-        prep[(size_t)u] = u; prefix[(size_t)u] = u;
-        items[(size_t)u].task = u; items[(size_t)u].P = 1; items[(size_t)u].obs = 0;  // a "permutation" row: k_hscan takes it
-    }
-    prefix[(size_t)count] = count;
     Dev hD;
     memset(&hD, 0, sizeof(hD));
-    hD.x = c->x.as<double>(); hD.unit_off = c->unit_off.as<long long>(); hD.n_units = count;
-    hD.prm.min_width = al0; hD.prm.kmax = k; hD.prm.hybrid = 1; hD.prm.nperm = 0; hD.prm.rng_mode = RNG_PHILOX;
-    hD.cur = c->cur.as<double>(); hD.gtab = c->gtab.as<double>(); hD.factab = c->factab.as<double>(); hD.bbtab = c->bbtab.as<int>();
-    hD.tasks = c->tasks.as<Task>(); hD.task_cap = count;
-    hD.arena = c->arena.as<double>(); hD.arena_cap = per * count; hD.rej = c->rej.as<int>(); hD.rej_cap = count;
-    hD.n_prep = count; hD.prep_task = c->prep_task.as<int>();
-    hD.n_items = count; hD.items = c->items.as<PermItem>(); hD.item_prefix = c->item_prefix.as<int>();
-    CUDA_TRY(c, cudaMemcpyAsync(c->x.p, px, sizeof(double) * (size_t)N, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(c, cudaMemcpyAsync(c->unit_off.p, off.data(), sizeof(long long) * off.size(), cudaMemcpyHostToDevice, st));
-    CUDA_TRY(c, cudaMemcpyAsync(c->tasks.p, tasks.data(), sizeof(Task) * tasks.size(), cudaMemcpyHostToDevice, st));
-    CUDA_TRY(c, cudaMemcpyAsync(c->prep_task.p, prep.data(), sizeof(int) * prep.size(), cudaMemcpyHostToDevice, st));
-    CUDA_TRY(c, cudaMemcpyAsync(c->items.p, items.data(), sizeof(PermItem) * items.size(), cudaMemcpyHostToDevice, st));
-    CUDA_TRY(c, cudaMemcpyAsync(c->item_prefix.p, prefix.data(), sizeof(int) * prefix.size(), cudaMemcpyHostToDevice, st));
-    CUDA_TRY(c, cudaMemcpyAsync(c->dev.p, &hD, sizeof(Dev), cudaMemcpyHostToDevice, st));
+    hD.prm.kmax = k; hD.prm.hybrid = 1;
+    const int rc = stage_raw_vectors(c, px, n, count, tss, al0, TS_PERM, 1, 0 /* a "permutation" row: k_hscan takes it */, hD);
+    if (rc) return rc;
     Dev* dD = c->dev.as<Dev>();
-    k_tables<<<dim3(16, 64), 256, 0, st>>>(dD);
-    k_prep<<<std::min(count, c->sm_count * 8), 32, 0, st>>>(dD);  // prefix sums of the vectors as given (CBS.cpp:396-398)
     k_hscan<<<std::min(count, c->sm_count * 4), 256, 0, st>>>(dD);
     CUDA_TRY(c, cudaGetLastError());
+    std::vector<Task> tasks((size_t)count);
     CUDA_TRY(c, cudaMemcpyAsync(tasks.data(), c->tasks.p, sizeof(Task) * tasks.size(), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(c, cudaStreamSynchronize(st));
     for (int u = 0; u < count; ++u) statistics[u] = tasks[(size_t)u].pval1;
@@ -1851,7 +1803,7 @@ int cbs_gpu_tailp(cbs_gpu_ctx* c, double b, double delta, int32_t m, int32_t ngr
     if (!c) return CBS_GPU_ERR_INVALID;
     if (!out || m < 1) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
     if (ngrid != TAILP_NGRID) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "ngrid must be 100");
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
+    BEGIN_CALL(c);
     cudaStream_t st = c->stream;
     ENSURE(c, c->tasks, sizeof(Task));
     ENSURE(c, c->prep_task, sizeof(int));
@@ -1881,7 +1833,7 @@ int cbs_gpu_tailp(cbs_gpu_ctx* c, double b, double delta, int32_t m, int32_t ngr
 int cbs_gpu_btmax(cbs_gpu_ctx* c, const double* x, int32_t n, double* out) {
     if (!c) return CBS_GPU_ERR_INVALID;
     if (!x || !out || n < 1) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
+    BEGIN_CALL(c);
     cudaStream_t st = c->stream;
     ENSURE(c, c->x, sizeof(double) * (size_t)(n + 1));
     ENSURE(c, c->means, sizeof(double) * 2);
@@ -1896,7 +1848,7 @@ int cbs_gpu_btmax(cbs_gpu_ctx* c, const double* x, int32_t n, double* out) {
 int cbs_gpu_btailp(cbs_gpu_ctx* c, double b, int32_t m, int32_t ng, double tol, double* out) {
     if (!c) return CBS_GPU_ERR_INVALID;
     if (!out || m < 5 || ng < 1 || ng > 100000) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
+    BEGIN_CALL(c);
     cudaStream_t st = c->stream;
     ENSURE(c, c->tailp, sizeof(double) * (size_t)(ng + 2));
     ENSURE(c, c->means, sizeof(double) * 2);
@@ -1948,7 +1900,7 @@ int cbs_gpu_summarize_cn(cbs_gpu_ctx* c, const int64_t* seg_offsets, int32_t n_u
     const long long P = poff[(size_t)n_units];
     if (P == 0) return CBS_GPU_OK;
     if (!out_pos || !out_value) return fail(c, CBS_GPU_ERR_INVALID, "output arrays are NULL");
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
+    BEGIN_CALL(c);
     cudaStream_t st = c->stream;
     std::vector<long long> soff((size_t)n_units + 1);
     for (int u = 0; u <= n_units; ++u) soff[(size_t)u] = seg_offsets[u];
@@ -1982,7 +1934,7 @@ int cbs_gpu_smooth(cbs_gpu_ctx* c, const double* values, const int32_t* chrom, i
     if (!c) return CBS_GPU_ERR_INVALID;
     if (n < 0 || (n > 0 && (!values || !chrom || !out))) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
     if (smooth_region < 0) return fail(c, CBS_GPU_ERR_INVALID, "smooth_region must be non-negative");
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
+    BEGIN_CALL(c);
     if (n == 0) return CBS_GPU_OK;
     cudaStream_t st = c->stream;
     ENSURE(c, c->x, sizeof(double) * (size_t)(n + 1));
@@ -2000,40 +1952,6 @@ int cbs_gpu_smooth(cbs_gpu_ctx* c, const double* values, const int32_t* chrom, i
     CUDA_TRY(c, cudaMemcpyAsync(out, c->x.p, sizeof(double) * (size_t)n, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(c, cudaStreamSynchronize(st));
     if (c->profiling) collect_timers(c);
-    return CBS_GPU_OK;
-}
-
-int cbs_gpu_segment(cbs_gpu_ctx* c, const double* x, int32_t n, const cbs_gpu_params* params, const uint64_t* mt_next312,
-                    int32_t cap, int32_t* lengths, double* means, int32_t* n_segments, uint64_t* draws_consumed) {
-    if (!c) return CBS_GPU_ERR_INVALID;
-    if (n < 0 || (n > 0 && !x) || !n_segments) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
-    if (cudaSetDevice(c->device) != cudaSuccess) return fail(c, CBS_GPU_ERR_CUDA, "cudaSetDevice failed");
-    cbs_gpu_params p = *params;
-    p.do_smooth = 0;  // cbs::segment does not smooth
-    int rc = validate_params(c, &p);
-    if (rc) return rc;
-    *n_segments = 0;
-    if (draws_consumed) *draws_consumed = 0;
-    if (n == 0) return CBS_GPU_OK;  // cbs::segment on an empty vector returns no segments
-    cudaStream_t st = c->stream;
-    ENSURE(c, c->x, sizeof(double) * (size_t)(n + 1));
-    ENSURE(c, c->flag, sizeof(int));
-    CUDA_TRY(c, cudaMemcpyAsync(c->x.p, x, sizeof(double) * (size_t)n, cudaMemcpyHostToDevice, st));
-    for (int i = 0; i < n; ++i) if (!std::isfinite(x[i])) return fail(c, CBS_GPU_ERR_NONFINITE, "non-finite values reach CBS");
-    std::vector<long long> off = {0, (long long)n};
-    Dev hD;
-    for (int k = 0; k < K_COUNT; ++k) c->kms[k] = 0.0;
-    rc = run_cbs(c, off, nullptr, 1, &p, mt_next312, false, hD);
-    if (rc) return rc;
-    ResultOwner R;
-    memset(&R.pub, 0, sizeof(R.pub));
-    rc = fetch_results(c, hD, 1, false, &R, &p, &off);
-    if (rc) return rc;
-    if (c->profiling) collect_timers(c);
-    *n_segments = (int32_t)R.pub.n_segments;
-    if (draws_consumed) *draws_consumed = R.draws[0];
-    if (R.pub.n_segments > cap) return fail(c, CBS_GPU_ERR_CAPACITY, "output capacity too small");
-    for (int64_t k = 0; k < R.pub.n_segments; ++k) { lengths[k] = R.lengths[k]; means[k] = R.means[k]; }
     return CBS_GPU_OK;
 }
 
