@@ -44,7 +44,7 @@ enum KernelId { K_SCHED = 0, K_GEN, K_PREP, K_PERM, K_SCAN, K_EDGEPREP, K_EDGEPE
 struct RoundConfig {
     Dev* dD;
     cudaStream_t st, side[5], gen;  // as resolved after `serial`
-    int weighted, mt, shared_stream, jump, hybrid, ibin, l2_shuffle_on, counting;
+    int weighted, mt, shared_stream, jump, hybrid, hybrid_wide, ibin, l2_shuffle_on, counting;  // hybrid_wide: kmax > 128
     int n_chains;
     int shuf_on[SHUF_CL2], shuf_occ[SHUF_CL2];
     int cl_R, cl_grid, cl2_grid;
@@ -71,7 +71,7 @@ struct cbs_gpu_ctx {
     int* d_done = nullptr;  // device alias of h_done
     DevBuf x, cur, gtab, factab, bbtab, unit_off, unit_ids, tasks, ring, act0, act1, chains, segs, splits, udraws, arena,
         rej, draws0, draws1, prep_task, items, item_prefix, edgeprep_task, edges, edge_prefix, gen_chain, means, seed312,
-        dev, staging, fv, fidx, flab, lab, diffs, diffs_sorted, sm_keys, sm_gid, cn_scratch, gout, cubtmp, flag, goff, stream_buf, shuf, jump, tailp,
+        dev, staging, fv, fidx, flab, lab, diffs, diffs_sorted, sm_keys, sm_gid, sm_nmed, cn_scratch, gout, cubtmp, flag, goff, stream_buf, shuf, jump, tailp,
         wts, rw, cw, ycur;  // weighted CBS
     bool jump_ready = false;
     bool profiling = false;   // per-launch CUDA events
@@ -177,16 +177,13 @@ void collect_timers(cbs_gpu_ctx* c) {
 int validate_params(cbs_gpu_ctx* c, const cbs_gpu_params* p) {
     if (!p) return fail(c, CBS_GPU_ERR_INVALID, "params is NULL");
     if (p->ibin && p->hybrid) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "ibin=true with hybrid=true is not implemented: htmaxp has no binary variant");
-    if (p->hybrid && (p->kmax < 1 || p->kmax > 128)) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "hybrid: kmax must be in 1..128");
+    if (p->hybrid && p->kmax < 1) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "hybrid: kmax must be >= 1");
     if (p->min_width < 1) return fail(c, CBS_GPU_ERR_INVALID, "min_width must be >= 1");
     if (p->nperm < 0) return fail(c, CBS_GPU_ERR_INVALID, "nperm must be >= 0");
     if (!(p->alpha >= 0.0)) return fail(c, CBS_GPU_ERR_INVALID, "alpha must be >= 0");
     if (p->rng_mode != CBS_GPU_RNG_MT19937_64 && p->rng_mode != CBS_GPU_RNG_PHILOX)
         return fail(c, CBS_GPU_ERR_INVALID, "unknown rng_mode");
-    if (p->do_smooth) {
-        if (p->smooth_region < 0) return fail(c, CBS_GPU_ERR_INVALID, "smooth_region must be non-negative");
-        if (p->smooth_region > SM_MAX_REGION) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "smooth_region > 64 is not supported");
-    }
+    if (p->do_smooth && p->smooth_region < 0) return fail(c, CBS_GPU_ERR_INVALID, "smooth_region must be non-negative");
     return CBS_GPU_OK;
 }
 
@@ -227,10 +224,46 @@ long long env_ll(const char* name, long long dflt) {
     return atoll(s);
 }
 
+// windows wider than SM_MAX_REGION (smooth.cuh): run bounds when there are labels, the outlier test, then the medians of
+// the markers it lists
+int smooth_wide(cbs_gpu_ctx* c, const long long* goff, const int* flab, int n_groups, long long N, int region,
+                const SmoothGroupOut* gout, dim3 wgrid, double* out) {
+    cudaStream_t st = c->stream;
+    int* run_start = nullptr;
+    int* run_end = nullptr;
+    if (flab) {
+        run_start = (int*)c->diffs.p;  // 2 ints per marker in the (now free) input of the sorted differences
+        run_end = run_start + N;        // also the input of the scan
+        LaunchTimer t(c, K_SMOOTH);
+        k_sm_run_mark<<<wgrid, 256, 0, st>>>(flab, goff, n_groups, gout, run_end);
+        size_t tmp = 0;
+        cub::DeviceScan::InclusiveScan(nullptr, tmp, run_end, run_start, SmMaxInt(), (int)N, st);
+        ENSURE(c, c->cubtmp, tmp + 16);
+        CUDA_TRY(c, cub::DeviceScan::InclusiveScan(c->cubtmp.p, tmp, run_end, run_start, SmMaxInt(), (int)N, st));
+        k_sm_run_end<<<wgrid, 256, 0, st>>>(flab, goff, n_groups, gout, run_start, run_end);
+    }
+    ENSURE(c, c->sm_nmed, 16);
+    unsigned* n_med = c->sm_nmed.as<unsigned>();
+    unsigned long long* med = (unsigned long long*)c->diffs_sorted.p;  // 8 B per marker, free once k_sm_sd has run
+    CUDA_TRY(c, cudaMemsetAsync(n_med, 0, sizeof(unsigned), st));
+    {
+        LaunchTimer t(c, K_SMOOTH);
+        k_sm_wide<<<wgrid, 256, 0, st>>>(c->fv.as<double>(), c->fidx.as<int>(), run_start, run_end, goff, n_groups, region, gout,
+                                         out, med, n_med);
+    }
+    {
+        LaunchTimer t(c, K_SMOOTH);
+        k_sm_median<<<c->sm_count * 2, 256, sizeof(double) * SM_MED_SMEM_VALUES, st>>>(c->fv.as<double>(), c->fidx.as<int>(),
+                                                                                        run_start, run_end, goff, region, gout,
+                                                                                        med, n_med, out);
+    }
+    CUDA_TRY(c, cudaGetLastError());
+    return CBS_GPU_OK;
+}
+
 int smooth_device(cbs_gpu_ctx* c, const double* xin, const long long* goff, const int* dlab, int n_groups, long long N,
                   int region, double oscale, double sscale, double trim, double* out, const std::vector<long long>& host_off) {
     if (region < 0) return fail(c, CBS_GPU_ERR_INVALID, "smooth_region must be non-negative");
-    if (region > SM_MAX_REGION) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "smooth_region > 64 is not supported");
     cudaStream_t st = c->stream;
     CUDA_TRY(c, cudaMemcpyAsync(out, xin, sizeof(double) * (size_t)N, cudaMemcpyDeviceToDevice, st));
     if (N == 0 || n_groups == 0) return CBS_GPU_OK;
@@ -308,10 +341,13 @@ int smooth_device(cbs_gpu_ctx* c, const double* xin, const long long* goff, cons
         k_sm_sd<<<std::min(n_groups, c->sm_count * 8), 32, 0, st>>>(c->diffs_sorted.as<double>(), goff, n_groups,
                                                                               trim, infl, oscale, sscale, gout);
     }
-    {
+    const dim3 wgrid((unsigned)std::max(1, std::min((maxn + 255) / 256, 256)), (unsigned)std::min(n_groups, 65535));
+    if (region <= SM_MAX_REGION) {
         LaunchTimer t(c, K_SMOOTH);
-        dim3 grid((unsigned)std::max(1, std::min((maxn + 255) / 256, 256)), (unsigned)std::min(n_groups, 65535));
-        k_sm_window<<<grid, 256, 0, st>>>(c->fv.as<double>(), c->fidx.as<int>(), flab, goff, n_groups, region, gout, out);
+        k_sm_window<<<wgrid, 256, 0, st>>>(c->fv.as<double>(), c->fidx.as<int>(), flab, goff, n_groups, region, gout, out);
+    } else {
+        const int rc = smooth_wide(c, goff, flab, n_groups, N, region, gout, wgrid, out);
+        if (rc) return rc;
     }
     CUDA_TRY(c, cudaGetLastError());
     (void)host_off;
@@ -432,12 +468,18 @@ int size_call(cbs_gpu_ctx* c, const std::vector<long long>& off, int n_units, co
     if (N > 2000000000LL) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "more than 2e9 markers per call are not supported");
     const bool mt = p->rng_mode == CBS_GPU_RNG_MT19937_64;
     if (weighted && p->ibin) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "weighted CBS has no binary mode (cbs::segment_weighted takes no ibin)");
-    if (weighted && p->hybrid && p->nmin < p->kmax + 2)
+    // kmax may be anything up to INT_MAX: the comparisons are taken in 64 bits
+    const long long nmin = p->nmin, kmax = p->kmax;
+    if (weighted && p->hybrid && nmin < kmax + 2)
         return fail(c, CBS_GPU_ERR_UNSUPPORTED, "weighted hybrid CBS needs nmin >= kmax + 2");
+    // k_whscan is hwtmaxp's value on segments of 2*kmax markers or more; on shorter ones hwtmaxp's pruning by the mncwt
+    // bound skips arcs (one block, as for htmaxp_one_block), and there is no weighted form of htmaxp's own loops yet
+    if (weighted && !api.mode && p->hybrid && nmin < 2 * kmax - 1)
+        return fail(c, CBS_GPU_ERR_UNSUPPORTED, "weighted hybrid CBS needs nmin >= 2*kmax - 1 (segments shorter than 2*kmax markers are not implemented)");
     // A hybrid segment has n > nmin markers.  The reference is undefined below n = kmax + 2: with n < kmax htmaxp has no
     // block (nb = int(n/kmax) = 0) and reads past its block tables (CBS.cpp:387-485); with n <= kmax + 1, delta =
     // (kmax+1)/n >= 1 makes tailp NaN or -inf and nrejc = (int)((alpha - pval1) * nperm) an out-of-range conversion.
-    if (!weighted && !api.mode && p->hybrid && p->nmin < p->kmax + 1)
+    if (!weighted && !api.mode && p->hybrid && nmin < kmax + 1)
         return fail(c, CBS_GPU_ERR_UNSUPPORTED, "hybrid CBS needs nmin >= kmax + 1 (the reference's hybrid p-value is undefined on segments of kmax + 1 markers or fewer)");
     cap.N = N; cap.Nmax = Nmax; cap.mt = mt;
 
@@ -658,7 +700,7 @@ int configure_round(cbs_gpu_ctx* c, const cbs_gpu_params* p, bool weighted, cons
     r.gen = c->serial ? r.st : c->gen_stream;
     for (int k = 0; k < 5; ++k) r.side[k] = c->serial ? r.st : c->side[k];
     r.weighted = weighted; r.mt = cap.mt; r.shared_stream = cap.shared_stream; r.jump = hD.jump_polys != nullptr;
-    r.hybrid = p->hybrid != 0; r.ibin = p->ibin != 0; r.counting = c->counting;
+    r.hybrid = p->hybrid != 0; r.hybrid_wide = p->hybrid && p->kmax > 128; r.ibin = p->ibin != 0; r.counting = c->counting;
     r.n_chains = cap.n_chains;
     r.tailp = c->tailp.p;
     const long long Nmax = cap.Nmax;
@@ -796,7 +838,7 @@ void enqueue_round(cbs_gpu_ctx* c, const RoundConfig& r, cudaGraphConditionalHan
     if (scan_split) cudaStreamWaitEvent(st, c->ev_side[0], 0);  // the tail probabilities read the observed statistics
     if (r.hybrid) {
         double* tailp = (double*)r.tailp;
-        if (r.weighted) k_whscan<<<sm * 4, 256, 0, st>>>(dD); else k_hscan<<<sm * 4, 256, 0, st>>>(dD);
+        if (r.weighted) k_whscan<<<sm * 4, 256, 0, st>>>(dD); else if (r.hybrid_wide) k_hscan<true><<<sm * 4, 256, 0, st>>>(dD); else k_hscan<false><<<sm * 4, 256, 0, st>>>(dD);
         k_tailp_terms<<<sm * 8, 128, 0, st>>>(dD, tailp);
         k_tailp_sum<<<sm, 64, 0, st>>>(dD, tailp);
         c->launches += 3;
@@ -1148,7 +1190,8 @@ int cbs_gpu_create(const int* device_ids, int ndev, cbs_gpu_ctx** out) {
         !set_max_smem(k_shuffle_cluster<1024, 4, 2, true>, mx) || !set_max_smem(k_shuffle_cluster<1024, 4, 4, true>, mx) ||
         !set_max_smem(k_shuffle_cluster<1024, 4, 8, true>, mx) || !set_max_smem(k_shuffle_cluster<1024, 4, 2, false>, mx) ||
         !set_max_smem(k_shuffle_cluster<1024, 4, 4, false>, mx) || !set_max_smem(k_shuffle_cluster<1024, 4, 8, false>, mx) ||
-        !set_max_smem(k_wscan<0>, mx) || !set_max_smem(k_wscan<1>, mx) || !set_max_smem(k_scan_binary, mx)) {
+        !set_max_smem(k_wscan<0>, mx) || !set_max_smem(k_wscan<1>, mx) || !set_max_smem(k_scan_binary, mx) ||
+        !set_max_smem(k_sm_median, (int)(sizeof(double) * SM_MED_SMEM_VALUES))) {
         delete c;
         return CBS_GPU_ERR_CUDA;
     }
@@ -1614,10 +1657,12 @@ static int decision_impl(cbs_gpu_ctx* c, const double* x, const double* weights,
     int rc = validate_params(c, &p);
     if (rc) return rc;
     if (!weights && api.mode == 1 && p.hybrid) {  // cbs_gpu_fndcpt; see the nmin rule in run_cbs
-        const double delta = api.delta > 0.0 ? api.delta : (double)(p.kmax + 1) / (double)n;
+        const double delta = api.delta > 0.0 ? api.delta : ((double)p.kmax + 1.0) / (double)n;
         if (n < p.kmax || !(delta < 1.0))
             return fail(c, CBS_GPU_ERR_UNSUPPORTED, "hybrid fndcpt needs n >= hk and delta < 1 (the reference's htmaxp or tailp is undefined otherwise)");
     }
+    if (weights && api.mode == 1 && p.hybrid && (long long)n < 2LL * p.kmax)  // cbs_gpu_wfindcpt; see the nmin rules in run_cbs
+        return fail(c, CBS_GPU_ERR_UNSUPPORTED, "weighted hybrid wfindcpt needs n >= 2*hk (segments shorter than 2*hk markers are not implemented)");
     rc = check_finite_host(c, x, n);
     if (rc) return rc;
     cudaStream_t st = c->stream;
@@ -1779,7 +1824,7 @@ int cbs_gpu_htmaxp(cbs_gpu_ctx* c, const double* px, int32_t n, int32_t count, d
     if (ibin) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "htmaxp with ibin=true is not implemented");
     if (n < 2 || count < 1 || !px || !statistics) return fail(c, CBS_GPU_ERR_INVALID, "bad arguments");
     // n < k leaves the reference's htmaxp without a block (nb = int(n/k) = 0): undefined there, as for the segmenter
-    if (al0 < 1 || k < al0 || k > 128 || n < k) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "need al0 <= k <= 128 and n >= k");
+    if (al0 < 1 || k < al0 || n < k) return fail(c, CBS_GPU_ERR_UNSUPPORTED, "need 1 <= al0 <= k and n >= k");
     if (n > CBS_GPU_MAX_UNIT) return fail(c, CBS_GPU_ERR_UNSUPPORTED, kTooLong);
     BEGIN_CALL(c);
     cudaStream_t st = c->stream;
@@ -1789,7 +1834,8 @@ int cbs_gpu_htmaxp(cbs_gpu_ctx* c, const double* px, int32_t n, int32_t count, d
     const int rc = stage_raw_vectors(c, px, n, count, tss, al0, TS_PERM, 1, 0 /* a "permutation" row: k_hscan takes it */, hD);
     if (rc) return rc;
     Dev* dD = c->dev.as<Dev>();
-    k_hscan<<<std::min(count, c->sm_count * 4), 256, 0, st>>>(dD);
+    if (k > 128) k_hscan<true><<<std::min(count, c->sm_count * 4), 256, 0, st>>>(dD);
+    else k_hscan<false><<<std::min(count, c->sm_count * 4), 256, 0, st>>>(dD);
     CUDA_TRY(c, cudaGetLastError());
     std::vector<Task> tasks((size_t)count);
     CUDA_TRY(c, cudaMemcpyAsync(tasks.data(), c->tasks.p, sizeof(Task) * tasks.size(), cudaMemcpyDeviceToHost, st));

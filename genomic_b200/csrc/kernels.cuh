@@ -1971,8 +1971,9 @@ __global__ void __launch_bounds__(256, 2) k_scan_obs(Dev* D, ScanLayout lay) { s
 //             fac(j)*d*d over ALL arcs of length al0..k (inside its ~k-wide blocks, straddling
 //             adjacent blocks, and wrapping around the end), plus the per-block (argmin,argmax)
 //             candidates, which use the other rounding fac*(d*d) (:415-416).  It is evaluated
-//             here by brute force, 25 arcs per marker.  That holds for n >= 2k; a segment with
-//             k > n/2 follows htmaxp's own loops instead (htmaxp_one_block).
+//             here by brute force, k arcs per marker, for every k.  That holds for n >= 2k; a segment
+//             with k > n/2 follows htmaxp's own loops instead (htmaxp_one_block on one thread for
+//             k <= 128, htmaxp_one_block_cta on the whole CTA above).
 // ------------------------------------------------------------------------------------
 __device__ double dev_fpnorm(double x) { return 0.5 * erfc(-x / sqrt(2.0)); }
 __device__ double dev_nu(double x, double tol) {
@@ -2130,8 +2131,84 @@ __device__ double htmaxp_one_block(const double* __restrict__ sx, int n, int k, 
     return out;
 }
 
+// htmaxp_one_block by the whole CTA (k_hscan<true>, k > 128: there n < 2k makes the one-thread form O(k n) on one thread).
+// The (argmin, argmax) of the row is a CTA reduction that keeps the first index on ties, as the sequential scan does.
+// The loops over j stay sequential with their break: each warp computes the widest arc of one j (a max-reduction, exact),
+// eight consecutive j per step, and thread 0 walks them in order, applying the break where htmaxp applies it; widths
+// computed past the break are not used.  The value is valid in thread 0.
+__device__ double htmaxp_one_block_cta(const double* __restrict__ sx, int n, int k, int al0) {
+    __shared__ double s_v[2][8], s_w[8];
+    __shared__ int s_i[2][8], s_stop;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = (int)(blockDim.x >> 5);
+    const double rn = (double)n;
+    double lo = sx[1], hi = lo;
+    int ilo = 1, ihi = 1;
+    for (int i = 1 + tid; i <= n; i += blockDim.x) {  // ascending per thread: strict comparisons keep the first index
+        const double v = sx[i];
+        if (v < lo || (v == lo && i < ilo)) { lo = v; ilo = i; }
+        if (v > hi || (v == hi && i < ihi)) { hi = v; ihi = i; }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        const double ol = shfl_d(lo, lane ^ o), oh = shfl_d(hi, lane ^ o);
+        const int oil = __shfl_sync(FULL, ilo, lane ^ o), oih = __shfl_sync(FULL, ihi, lane ^ o);
+        if (ol < lo || (ol == lo && oil < ilo)) { lo = ol; ilo = oil; }
+        if (oh > hi || (oh == hi && oih < ihi)) { hi = oh; ihi = oih; }
+    }
+    if (lane == 0) { s_v[0][warp] = lo; s_i[0][warp] = ilo; s_v[1][warp] = hi; s_i[1][warp] = ihi; }
+    __syncthreads();
+    double out = 0.0, spread_sq = 0.0;
+    if (tid == 0) {
+        for (int w = 1; w < nw; ++w) {
+            if (s_v[0][w] < lo || (s_v[0][w] == lo && s_i[0][w] < ilo)) { lo = s_v[0][w]; ilo = s_i[0][w]; }
+            if (s_v[1][w] > hi || (s_v[1][w] == hi && s_i[1][w] < ihi)) { hi = s_v[1][w]; ihi = s_i[1][w]; }
+        }
+        const int d = abs(ilo - ihi);
+        if (d <= k && d >= al0) {
+            const double rj = (double)d;
+            const double fac = rn / (rj * (rn - rj));
+            const double v = fac * ((hi - lo) * (hi - lo));
+            if (out < v) out = v;
+        }
+        spread_sq = (hi - lo) * (hi - lo);  // also the wrap-around spread when nb = 1 (:441-443)
+    }
+    for (int wrap = 0; wrap < 2; ++wrap) {
+        for (int jb = al0; jb <= k; jb += nw) {
+            const int j = jb + warp;
+            double widest = 0.0;
+            if (j <= k) {
+                if (!wrap) { for (int i = 1 + lane; i <= n - j; i += 32) { const double w = fabs(sx[i + j] - sx[i]); if (widest < w) widest = w; } }
+                else       { for (int i = 1 + lane; i <= j; i += 32) { const double w = fabs(sx[i + n - j] - sx[i]); if (widest < w) widest = w; } }
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) { const double w = shfl_d(widest, lane ^ o); if (widest < w) widest = w; }
+            }
+            if (lane == 0) s_w[warp] = widest;
+            __syncthreads();
+            if (tid == 0) {
+                int stop = 0;
+                for (int q = 0; q < nw && jb + q <= k; ++q) {  // htmaxp's loop over j, in order
+                    const double rj = (double)(jb + q);
+                    const double fac = rn / (rj * (rn - rj));
+                    if (fac * spread_sq < out) { stop = 1; break; }
+                    const double v = fac * s_w[q] * s_w[q];
+                    if (out < v) out = v;
+                }
+                s_stop = stop;
+            }
+            __syncthreads();
+            if (s_stop) break;
+        }
+    }
+    return out;
+}
+
+// k_hscan<false> serves kmax <= 128 with the whole fac(j) table in shared memory.  k_hscan<true> serves larger kmax: the
+// lengths are taken in tiles of HS_TILE, each tile's fac(j) computed into shared memory with the same expression, and a
+// segment with n < 2k takes htmaxp_one_block_cta.
+#define HS_TILE 1024
+template <bool WIDE>
 __global__ void __launch_bounds__(256) k_hscan(Dev* D) {
-    __shared__ double s_fac[132];
+    __shared__ double s_fac[WIDE ? HS_TILE : 132];
     __shared__ double s_red[8];
     __shared__ int s_g;
     if (D->done || !D->prm.hybrid) return;
@@ -2152,12 +2229,42 @@ __global__ void __launch_bounds__(256) k_hscan(Dev* D) {
         const int n = t.n;
         const double rn = (double)n;
         const double* __restrict__ sx = D->arena + t.off_sx + (long long)p * Sched::sx_stride(n);
+        double best = 0.0;
+        if constexpr (WIDE) {
+            if (2 * kk > n) {  // fac(j) grows again past j = n/2: htmaxp's own loops
+                best = htmaxp_one_block_cta(sx, n, kk, al0);
+            } else {
+                // all arcs (i, i+j) and the wrap-around arcs (i, i+n-j), i <= j, tile by tile of lengths
+                for (int j0 = al0; j0 <= kk; j0 += HS_TILE) {
+                    const int j1 = min(kk, j0 + HS_TILE - 1);
+                    __syncthreads();
+                    for (int j = j0 + tid; j <= j1; j += blockDim.x) {
+                        const double rj = (double)j;
+                        s_fac[j - j0] = rn / (rj * (rn - rj));
+                    }
+                    __syncthreads();
+                    for (int i = 1 + tid; i <= n; i += blockDim.x) {
+                        const double si = sx[i];
+                        const int je = min(j1, n - i);
+                        for (int j = j0; j <= je; ++j) {
+                            const double d = fabs(sx[i + j] - si);
+                            const double v = s_fac[j - j0] * d * d;
+                            if (v > best) best = v;
+                        }
+                        for (int j = (i > j0 ? i : j0); j <= j1; ++j) {  // wrap: i <= j
+                            const double d = fabs(sx[i + n - j] - si);
+                            const double v = s_fac[j - j0] * d * d;
+                            if (v > best) best = v;
+                        }
+                    }
+                }
+            }
+        } else {
         for (int j = tid; j <= kk && j < 132; j += blockDim.x) {
             const double rj = (double)j;
             s_fac[j] = (j >= 1) ? rn / (rj * (rn - rj)) : 0.0;
         }
         __syncthreads();
-        double best = 0.0;
         if (2 * kk > n) {  // fac(j) grows again past j = n/2: htmaxp's own loops, one thread (n < 2k <= 256)
             if (tid == 0) best = htmaxp_one_block(sx, n, kk, al0);
         } else
@@ -2176,6 +2283,7 @@ __global__ void __launch_bounds__(256) k_hscan(Dev* D) {
                 const double v = s_fac[j] * d * d;
                 if (v > best) best = v;
             }
+        }
         }
         // per-block (argmin, argmax) candidates of htmaxp's own blocks, nb = int(n/k) (CBS.cpp:390-419)
         const int nbh = (int)(rn / (double)kk);

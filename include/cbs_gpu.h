@@ -46,7 +46,7 @@ typedef struct cbs_gpu_ctx cbs_gpu_ctx;
 typedef struct cbs_gpu_params {
     double alpha;
     int32_t nperm;
-    int32_t hybrid;        /* needs kmax in 1..128 and nmin >= kmax + 1 (weighted: nmin >= kmax + 2) */
+    int32_t hybrid;        /* needs kmax >= 1 (any size) and nmin >= kmax + 1 (weighted: nmin >= max(kmax + 2, 2*kmax - 1)) */
     int32_t min_width;
     int32_t kmax;
     int32_t nmin;
@@ -56,7 +56,7 @@ typedef struct cbs_gpu_params {
     int32_t undo_prune;
     double undo_prune_cutoff;
     int32_t do_smooth;
-    int32_t smooth_region;
+    int32_t smooth_region;  /* any value >= 0 (windows wider than 64 markers take a path of their own) */
     double outlier_sd_scale;
     double smooth_sd_scale;
     double trim;
@@ -171,7 +171,8 @@ int cbs_gpu_fndcpt(cbs_gpu_ctx* ctx, const double* x, int32_t n, double tss, con
                    int32_t ngrid, const uint64_t* mt_next312, cbs_gpu_split* out, uint64_t* draws_consumed);
 /* cbs::wfindcpt (CBS.hpp:81-97, CBS.cpp:894-957).  The reference also takes rwts = sqrt(wts) and cwts =
  * cumsum(wts)/sqrt(sum wts); they are derived from `weights` on the device with the reference's own expressions
- * (CBS.cpp:1056-1066), and delta comes from getmncwt as in wfindcpt (:908). */
+ * (CBS.cpp:1056-1066), and delta comes from getmncwt as in wfindcpt (:908).  With hybrid it needs n >= 2*hk
+ * (CBS_GPU_ERR_UNSUPPORTED otherwise: shorter segments are not implemented). */
 int cbs_gpu_wfindcpt(cbs_gpu_ctx* ctx, const double* x, const double* weights, int32_t n, double tss,
                      const cbs_gpu_params* params, int32_t ngrid, const uint64_t* mt_next312, cbs_gpu_split* out,
                      uint64_t* draws_consumed);
@@ -190,7 +191,7 @@ int cbs_gpu_wtmaxo(cbs_gpu_ctx* ctx, const double* x, const double* weights, int
 int cbs_gpu_xperm(cbs_gpu_ctx* ctx, const double* x, const double* rwts, int32_t n, const uint64_t* mt_next312, uint64_t seed,
                   double* px);
 /* cbs::htmaxp (CBS.hpp:34, CBS.cpp:387-485) for `count` vectors of length n laid end to end; ibin must be 0,
- * al0 <= k <= 128 and n >= k (with n < k the reference's htmaxp has no block and is undefined) */
+ * 1 <= al0 <= k (any k) and n >= k (with n < k the reference's htmaxp has no block and is undefined) */
 int cbs_gpu_htmaxp(cbs_gpu_ctx* ctx, const double* px, int32_t n, int32_t count, double tss, int32_t k, int32_t al0,
                    int32_t ibin, double* statistics);
 /* cbs::tailp (CBS.hpp:29, CBS.cpp:324-339); ngrid must be 100.  Evaluated with the CUDA erfc/log/exp/pow (<= 4 ulp each), so
